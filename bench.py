@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — points/sec through kNN(k=16) + PCA normals + plane slicing + ordered contours.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 1M-point synthetic freeform panel per GPU, k=16 normals +
 200*sqrt(N) slices (5 mm apart, band +-2 mm, SectPath pairing); weak scaling: the ONE cloud has N x 1M
@@ -26,6 +26,11 @@ pcl::PointXYZRGB records.
   roofline : dominant kernel's algorithmic bytes / its CUDA-event duration vs MEASURED_PEAKS.json.
   cpu_baseline / --impl reference : the CPU oracle (port of the reference's PCL/FLANN path; the
           reference itself cannot be built here, see DESIGN.md) on the box's host cores.
+  --dump-outputs DIR (one GPU) : after the timed steps, what the last of them computed, as DIR/<name>.npy
+          (float32 / float64, integers stored exactly): normals (pcl::Normal records), neighbour_ids,
+          contour_offsets (per plane) and contour_y / _x / _z.  An output with more rows than DUMP_ROWS allows
+          is written as a fixed seeded sample of rows, their indices in <name>_rows.npy.  The inputs depend on
+          the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -38,6 +43,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True      # the tree bench.py runs from may be read-only: nothing is written there
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -49,6 +55,10 @@ HALO_MM = 12.0
 SETTLE_STEPS = 10         # untimed steps in front of the W warm-up steps (see timed_device_steps)
 PAIRING = "B"             # SectPath::insert_point (src/contour_alg.cpp:165-237)
 CPU_SAMPLE_MAX = 2_000_000   # --impl reference: points of the workload one CPU step processes
+# --dump-outputs: rows written per output before it is sampled, so that every configuration stays under
+# DUMP_MAX_BYTES (cfg2 on one GPU is written whole except for the neighbour ids)
+DUMP_ROWS = {"normals": 1 << 20, "neighbour_ids": 1 << 15, "contour": 1 << 18}
+DUMP_MAX_BYTES = 64_000_000
 
 
 def make_cfg(name, gpus):
@@ -278,8 +288,9 @@ class Env:
         self.ctx.close()
 
 
-def timed_device_steps(env, step, steps, warmup):
-    """W warm-up + K timed steps, each behind an L2 flush; CUDA events on the library's stream."""
+def timed_device_steps(env, step, steps, warmup, last_step=None):
+    """W warm-up + K timed steps, each behind an L2 flush; CUDA events on the library's stream.
+    last_step: run in place of step for the last timed step (one that keeps its outputs readable)."""
     ctx = env.ctx
     # settle first: the first steps of a process see one-off costs (memory pools growing to their working size, lazy
     # module loads, clocks leaving idle) that have shown up as single steps of tens of milliseconds; then the W warm-ups
@@ -293,11 +304,11 @@ def timed_device_steps(env, step, steps, warmup):
     l0 = ctx.launch_count()
     env.sync_all()
     t_wall0 = time.perf_counter()
-    for _ in range(steps):
+    for i in range(steps):
         env.flush_l2()
         env.stream.synchronize()
         ctx.timer_begin(0)
-        step()
+        (last_step if last_step is not None and i == steps - 1 else step)()
         ctx.timer_end(0)
     env.sync_all()
     t_wall = time.perf_counter() - t_wall0
@@ -361,7 +372,40 @@ def normals_call(c, cfg, normals_ptr, stride, idx_ptr):
         c.dev_normals_knn(cfg["k"], normals_ptr, stride, idx_ptr=idx_ptr)
 
 
-def measure_single(env, cfg, steps, warmup, e2e=True):
+def dump_rows(n, cap):
+    """The rows of an n-row output that --dump-outputs writes: all of them, or a fixed seeded sample of cap."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def last_step_outputs(env, cfg, contours, normals_d, idx_d):
+    """The outputs of the last timed step as host arrays, for --dump-outputs (read after the timed window)."""
+    torch, ctx = env.torch, env.ctx
+    out = {}
+    for name, t, dtype in (("normals", normals_d, np.float32), ("neighbour_ids", idx_d, np.float64)):
+        rows = dump_rows(t.shape[0], DUMP_ROWS[name])
+        out[name] = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy().astype(dtype)
+        if len(rows) < t.shape[0]:
+            out[name + "_rows"] = rows.astype(np.float64)
+    nodes = int(contours["total_nodes"])
+    out["contour_offsets"] = ctx.download(contours["node_offsets"], (cfg["S"] + 1,), np.int64).astype(np.float64)
+    rows = dump_rows(nodes, DUMP_ROWS["contour"])
+    for axis in "yxz":
+        out["contour_" + axis] = ctx.download(contours[axis], (nodes,), np.float64)[rows]
+    if len(rows) < nodes:
+        out["contour_rows"] = rows.astype(np.float64)
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    return out
+
+
+def write_outputs(path, outputs):
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def measure_single(env, cfg, steps, warmup, e2e=True, dump=False):
     from polishpathplanning_b200 import api, synth
     torch, ctx, dev = env.torch, env.ctx, env.dev
     n, k, S = cfg["n_total"], cfg["k"], cfg["S"]
@@ -374,20 +418,28 @@ def measure_single(env, cfg, steps, warmup, e2e=True):
     env.stream.synchronize()
     last = {}
 
-    def dev_step():
+    def dev_step(keep=False):
         c = api.Cloud(ctx, device_ptr=raw_d.data_ptr(), n=n, stride_bytes=32)
         normals_call(c, cfg, normals_d.data_ptr(), 32, idx_d.data_ptr())
         res = c.dev_slice_contours(planes, PAIRING, HALF_WIDTH, True)
         last["nodes"], last["members"] = res["total_nodes"], res["total_members"]
-        c.close()
+        if keep:        # the cloud owns the contour buffers: read back after the timed window, then closed
+            last["cloud"], last["contours"] = c, res
+        else:
+            c.close()
 
-    total_ms, _, launches, t_wall = timed_device_steps(env, dev_step, steps, warmup)
+    total_ms, _, launches, t_wall = timed_device_steps(env, dev_step, steps, warmup,
+                                                       last_step=(lambda: dev_step(keep=True)) if dump else None)
+    outputs = None
+    if dump:
+        outputs = last_step_outputs(env, cfg, last["contours"], normals_d, idx_d)
+        last.pop("cloud").close()
     prof = kernel_profile(env, dev_step, steps)
     if not e2e:
         del raw_d, normals_d, idx_d
         return {"units": n, "total_ms": total_ms, "launches": launches, "t_wall": t_wall, "prof": prof, "e2e_s": float("nan"),
                 "h2d": 0, "d2h": 0, "n_local": n, "members": last.get("members", 0), "nodes": last.get("nodes", 0),
-                "exchange_ms": None, "parity": None}
+                "exchange_ms": None, "parity": None, "outputs": outputs}
 
     # ---- end to end through the host-pointer C ABI (pinned buffers) ----
     pin_cloud = ctx.pinned_empty(cloud.shape, np.float32)
@@ -420,7 +472,7 @@ def measure_single(env, cfg, steps, warmup, e2e=True):
     del raw_d, normals_d, idx_d
     return {"units": n, "total_ms": total_ms, "launches": launches, "t_wall": t_wall, "prof": prof, "e2e_s": e2e_s,
             "h2d": e2e_bytes.get("h2d", 0), "d2h": e2e_bytes.get("d2h", 0), "n_local": n, "members": last.get("members", 0),
-            "nodes": last.get("nodes", 0), "exchange_ms": None, "parity": None}
+            "nodes": last.get("nodes", 0), "exchange_ms": None, "parity": None, "outputs": outputs}
 
 
 # ---- N GPUs, one rank each ----------------------------------------------------------------------
@@ -634,18 +686,22 @@ def measure_multi(env, cfg, steps, warmup, verify=True, e2e=True):
 def run_ours(args):
     env = Env(args)
     cfg = make_cfg(args.config, env.world)
-    measure = measure_single if env.world == 1 else measure_multi
     sampler = ClockSampler(env.local_rank)
     if env.rank == 0:
         sampler.start()
-    m = measure(env, cfg, args.steps, args.warmup)
+    if env.world == 1:
+        m = measure_single(env, cfg, args.steps, args.warmup, dump=args.dump_outputs is not None)
+    else:
+        m = measure_multi(env, cfg, args.steps, args.warmup)
     clocks = sampler.stop() if env.rank == 0 else None
+    if args.dump_outputs is not None:
+        write_outputs(args.dump_outputs, m.pop("outputs"))
     extra = None
     if args.config == "cfg2" and not args.no_cfg3:
         # the north-star configuration (BASELINE.json configs[2]: 10M points, k = 32, 1000 slices) on the same GPUs,
         # a few steps, so that the driver's record carries the "< 50 ms on 8 GPUs" figure next to the headline
         cfg3 = make_cfg("cfg3", env.world)
-        m3 = measure(env, cfg3, 5, 3) if env.world == 1 else measure_multi(env, cfg3, 5, 3, verify=False)
+        m3 = measure_single(env, cfg3, 5, 3) if env.world == 1 else measure_multi(env, cfg3, 5, 3, verify=False)
         extra = {"workload": cfg3["text"], "n_gpus": env.world, "steps": 5, "warmup": 3,
                  "device_ms_per_step": m3["total_ms"] / 5, "e2e_ms_per_step": 1e3 * m3["e2e_s"] / 5,
                  "exchange_ms_per_step": m3["exchange_ms"], "target_ms": 50.0}
@@ -693,7 +749,13 @@ def main():
                     help="cfg2 (default, the driver's contract): 1M points per GPU, k=16, 200*sqrt(N) planes, weak scaling. "
                          "cfg3 (SURVEY 8d): 10M points in TOTAL split over the GPUs, k=32, 1000 planes.")
     ap.add_argument("--no-cfg3", action="store_true", help="skip the extra north-star (cfg3) measurement of a cfg2 run")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (one GPU, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.gpus != 1 or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of the one-GPU path: use it with --gpus 1 --impl ours")
     if args.impl != "reference" and args.warmup < 3:
         args.warmup = 3       # timing rule: at least three warm-up steps
     if args.impl == "reference":

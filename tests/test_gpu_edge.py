@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from oracle import ppp_oracle as po
+from pinned_golden import assert_pinned
 from polishpathplanning_b200 import api, reference_api as ra, synth
 
 pytestmark = pytest.mark.gpu
@@ -32,8 +33,8 @@ def test_golden_independent_vectors(ctx):
         gc = api.Cloud(ctx, synth.panel(n, seed))
         for k in ks:
             idx, d2 = gc.knn(k)
-            assert np.array_equal(idx, g["knn_idx_n%d_s%d_k%d" % (n, seed, k)])
-            assert np.array_equal(d2.view(np.uint32), g["knn_d2_n%d_s%d_k%d" % (n, seed, k)].view(np.uint32))
+            assert_pinned(g, "knn_idx_n%d_s%d_k%d" % (n, seed, k), idx)
+            assert_pinned(g, "knn_d2_n%d_s%d_k%d" % (n, seed, k), d2)
         gc.close()
     gc = api.Cloud(ctx, synth.panel(4000, 1))
     counts, off, idx, d2 = gc.radius(2.5)
