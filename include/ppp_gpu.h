@@ -174,6 +174,20 @@ int ppp_coverage_mark(ppp_cloud* cloud, const float* q, size_t nq, size_t q_stri
 int ppp_coverage_mark_radii(ppp_cloud* cloud, const float* q, size_t nq, size_t q_stride_bytes, const double* radii,
                             unsigned char* flags);
 
+/* smooth(): the MLS pre-filter (src/Path_Generation.cpp:340-360; SectPath with Smooth = true,
+ * src/contour_alg.cpp:27): pcl::MovingLeastSquares, polynomial order `order` (0..3; 0 and 1 project onto the
+ * local plane), search radius `radius`, no upsampling, SIMPLE projection, weight exp(-d^2 / radius^2), normals
+ * computed.  One output row per finite point with at least 3 neighbours (d2 < (float)(radius*radius), the point
+ * itself included), in ascending source order; other points have none.  The caller provides room for n rows:
+ * points_out: records of out_stride_bytes (>= 12, multiple of 4) of which only x, y, z are written;
+ * normals_out (nullable): {nx, ny, nz, curvature} per row; src_index_out: source index of each row;
+ * *n_out: rows written.
+ * Tolerance contract (the fit is double-precision arithmetic summed in a different order than PCL's):
+ * the rows and the branch taken per row (polynomial fit or plane) are exact; x, y, z are within 2 float ulps
+ * of the CPU restatement and almost always identical; normals and curvature within 1e-5.               */
+int ppp_mls_smooth(ppp_cloud* cloud, double radius, int order, void* points_out, size_t out_stride_bytes,
+                   float* normals_out, int32_t* src_index_out, int64_t* n_out);
+
 /* estimate_normal() followed by the plane sweep, as one call: what SectPath-derived GenPath does
  * (src/Path_Alg/path_dynamic_alg.cpp:343-366: estimate_normal(); kdtree.setInputCloud; sweep).
  * Exactly the results of ppp_normals_knn (k >= 1, radius = 0) or ppp_normals_radius (k = 0,

@@ -167,18 +167,21 @@ class Cloud:
         self.ctx = ctx
         self.lib = ctx.lib
         h = _vp()
+        self._records = None   # where mls_smooth copies the fields other than x, y, z from
         if handle is not None:         # an existing ppp_cloud* (e.g. from ppp_exch_attach); owned from here on
             h = handle
             self.n = int(self.lib.ppp_cloud_size(h))
         elif device_ptr is not None:
             check(self.lib.ppp_dev_cloud_attach(ctx._h, _vp(device_ptr), int(n), int(stride_bytes), C.byref(h)))
             self.n = int(n)
+            self._records = (int(device_ptr), int(stride_bytes))
         else:
             pts = np.asarray(points)
             if pts.dtype != np.float32 or pts.ndim != 2 or pts.shape[1] < 3 or not pts.flags.c_contiguous:
                 raise ValueError("points must be a C-contiguous float32 array of shape (N, >=3)")
             check(self.lib.ppp_cloud_upload(ctx._h, _ptr(pts), pts.shape[0], pts.shape[1] * 4, C.byref(h)))
             self.n = pts.shape[0]
+            self._records = pts
         self._h = h
         ctx._clouds.add(self)
 
@@ -358,6 +361,29 @@ class Cloud:
         check(self.lib.ppp_coverage_mark_radii(self._h, _ptr(queries), queries.shape[0], queries.shape[1] * 4, _ptr(radii),
                                                _ptr(flags)))
         return flags
+
+    def mls_smooth(self, radius=15.0, order=3, normals=False):
+        """smooth(): MovingLeastSquares (no upsampling, SIMPLE projection).  Returns (points, src_index, normals):
+        points (m, stride) float32 records -- x, y, z smoothed, every other field copied from source row
+        src_index[i] --, normals (m, 4) {nx, ny, nz, curvature} or None.  Points with fewer than 3 neighbours
+        within the radius, and non-finite points, have no row."""
+        recs = self._records
+        if recs is None:
+            raise ValueError("mls_smooth needs the cloud's records (not available for a cloud built from a handle)")
+        if not isinstance(recs, np.ndarray):   # device-attached cloud: fetch the records once
+            ptr, stride = recs
+            recs = self.ctx.download(ptr, (self.n, stride // 4), np.float32)
+        pts = np.empty((self.n, recs.shape[1]), np.float32)
+        src = np.empty(self.n, np.int32)
+        nrm = np.empty((self.n, 4), np.float32) if normals else None
+        m = C.c_int64(0)
+        check(self.lib.ppp_mls_smooth(self._h, float(radius), int(order), _ptr(pts), pts.shape[1] * 4, _ptr(nrm),
+                                      _ptr(src), C.byref(m)))
+        m = m.value
+        src = src[:m].copy()
+        out = recs[src].copy()
+        out[:, 0:3] = pts[:m, 0:3]
+        return out, src, (nrm[:m].copy() if normals else None)
 
     # ---- device-resident pipeline ---------------------------------------------------------------
     def dev_index(self, k_hint=16, radius_hint=0.0):

@@ -935,4 +935,37 @@ int ppp_sor_mean_distances(ppp_cloud* c, int mean_k, unsigned flags, float* dist
   return PPP_OK;
 }
 
+// smooth(): pcl::MovingLeastSquares with polynomial order `order` and search radius `radius`
+// (src/Path_Generation.cpp:340-360), no upsampling, SIMPLE projection.  Rows are written for the finite points
+// with at least 3 neighbours, in ascending source order; points_out / normals_out / src_index_out hold n rows.
+int ppp_mls_smooth(ppp_cloud* c, double radius, int order, void* points_out, size_t out_stride_bytes, float* normals_out,
+                   int32_t* src_index_out, int64_t* n_out) {
+  REQUIRE(c && n_out && ((points_out && src_index_out) || c->n == 0), "NULL argument");
+  REQUIRE(radius > 0 && std::isfinite(radius), "radius must be > 0");
+  REQUIRE(order >= 0 && order <= 3, "order must be 0..3");
+  REQUIRE(out_stride_bytes >= 12 && out_stride_bytes % 4 == 0, "output stride must be >= 12 and a multiple of 4");
+  ppp_ctx* ctx = c->ctx;
+  LOCK(ctx);
+  PPP_CUDA(cudaSetDevice(ctx->device));
+  *n_out = 0;
+  if (c->n == 0) return PPP_OK;
+  float* xyz_d = nullptr; float4* nrm_d = nullptr; int32_t* src_d = nullptr;
+  PPP_TRY(dev_alloc(ctx, &xyz_d, (size_t)c->n * 3));
+  if (normals_out) PPP_TRY(dev_alloc(ctx, &nrm_d, (size_t)c->n));
+  PPP_TRY(dev_alloc(ctx, &src_d, (size_t)c->n));
+  int64_t m = 0;
+  int st = mls_smooth_launch(c, radius, order, xyz_d, nrm_d, src_d, &m);
+  if (st == PPP_OK && m > 0) {
+    PPP_CUDA(cudaMemcpy2DAsync(points_out, out_stride_bytes, xyz_d, 12, 12, (size_t)m, cudaMemcpyDeviceToHost, ctx->stream));
+    if (normals_out) PPP_CUDA(cudaMemcpyAsync(normals_out, nrm_d, (size_t)m * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    PPP_CUDA(cudaMemcpyAsync(src_index_out, src_d, (size_t)m * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  dev_free(ctx, xyz_d); dev_free(ctx, nrm_d); dev_free(ctx, src_d);
+  if (st != PPP_OK) return st;
+  PPP_CUDA(e);
+  *n_out = m;
+  return PPP_OK;
+}
+
 }  // extern "C"

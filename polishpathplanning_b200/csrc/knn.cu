@@ -1897,6 +1897,8 @@ int pick_block(ppp_ctx* ctx, int cap, int* block, size_t* smem) {
   return PPP_ERR_UNSUPPORTED;
 }
 
+}  // namespace
+
 int radius_rings(const GridView& g, double r) {
   // need R*h - slack >= r
   // r comes from sqrt((float)(r*r)); a float32 d2 below r2 can belong to a point up to ~1e-7 beyond it
@@ -1905,8 +1907,6 @@ int radius_rings(const GridView& g, double r) {
   while ((double)R * (double)g.h - (double)g.slack < r) R++;
   return std::max(R, 0);
 }
-
-}  // namespace
 
 static int launch_search(ppp_cloud* c, SearchParams& P) {
   ppp_ctx* ctx = c->ctx;

@@ -353,8 +353,15 @@ int principal_curvatures_launch(ppp_cloud* c, const int32_t* idx_dev, int64_t nq
                                 int normal_stride_f, float* out_dev, int32_t* nn0_dev);
 int sor_mean_distances_launch(ppp_cloud* c, const GridStore& gs, int mean_k, int sqrt_float, float* dist_dev,
                               unsigned long long* n_valid_dev);
+// Cells of the ring block around a query that cover radius r on grid g (two at cloud_cell_for_radius's cell size).
+int radius_rings(const GridView& g, double r);
 int coverage_mark_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f, float r2,
                          unsigned char* flags_dev, const float* r2_per_query_dev = nullptr);
+
+// mls.cu
+// ppp_mls_smooth's device part: compacted rows (xyz_c: 3 floats per row; nrm_c nullable: nx ny nz curvature;
+// src_c: source index) for every finite point with >= 3 neighbours, in ascending source order.  Synchronises.
+int mls_smooth_launch(ppp_cloud* c, double radius, int order, float* xyz_c, float4* nrm_c, int32_t* src_c, int64_t* n_rows);
 
 // slices.cu
 int bands_launch(ppp_cloud* c, const float* plane_x_host, int S, float half_width, int truncate_center, int sort_bands,

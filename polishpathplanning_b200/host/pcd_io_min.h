@@ -1,5 +1,5 @@
-// Minimal PCD reader (ascii / binary, float x y z [rgb|rgba]) standing in for
-// pcl::io::loadPCDFile<pcl::PointXYZRGB> (src/Path_Generation.cpp:8) when PCL is absent.
+// Minimal PCD reader (ascii / binary, float x y z [rgb|rgba]) and writer (binary, FIELDS x y z rgb) standing in
+// for pcl::io::loadPCDFile / savePCDFile<pcl::PointXYZRGB> (src/Path_Generation.cpp:8,340-360) when PCL is absent.
 #pragma once
 #include <cstdio>
 #include <cstring>
@@ -70,5 +70,20 @@ inline int loadPCDFile(const std::string& path, pcl::PointCloud<pcl::PointXYZRGB
     return -1;
   }
   return 0;
+}
+
+// binary PCD v0.7, FIELDS x y z rgb (the layout polishpathplanning_b200.synth.write_pcd writes); 0 / -1
+inline int savePCDFile(const std::string& path, const pcl::PointCloud<pcl::PointXYZRGB>& cloud) {
+  std::ofstream f(path, std::ios::binary);
+  if (!f) return -1;
+  const size_t n = cloud.points.size();
+  f << "# .PCD v0.7 - Point Cloud Data file format\nVERSION 0.7\nFIELDS x y z rgb\nSIZE 4 4 4 4\nTYPE F F F F\n"
+       "COUNT 1 1 1 1\nWIDTH " << n << "\nHEIGHT 1\nVIEWPOINT 0 0 0 1 0 0 0\nPOINTS " << n << "\nDATA binary\n";
+  for (const pcl::PointXYZRGB& p : cloud.points) {
+    float rec[4] = {p.x, p.y, p.z, 0.0f};
+    memcpy(&rec[3], &p.rgba, 4);
+    f.write(reinterpret_cast<const char*>(rec), sizeof(rec));
+  }
+  return f ? 0 : -1;
 }
 }  // namespace ppp_host

@@ -157,6 +157,27 @@ inline MAP insert_point(ppp_cloud* c, const std::vector<int>& indices, float pla
   return m;
 }
 
+// smooth() (src/Path_Generation.cpp:340-360): MovingLeastSquares, order 3, radius 15, on the device.  The cloud
+// is replaced by the smoothed records (x, y, z from the fit, every other field from the source point; points with
+// fewer than 3 neighbours are dropped) and written to smooth_<file name>.pcd in the working directory.
+inline void mls_smooth(ppp_cloud* dc, PointCloudType& cloud, const std::string& cloud_name) {
+  const size_t n = cloud.points.size();
+  std::vector<PointType> xyz(n);
+  std::vector<int32_t> src(n);
+  int64_t m = 0;
+  check(ppp_mls_smooth(dc, 15.0, 3, xyz.data(), sizeof(PointType), nullptr, src.data(), &m), "ppp_mls_smooth");
+  std::vector<PointType, decltype(cloud.points.get_allocator())> out((size_t)m);
+  for (int64_t i = 0; i < m; i++) {
+    out[(size_t)i] = cloud.points[(size_t)src[(size_t)i]];
+    out[(size_t)i].x = xyz[(size_t)i].x; out[(size_t)i].y = xyz[(size_t)i].y; out[(size_t)i].z = xyz[(size_t)i].z;
+  }
+  cloud.points.swap(out);
+  cloud.width = (uint32_t)m; cloud.height = 1;
+  const size_t slash = cloud_name.find_last_of('/');
+  const std::string out_name = "smooth_" + (slash == std::string::npos ? cloud_name : cloud_name.substr(slash + 1));
+  if (savePCDFile(out_name, cloud) != 0) fprintf(stderr, "smooth: could not write %s\n", out_name.c_str());
+}
+
 inline MAP to_map(const Contours& c, int s) {
   MAP m;
   for (int64_t i = c.offsets[s]; i < c.offsets[s + 1]; i++) m[c.y[i]] = {c.x[i], c.z[i]};
@@ -188,6 +209,11 @@ public:
   }
 
   void Set_kdtree() { dev_.get(*cloud); }  // kdtree.setInputCloud(cloud)
+
+  void smooth() {  // src/Path_Generation.cpp:340-360
+    ppp_host::mls_smooth(dev_.get(*cloud), *cloud, file_name);
+    dev_.invalidate();
+  }
 
   void estimate_normal() {  // NormalEstimation, setRadiusSearch(2.5), viewpoint (0,0,0)
     const float vp[3] = {0, 0, 0};
@@ -274,13 +300,18 @@ public:
         if (ifChangeRange) { cloud->points[i].x *= 1000; cloud->points[i].y *= 1000; cloud->points[i].z *= 1000; }
       }
     }
-    // src/contour_alg.cpp:27-29.  smooth (MLS) and trans2center (PCA alignment) are outside the
-    // accelerated path (DESIGN.md, out of scope): say so instead of silently skipping them.
-    if (ifSmooth) fprintf(stderr, "SectPath: Smooth=true is not available in this build (MLS is out of scope)\n");
+    // src/contour_alg.cpp:27-29.  trans2center (PCA alignment) is outside the accelerated path (DESIGN.md, out of
+    // scope): say so instead of silently skipping it.
+    if (ifSmooth) smooth();
     if (ifAlign) fprintf(stderr, "SectPath: Alignment=true is not available in this build (trans2center is out of scope)\n");
     if (ifRemove && cloud->points.size() > 50) remove_outlier();
   }
   virtual ~SectPath() {}
+
+  void smooth() {  // the MLS pre-filter shared with path_generater::smooth()
+    ppp_host::mls_smooth(dev_.get(*cloud), *cloud, cloud_name);
+    dev_.invalidate();
+  }
 
   void estimate_normal() {
     const float vp[3] = {0, 0, 0};

@@ -13,6 +13,8 @@ for ALL nodes of a path in one device call where the reference loops node by nod
 hand-eye / flange transforms and file export stay with the reference's own host code.
 Plane positions are generated here exactly as each reference loop does, in float32.
 """
+import os
+
 import numpy as np
 
 from . import api, synth
@@ -159,6 +161,8 @@ class Spline:
 class _Base:
     NORMAL_RADIUS = 2.5   # normal_estimation.setRadiusSearch(2.5): src/Path_Generation.cpp:329
     BAND_HALF_WIDTH = 2.0  # setFilterLimits(-2 + position, 2 + position): src/Path_Generation.cpp:100
+    SMOOTH_RADIUS = 15.0   # mls.setSearchRadius(15): src/Path_Generation.cpp:340-360
+    SMOOTH_ORDER = 3       # mls.setPolynomialOrder(3)
 
     def __init__(self, ctx=None, device=0, backend=None):
         # backend: callable(cloud) -> an object with api.Cloud's methods; the CPU tests pass an oracle-backed
@@ -171,6 +175,7 @@ class _Base:
         self.Path_set = []
 
     def _load(self, cloud_name, change_range=True):
+        self.cloud_name = cloud_name if isinstance(cloud_name, str) else "cloud.pcd"
         if isinstance(cloud_name, str):
             try:
                 cloud = synth.read_pcd(cloud_name)
@@ -206,6 +211,17 @@ class _Base:
         """NormalEstimation, radius 2.5, viewpoint (0,0,0) -> (N, 8) pcl::Normal records."""
         self.cloud_with_normals = self._dev().normals_radius(self.NORMAL_RADIUS)
         return self.cloud_with_normals
+
+    def smooth(self):
+        """smooth() (src/Path_Generation.cpp:340-360): MovingLeastSquares, order 3, radius 15, no upsampling,
+        SIMPLE projection.  The cloud becomes the smoothed records (points with fewer than 3 neighbours are
+        dropped; fields other than x, y, z come from the source point), is written to smooth_<file name>.pcd in
+        the working directory, and the device copy is rebuilt on next use.  Returns the source index per row."""
+        pts, src, _ = self._dev().mls_smooth(self.SMOOTH_RADIUS, self.SMOOTH_ORDER)
+        self.cloud = np.ascontiguousarray(pts)
+        self._invalidate()
+        synth.write_pcd("smooth_" + os.path.basename(self.cloud_name), self.cloud)
+        return src
 
     def rangedX_index(self, position):
         """std::vector<int> rangedX_index(int position): the argument is truncated to int."""
@@ -499,10 +515,13 @@ def sor_select(distances, n_valid, stddev_mul=1.0, negative=False):
 class SectPath(_Base):
     """SectPath (contour_alg.h): kd-tree pairing without flags (variant B), centre-out sweep."""
 
-    def __init__(self, cloud_name, Tool_Radius, ChangeRange=True, RemoveOutlier=False, ctx=None, device=0, backend=None):
+    def __init__(self, cloud_name, Tool_Radius, ChangeRange=True, RemoveOutlier=False, Smooth=False, ctx=None, device=0,
+                 backend=None):
         super().__init__(ctx, device, backend)
         self.toolRadius = float(Tool_Radius)
         self._load(cloud_name, change_range=ChangeRange)
+        if Smooth:                                          # src/contour_alg.cpp:27, before remove_outlier
+            self.smooth()
         if RemoveOutlier and self.cloud.shape[0] > 50:      # src/contour_alg.cpp:29
             self.remove_outlier()
 
