@@ -796,14 +796,18 @@ int ppp_coverage_mark_radii(ppp_cloud* c, const float* q, size_t nq, size_t q_st
   PPP_CUDA(cudaSetDevice(ctx->device));
   if (c->n == 0 || nq == 0) return PPP_OK;
   std::vector<float> r2(nq);
-  double rmax = 0;
+  double rmax = 0, rfin = 0;   // largest |radius| (NaN radii mark nothing), largest finite one
   for (size_t i = 0; i < nq; i++) {
     r2[i] = (float)(radii[i] * radii[i]);   // [upstream] pcl::KdTreeFLANN::radiusSearch squares the radius in double
-    if (std::isfinite(radii[i])) rmax = std::max(rmax, std::fabs(radii[i]));
+    const double a = std::fabs(radii[i]);
+    if (a > rmax) rmax = a;
+    if (std::isfinite(a) && a > rfin) rfin = a;
   }
   if (!(rmax > 0)) return PPP_OK;
+  // The block radius below covers the largest radius, infinite ones included (an infinite float32 r2 marks every
+  // finite point); any cell size serves those, so the grid is sized by the finite radii.
   GridStore* g;
-  PPP_TRY(cloud_get_grid(c, cloud_cell_for_radius(c, rmax), &g));
+  PPP_TRY(cloud_get_grid(c, rfin > 0 ? cloud_cell_for_radius(c, rfin) : cloud_cell_for_k(c, 16), &g));
   unsigned char* f_d = nullptr; float* q_d = nullptr; float* r_d = nullptr;
   PPP_TRY(dev_alloc(ctx, &f_d, (size_t)c->n));
   PPP_TRY(dev_alloc(ctx, (char**)&q_d, nq * q_stride_bytes + 16));
@@ -941,7 +945,7 @@ int ppp_sor_mean_distances(ppp_cloud* c, int mean_k, unsigned flags, float* dist
 int ppp_mls_smooth(ppp_cloud* c, double radius, int order, void* points_out, size_t out_stride_bytes, float* normals_out,
                    int32_t* src_index_out, int64_t* n_out) {
   REQUIRE(c && n_out && ((points_out && src_index_out) || c->n == 0), "NULL argument");
-  REQUIRE(radius > 0 && std::isfinite(radius), "radius must be > 0");
+  REQUIRE(radius > 0 && std::isfinite((float)(radius * radius)), "radius must be > 0 with a finite float32 square");
   REQUIRE(order >= 0 && order <= 3, "order must be 0..3");
   REQUIRE(out_stride_bytes >= 12 && out_stride_bytes % 4 == 0, "output stride must be >= 12 and a multiple of 4");
   ppp_ctx* ctx = c->ctx;

@@ -1901,10 +1901,14 @@ int pick_block(ppp_ctx* ctx, int cap, int* block, size_t* smem) {
 
 int radius_rings(const GridView& g, double r) {
   // need R*h - slack >= r
-  // r comes from sqrt((float)(r*r)); a float32 d2 below r2 can belong to a point up to ~1e-7 beyond it
+  // r comes from sqrt((float)(r*r)); a float32 d2 below r2 can belong to a point up to ~1e-7 beyond it.
+  // A radius whose float32 square is infinite (r = inf here) admits every finite point: capped at PPP_RING_MAX,
+  // the block around any (clamped) query cell covers the whole grid, and the d2 < r2 test decides.
   r *= 1.0 + 1e-6;
-  int R = (int)std::ceil((r + (double)g.slack) / (double)g.h - 1e-12);
-  while ((double)R * (double)g.h - (double)g.slack < r) R++;
+  const double Rd = std::ceil((r + (double)g.slack) / (double)g.h - 1e-12);
+  if (!(Rd < (double)PPP_RING_MAX)) return PPP_RING_MAX;
+  int R = (int)Rd;
+  while (R < PPP_RING_MAX && (double)R * (double)g.h - (double)g.slack < r) R++;
   return std::max(R, 0);
 }
 

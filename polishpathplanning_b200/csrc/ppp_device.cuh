@@ -53,12 +53,22 @@ __device__ __forceinline__ u64 make_key(float d2, int idx) {
 __device__ __forceinline__ float key_d2(u64 k) { return __uint_as_float((uint32_t)(k >> 32)); }
 __device__ __forceinline__ int key_idx(u64 k) { return (int)(uint32_t)(k & 0xFFFFFFFFull); }
 
-// Cell coordinate along one axis. Monotone non-decreasing in `a` (float sub, mul by a positive
-// constant and floor are monotone), which is what the ring-termination bound relies on.
-__device__ __forceinline__ int cell_coord_raw(float a, float amin, float inv_h) {
-  return __float2int_rd(__fmul_rn(__fsub_rn(a, amin), inv_h));
-}
 __device__ __forceinline__ int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
+
+// Cell coordinate along one axis, clamped to [-PPP_CELL_LIM, PPP_CELL_LIM]. Monotone non-decreasing in `a`
+// (float sub, mul by a positive constant, floor and the clamp are monotone), which is what the ring-termination
+// bound relies on.  Why the clamp keeps every search exact: grid cells lie in [0, nu - 1] and nu, nv <= 2^27
+// (nu * nv <= 2^28, both >= 2), so clamping moves a far query's cell TOWARDS every grid cell and the cell distance
+// to any point only shrinks.  ring_bound2 is a lower bound on the distance derived from that cell distance, so it
+// stays a lower bound; the rounding of the unclamped coordinate (<= 3 * 2^-24 of it) is covered by its slack term,
+// which grows with |cu| + |cv| >= 2^29 for a clamped query.  The clamp keeps every sum a search forms in int32:
+// |cu|, |cv| <= 2^29, rings R <= PPP_RING_MAX = 2^30 (a ring loop stops once its block covers the grid, R <=
+// 2^29 + 2^27), so cu +- R, cv +- R and their differences stay below 2^31 in magnitude.
+constexpr int PPP_CELL_LIM = 1 << 29;
+constexpr int PPP_RING_MAX = 1 << 30;   // a block of this half-width around any clamped cell covers the whole grid
+__device__ __forceinline__ int cell_coord_raw(float a, float amin, float inv_h) {
+  return clampi(__float2int_rd(__fmul_rn(__fsub_rn(a, amin), inv_h)), -PPP_CELL_LIM, PPP_CELL_LIM);
+}
 
 __device__ __forceinline__ float axis_of(float x, float y, float z, int a) { return a == 0 ? x : (a == 1 ? y : z); }
 
@@ -67,7 +77,9 @@ __device__ __forceinline__ float axis_of(float x, float y, float z, int a) { ret
 // float32 d2 (relative error <= 3*2^-24) of an unseen point can never tie or beat an accepted one.
 __device__ __forceinline__ float ring_bound2(const GridView& g, int R, int cu, int cv) {
   // slack grows with the magnitude of the cell coordinates involved (queries may lie far outside the grid)
-  float extra = __fmul_ru(g.h, __fmul_ru((float)(abs(cu) + abs(cv) + R + 2), 4.76837158203125e-07f));
+  // (the magnitude sum is formed in float: |cu| + |cv| + R can pass 2^31 for a clamped far query)
+  const float mag = __fadd_ru(__fadd_ru(__int2float_ru(abs(cu)), __int2float_ru(abs(cv))), __fadd_ru(__int2float_ru(R), 2.0f));
+  float extra = __fmul_ru(g.h, __fmul_ru(mag, 4.76837158203125e-07f));
   float rb = __fsub_rd(__fsub_rd(__fmul_rd((float)R, g.h), g.slack), extra);
   if (rb <= 0.0f) return 0.0f;
   return __fmul_rd(__fmul_rd(rb, rb), 0.999999f);
