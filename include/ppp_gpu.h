@@ -146,7 +146,12 @@ int ppp_slice_contours(ppp_cloud* cloud, const float* plane_x, int S, float half
 /* insert_point(indices, PlanePoint) with the CALLER's index list instead of the band of the plane
  * (same reference lines as above; every reference call site passes rangedX_index(PlanePoint[0]),
  * for which ppp_slice_contours is the one-call equivalent).  indices: strictly ascending.
- * *n_nodes = node count; y == NULL: count only; PPP_ERR_CAPACITY if node_cap is too small.       */
+ * *n_nodes = node count; y == NULL: count only; PPP_ERR_CAPACITY if node_cap is too small.
+ * The list may name points that are not finite (a band never does: PassThrough drops them).  Such
+ * a point is on neither side of the plane and never a nearest neighbour.  For a NaN or infinite y
+ * or z that is the reference's own result: its (p - PlanePoint).dot((1,0,0)) is NaN.  For x = +-inf
+ * with finite y and z the reference would put the point on a side and hand it to FLANN as a query,
+ * whose answer is not defined; it is dropped here as well.                                      */
 int ppp_insert_point(ppp_cloud* cloud, const int32_t* indices, int64_t m, float plane_x, int pairing_mode,
                      double* y, double* x, double* z, int64_t node_cap, int64_t* n_nodes);
 

@@ -364,7 +364,7 @@ __device__ int2 nn_side(const GridView& g, const float4* __restrict__ xyz4, floa
         consider(c.x, c.y, c.z, __float_as_int(c.w), e);
       } else {
         float4 c = __ldg(xyz4 + e);
-        consider(c.x, c.y, c.z, e, -1);
+        if (c.w == c.w) consider(c.x, c.y, c.z, e, -1);   // w = NaN: not finite (explicit lists), on neither side
       }
     }
   }
@@ -432,7 +432,9 @@ __global__ void __launch_bounds__(1024) k_contour(ContourParams P, int smem_cap)
   {
     int cl = 0, cr = 0;
     for (int i = threadIdx.x; i < B; i += (int)blockDim.x) {
-      float d = __fsub_rn(__ldg(&P.xyz4[band[i]].x), plane);  // (point - PlanePoint).dot((1,0,0))
+      const float4 p = __ldg(P.xyz4 + band[i]);
+      // (point - PlanePoint).dot((1,0,0)); a non-finite point (w = NaN; explicit lists only) is on neither side
+      float d = p.w == p.w ? __fsub_rn(p.x, plane) : 0.0f;
       cl += d > 0.0f;
       cr += d < 0.0f;
     }
@@ -455,7 +457,8 @@ __global__ void __launch_bounds__(1024) k_contour(ContourParams P, int smem_cap)
       bool isL = false, isR = false;
       if (i < B) {
         idx = band[i];
-        float d = __fsub_rn(__ldg(&P.xyz4[idx].x), plane);
+        const float4 p = __ldg(P.xyz4 + idx);
+        float d = p.w == p.w ? __fsub_rn(p.x, plane) : 0.0f;
         isL = d > 0.0f;
         isR = d < 0.0f;
       }
@@ -605,7 +608,8 @@ __global__ void __launch_bounds__(PAIR_WARPS * 32) k_pair_nodes(PairParams P) {
       s = l;
       float4 rec;
       member_handle(P, m, &rec);
-      isL = __fsub_rn(rec.x, __ldg(P.planes + s)) > 0.0f;
+      // index lists hold packed records, whose w = NaN marks a non-finite point (explicit lists only): neither side
+      isL = (P.by_pos || rec.w == rec.w) && __fsub_rn(rec.x, __ldg(P.planes + s)) > 0.0f;
       if (!isL) { P.keys[m] = PPP_KEY_INF; P.ys[m] = 0.f; P.zs[m] = 0.f; }
     }
     const unsigned bal = __ballot_sync(0xffffffffu, isL);
