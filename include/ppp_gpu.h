@@ -204,6 +204,38 @@ int ppp_coverage_mark_radii(ppp_cloud* cloud, const float* q, size_t nq, size_t 
 int ppp_mls_smooth(ppp_cloud* cloud, double radius, int order, void* points_out, size_t out_stride_bytes,
                    float* normals_out, int32_t* src_index_out, int64_t* n_out);
 
+/* smooth() with the results left in device memory, on one GPU or on the x-slabs of a multi-GPU exchange
+ * (src/Path_Generation.cpp:340-360, as ppp_mls_smooth; same radius, order and contract).  Every point gets one
+ * record of row_stride_bytes = 32: {x, y, z, flag, nx, ny, nz, curvature}, flag 1.0f where the point has an output
+ * row; other records (fewer than 3 neighbours, a non-finite point) have flag 0 and NaN elsewhere.  Every record is
+ * written by every call.
+ *  - plain cloud: record i of rows_dev (16-byte aligned) is point i's.
+ *  - slab from ppp_exch_attach / ppp_exch_finish_attach: rows_dev is ignored; only owned rows are queries (halo copies
+ *    are candidates only) and each record is stored into its HOME rank's buffer (ppp_exch_home_normals, record =
+ *    global index - starts[home]), over NVLink where the home is another GPU.  ppp_exch_results_signal / _wait with
+ *    PPP_EXCH_NORMALS cover these records.  PPP_ERR_INVALID if the exchange was created with 16-byte normal records,
+ *    or if the halo any rank's phases were given is narrower than ppp_mls_halo(radius, largest finite |x| of the
+ *    cloud) (the ranks publish their halos with the exchange, so every rank refuses together). PPP_ERR_INVALID too if
+ *    the slab's row map was cleared.
+ * Does not synchronise.  PPP_ERR_INVALID for the radii and orders ppp_mls_smooth refuses. */
+int ppp_dev_mls_smooth(ppp_cloud* cloud, double radius, int order, void* rows_dev, size_t row_stride_bytes);
+/* Records [0, n) of rows_dev (device memory, e.g. a home buffer) -> rows in ascending record order: *n_rows = rows
+ * with flag 1.  Counting call: points_out, normals_out and src_index_out all NULL.  Filling call: rows
+ * [row_base, row_base + *n_rows) of points_out (out_stride_bytes; x, y, z from the records, every other field from
+ * src_dev, the source records of stride src_stride_bytes = out_stride_bytes, when it is not NULL), normals_out
+ * (nullable, 16 bytes a row: nx, ny, nz, curvature) and src_index_out (src_index_base + record number).  The outputs
+ * may be device memory or mapped host memory (ppp_host_register, ppp_host_alloc).  PPP_ERR_CAPACITY when
+ * row_base + *n_rows > cap_rows (*n_rows is still reported).  Synchronises: after a filling call the rows are in
+ * place.  Ranks of an exchange compact their
+ * home ranges with row_base = the rows of the lower ranks: together the ranks write ppp_mls_smooth's rows.       */
+int ppp_dev_mls_compact(ppp_ctx* ctx, const void* rows_dev, int64_t n, const void* src_dev, size_t src_stride_bytes,
+                        int64_t src_index_base, int64_t row_base, void* points_out, size_t out_stride_bytes,
+                        float* normals_out, int32_t* src_index_out, int64_t cap_rows, int64_t* n_rows);
+/* The exchange halo an MLS call of this radius needs on a cloud whose finite x lie within [-x_abs_max, x_abs_max]:
+ * the smallest float t with fl32(t * t) >= (float)(radius * radius), plus 2^-44 * (x_abs_max + t + 1) for the double
+ * rounding of the exchange's cut positions (derivation in csrc/mls.cu).  NaN for a radius ppp_mls_smooth refuses. */
+double ppp_mls_halo(double radius, double x_abs_max);
+
 /* estimate_normal() followed by the plane sweep, as one call: what SectPath-derived GenPath does
  * (src/Path_Alg/path_dynamic_alg.cpp:343-366: estimate_normal(); kdtree.setInputCloud; sweep).
  * Exactly the results of ppp_normals_knn (k >= 1, radius = 0) or ppp_normals_radius (k = 0,

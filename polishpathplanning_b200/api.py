@@ -143,6 +143,19 @@ class Context:
     def host_unregister(self, host_ptr):
         check(self.lib.ppp_host_unregister(_vp(host_ptr)))
 
+    def dev_mls_compact(self, rows_ptr, n, src_ptr=None, src_stride_bytes=0, src_index_base=0, row_base=0, points_ptr=None,
+                        out_stride_bytes=32, normals_ptr=None, src_index_ptr=None, cap_rows=0):
+        """ppp_dev_mls_compact: MLS records [0, n) at rows_ptr -> output rows in source order from row_base on.
+        Without points_ptr / src_index_ptr only counts.  Returns the number of rows of the range (raises PPPError with
+        status PPP_ERR_CAPACITY when row_base + that number exceeds cap_rows)."""
+        m = C.c_int64(0)
+        check(self.lib.ppp_dev_mls_compact(self._h, _vp(rows_ptr) if rows_ptr else None, int(n), _vp(src_ptr) if src_ptr else None,
+                                           int(src_stride_bytes), int(src_index_base), int(row_base),
+                                           _vp(points_ptr) if points_ptr else None, int(out_stride_bytes),
+                                           _vp(normals_ptr) if normals_ptr else None,
+                                           _vp(src_index_ptr) if src_index_ptr else None, int(cap_rows), C.byref(m)))
+        return m.value
+
     def pinned_empty(self, shape, dtype):
         """numpy array over pinned host memory from ppp_host_alloc (freed with the array)."""
         dtype = np.dtype(dtype)
@@ -401,6 +414,12 @@ class Cloud:
         vp = np.asarray(viewpoint, np.float32)
         check(self.lib.ppp_dev_normals_radius(self._h, float(r), vp.ctypes.data_as(_lib._f32p), flags, int(first),
                                               int(count), _vp(normals_ptr), int(normal_stride_bytes)))
+
+    def dev_mls_smooth(self, radius=15.0, order=3, rows_ptr=None, row_stride_bytes=32):
+        """ppp_dev_mls_smooth: one 32-byte record {x, y, z, flag, nx, ny, nz, curvature} per point into the device buffer
+        rows_ptr (plain cloud) or, on a slab from Exchange.attach, into the home ranks' buffers.  Does not synchronise."""
+        check(self.lib.ppp_dev_mls_smooth(self._h, float(radius), int(order), _vp(rows_ptr) if rows_ptr else None,
+                                          int(row_stride_bytes)))
 
     def dev_set_normal_row_map(self, map_ptr):
         """Device int32 map row -> record of the normals buffer (negative: skip); None = identity."""

@@ -972,4 +972,56 @@ int ppp_mls_smooth(ppp_cloud* c, double radius, int order, void* points_out, siz
   return PPP_OK;
 }
 
+double ppp_mls_halo(double radius, double x_abs_max) { return mls_halo(radius, x_abs_max); }
+
+// ppp_mls_smooth's per-point part with the results left in device memory: one 32-byte record per point, by original
+// index, or on an exchange slab to the home ranks (only owned rows are queries there).  Does not synchronise.
+int ppp_dev_mls_smooth(ppp_cloud* c, double radius, int order, void* rows_dev, size_t row_stride_bytes) {
+  REQUIRE(c, "cloud is NULL");
+  REQUIRE(radius > 0 && std::isfinite((float)(radius * radius)), "radius must be > 0 with a finite float32 square");
+  REQUIRE(order >= 0 && order <= 3, "order must be 0..3");
+  REQUIRE(row_stride_bytes == 32, "records are 32 bytes: {x, y, z, flag, nx, ny, nz, curvature}");
+  if (c->route) {
+    REQUIRE(c->nmap, "an exchange slab needs its row map (ppp_dev_set_normal_row_map(NULL) cleared it)");
+    REQUIRE(c->ex_home_bytes == 32, "the exchange keeps 16-byte home records; MLS records need an exchange created with 32");
+    const double need = mls_halo(radius, c->ex_xmag);
+    if (!(c->ex_halo >= need)) {
+      ppp_set_error("ppp_dev_mls_smooth: the exchange halo %.17g is narrower than the %.17g radius %.17g needs (ppp_mls_halo)",
+                    c->ex_halo, need, radius);
+      return PPP_ERR_INVALID;
+    }
+  } else {
+    REQUIRE(rows_dev || c->n == 0, "rows_dev is NULL");
+    REQUIRE((uintptr_t)rows_dev % 16 == 0, "rows_dev must be 16-byte aligned");
+  }
+  LOCK(c->ctx);
+  PPP_CUDA(cudaSetDevice(c->ctx->device));
+  return mls_smooth_records(c, radius, order, (float*)rows_dev);
+}
+
+// Records [0, n) -> rows in source order (see the header).  Synchronises once.
+int ppp_dev_mls_compact(ppp_ctx* ctx, const void* rows_dev, int64_t n, const void* src_dev, size_t src_stride_bytes,
+                        int64_t src_index_base, int64_t row_base, void* points_out, size_t out_stride_bytes, float* normals_out,
+                        int32_t* src_index_out, int64_t cap_rows, int64_t* n_rows) {
+  REQUIRE(ctx && n_rows, "NULL argument");
+  *n_rows = 0;
+  REQUIRE(n >= 0 && (rows_dev || n == 0) && (uintptr_t)rows_dev % 16 == 0, "rows_dev: n 16-byte aligned records");
+  REQUIRE(src_index_base >= 0 && src_index_base + n <= 2147483647ll, "source indices must fit int32");
+  const bool fill = points_out || src_index_out || normals_out;
+  if (fill) {
+    REQUIRE(points_out && src_index_out, "points_out and src_index_out are both needed to fill");
+    REQUIRE(out_stride_bytes >= 12 && out_stride_bytes % 4 == 0, "output stride must be >= 12 and a multiple of 4");
+    REQUIRE(!src_dev || src_stride_bytes == out_stride_bytes, "source records must have the output stride");
+    REQUIRE((uintptr_t)normals_out % 16 == 0, "normals_out must be 16-byte aligned");
+    REQUIRE(row_base >= 0 && cap_rows >= 0, "bad row base / capacity");
+  }
+  LOCK(ctx);
+  PPP_CUDA(cudaSetDevice(ctx->device));
+  PPP_TRY(mls_compact_launch(ctx, (const float*)rows_dev, n, fill ? (const float*)src_dev : nullptr, (int)(out_stride_bytes / 4),
+                            (int32_t)src_index_base, row_base, fill ? (float*)points_out : nullptr, (float4*)normals_out,
+                            src_index_out, cap_rows, n_rows));
+  if (fill) PPP_CUDA(cudaStreamSynchronize(ctx->stream));   // the rows are in place (host memory included) on return
+  return PPP_OK;
+}
+
 }  // extern "C"

@@ -30,6 +30,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include "ppp_device.cuh"
@@ -43,7 +44,7 @@ constexpr int EX_THREADS = 256;
 constexpr unsigned long long EX_TIMEOUT_NS = 10ull * 1000 * 1000 * 1000;
 
 struct ExLayout {
-  size_t flags, mm, hist, cnt, recv, home, nodes, node_off_bytes, node_arr_bytes, node_region, total;
+  size_t flags, mm, hist, cnt, halo, recv, home, nodes, node_off_bytes, node_arr_bytes, node_region, total;
 };
 
 inline size_t a256(size_t v) { return (v + 255) / 256 * 256; }
@@ -55,6 +56,7 @@ ExLayout ex_layout(int world, int64_t cap_recv, int64_t cap_home, int home_strid
   L.mm = at;    at += a256((size_t)2 * PPP_MAX_RANKS * sizeof(float4));       // [parity][src] = {min, max, finite lo, finite hi}
   L.hist = at;  at += a256((size_t)PPP_MAX_RANKS * EX_BINS * sizeof(int32_t)); // [src][bin]
   L.cnt = at;   at += a256((size_t)2 * PPP_MAX_RANKS * PPP_MAX_RANKS * sizeof(int32_t));  // [0]: records, [1]: owned; [src][dst]
+  L.halo = at;  at += a256((size_t)PPP_MAX_RANKS * sizeof(double));          // [src]: the halo src cut its copies with
   L.recv = at;  at += a256((size_t)std::max<int64_t>(cap_recv, 1) * sizeof(float4));
   L.home = at;  at += a256((size_t)std::max<int64_t>(cap_home, 1) * home_stride_f * sizeof(float));
   L.node_off_bytes = a256(((size_t)S_cap + 1) * sizeof(int64_t));
@@ -70,7 +72,7 @@ ExLayout ex_layout(int world, int64_t cap_recv, int64_t cap_home, int home_strid
 struct ExView {
   int rank, world;
   unsigned char* arena[PPP_MAX_RANKS];
-  unsigned long long off_flags, off_mm, off_hist, off_cnt, off_recv;
+  unsigned long long off_flags, off_mm, off_hist, off_cnt, off_halo, off_recv;
   long long cap_recv;
 };
 
@@ -83,6 +85,7 @@ struct ExScratch {
   int32_t cutbin[PPP_MAX_RANKS + 1];
   double cutx[PPP_MAX_RANKS + 1];
   double gmin, gmax, inv;           // global finite x-range, bins per unit
+  double halo_min;                  // narrowest halo any rank cut its copies with this step
   int32_t sendcnt[PPP_MAX_RANKS], sendown[PPP_MAX_RANKS];
   // summary fetched by the host after the exchange
   long long n_local, n_owned;
@@ -408,6 +411,7 @@ __global__ void __launch_bounds__(EX_THREADS) k_ex_count(ExView V, const float* 
     tab[V.rank * PPP_MAX_RANKS + dst] = *(volatile int32_t*)&sc->sendcnt[dst];
     tab[PPP_MAX_RANKS * PPP_MAX_RANKS + V.rank * PPP_MAX_RANKS + dst] = *(volatile int32_t*)&sc->sendown[dst];
   }
+  if ((int)threadIdx.x < world) reinterpret_cast<double*>(V.arena[threadIdx.x] + V.off_halo)[V.rank] = halo;
   __syncthreads();
   if (threadIdx.x < PPP_MAX_RANKS) { sc->sendown[threadIdx.x] = 0; sc->sendcnt[threadIdx.x] = 0; }
   ex_publish(V, 2, step);
@@ -509,7 +513,13 @@ __global__ void __launch_bounds__(256) k_ex_rowmap(ExView V, ExScratch* sc, int3
       n_local = V.cap_recv;
       if (blockIdx.x == 0) atomicMax(&sc->err, 2);
     }
-    if (blockIdx.x == 0) { sc->n_local = n_local; sc->n_owned = n_owned; }
+    if (blockIdx.x == 0) {
+      sc->n_local = n_local; sc->n_owned = n_owned;
+      const double* hs = reinterpret_cast<const double*>(V.arena[V.rank] + V.off_halo);
+      double hm = *(volatile const double*)hs;
+      for (int s = 1; s < V.world; s++) hm = fmin(hm, *(volatile const double*)(hs + s));
+      sc->halo_min = hm;
+    }
     s_n[0] = n_local;
   }
   __syncthreads();
@@ -550,7 +560,8 @@ struct ppp_exch {
   const float* raw = nullptr;
   int64_t n = 0;
   int sf = 0, vec_ok = 0, ntiles = 0;
-  double halo = 0;
+  double halo = 0;     // the narrowest halo any rank's phases were given this step (checked by ppp_dev_mls_smooth)
+  double xmag = 0;     // largest finite |x| of the step's cloud (ppp_dev_mls_smooth checks the halo against it)
   int64_t n_local = 0;
 };
 
@@ -567,7 +578,7 @@ static void ex_refresh_view(ppp_exch* ex) {
   ExView& V = ex->V;
   V.rank = ex->rank; V.world = ex->world;
   for (int r = 0; r < PPP_MAX_RANKS; r++) V.arena[r] = r < ex->world ? ex->peer[r] : nullptr;
-  V.off_flags = ex->L.flags; V.off_mm = ex->L.mm; V.off_hist = ex->L.hist; V.off_cnt = ex->L.cnt; V.off_recv = ex->L.recv;
+  V.off_flags = ex->L.flags; V.off_mm = ex->L.mm; V.off_hist = ex->L.hist; V.off_cnt = ex->L.cnt; V.off_halo = ex->L.halo; V.off_recv = ex->L.recv;
   V.cap_recv = ex->cap_recv;
 }
 
@@ -735,6 +746,7 @@ int ppp_exch_phase(ppp_exch* ex, int phase, const void* chunk_dev, int64_t n, si
     return PPP_OK;
   }
   EX_REQUIRE(raw == ex->raw && n == ex->n, "phases of one step must be given the same chunk");
+  ex->halo = std::min(ex->halo, halo);
   if (phase == 1) {
     PPP_LAUNCH(ctx, "ex_wait", k_ex_wait, 1, 32, 0, ex->V, 0, ex->step, -1, ex->sc);
     // two 1024-thread blocks per SM: every block ends with one atomic per non-empty bin
@@ -776,7 +788,7 @@ int ppp_exch_finish(ppp_exch* ex, int64_t* n_local, int64_t* n_owned, double* cu
   // summary: one fetch of the scratch block from the cut positions to the error word
   struct Summary {
     double cutx[PPP_MAX_RANKS + 1];
-    double gmin, gmax, inv;
+    double gmin, gmax, inv, halo_min;
     int32_t sendcnt[PPP_MAX_RANKS], sendown[PPP_MAX_RANKS];
     long long n_local, n_owned;
     int32_t err, pad;
@@ -792,6 +804,8 @@ int ppp_exch_finish(ppp_exch* ex, int64_t* n_local, int64_t* n_owned, double* cu
     return tail.err == 1 ? PPP_ERR_CUDA : PPP_ERR_CAPACITY;
   }
   ex->n_local = tail.n_local;
+  ex->xmag = std::max(std::fabs(mid.gmin), std::fabs(mid.gmax));
+  ex->halo = std::min(ex->halo, sum.halo_min);
   if (n_local) *n_local = tail.n_local;
   if (n_owned) *n_owned = tail.n_owned;
   if (cuts) for (int r = 0; r <= ex->world; r++) cuts[r] = mid.cutx[r];
@@ -813,6 +827,7 @@ int ppp_exch_attach(ppp_exch* ex, int to_rank0, ppp_cloud** out) {
   PPP_TRY(ppp_dev_cloud_attach(ex->ctx, ex->arena + ex->L.recv, (size_t)ex->n_local, 16, out));
   (*out)->nmap = ex->rowmap;
   (*out)->route = ex->route;
+  (*out)->ex_halo = ex->halo; (*out)->ex_xmag = ex->xmag; (*out)->ex_home_bytes = ex->home_sf * 4;
   if (to_rank0) {
     unsigned char* reg = ex->peer[0] + ex->L.nodes + (size_t)ex->rank * ex->L.node_region;
     PPP_TRY(ppp_dev_set_contour_offsets_buffer(*out, (int64_t*)reg, (int64_t)ex->S_cap + 1));
@@ -838,7 +853,7 @@ int ppp_exch_finish_attach(ppp_exch* ex, int to_rank0, int64_t* n_local, int64_t
   PPP_CHECK_LAUNCH();
   struct Summary {
     double cutx[PPP_MAX_RANKS + 1];
-    double gmin, gmax, inv;
+    double gmin, gmax, inv, halo_min;
     int32_t sendcnt[PPP_MAX_RANKS], sendown[PPP_MAX_RANKS];
     long long n_local, n_owned;
     int32_t err, pad;
@@ -859,12 +874,15 @@ int ppp_exch_finish_attach(ppp_exch* ex, int to_rank0, int64_t* n_local, int64_t
   }
   if (st != PPP_OK) { ppp_cloud_free(c); return st; }
   ex->n_local = sum.n_local;
+  ex->xmag = std::max(std::fabs(sum.gmin), std::fabs(sum.gmax));
+  ex->halo = std::min(ex->halo, sum.halo_min);
   if (n_local) *n_local = sum.n_local;
   if (n_owned) *n_owned = sum.n_owned;
   if (cuts) for (int r = 0; r <= ex->world; r++) cuts[r] = sum.cutx[r];
   if (x_range) { x_range[0] = sum.gmin; x_range[1] = sum.gmax; }
   c->nmap = ex->rowmap;
   c->route = ex->route;
+  c->ex_halo = ex->halo; c->ex_xmag = ex->xmag; c->ex_home_bytes = ex->home_sf * 4;
   if (to_rank0) {
     unsigned char* reg = ex->peer[0] + ex->L.nodes + (size_t)ex->rank * ex->L.node_region;
     st = ppp_dev_set_contour_offsets_buffer(c, (int64_t*)reg, (int64_t)ex->S_cap + 1);

@@ -15,6 +15,12 @@
 //   the SIMPLE projection.
 // The contract is a tolerance against the FMA-free CPU oracle (DESIGN.md §2), so the accumulations use
 // explicit FMAs although the library is built with --fmad=false.
+//
+// Device records and several GPUs (ppp_dev_mls_smooth): each query stores one 32-byte record
+// {x, y, z, flag, nx, ny, nz, curvature} instead of the compacted rows, by original index on a plain cloud and, on
+// a slab attached by ppp_exch_attach, through the cloud's route into the home rank's buffer (as store_normal does
+// for the normal estimators).  Only owned rows (nmap >= 0) are queries there; halo copies are candidates only.
+// ppp_dev_mls_compact turns a range of records into rows in source order at a caller-given row base.
 #include <cmath>
 
 #include "ppp_device.cuh"
@@ -32,6 +38,14 @@ struct MlsParams {
   float4* xyz_out;      // by original index: smoothed x, y, z
   float4* nrm_out;      // by original index: nx, ny, nz, curvature (nullptr: not wanted)
   int32_t* emit;        // by original index: 1 = the point has an output row (zero-filled by the caller)
+};
+
+// Record mode (k_mls<ORDER, true>; MlsParams' xyz_out / nrm_out / emit unused): every query stores its 32-byte record.
+// A parameter of its own, so that the single-GPU instance is compiled from MlsParams alone.
+struct MlsRecords {
+  float* rec;                    // records by original index, or unused with a route
+  const int32_t* nmap;           // slab row -> global index, negative for halo copies (nullptr: every row is a query)
+  const NormalRoute* route;      // with nmap: the record goes to the home rank of the global index
 };
 
 // Candidates of the (2R+1)^2 cell block around (cu, cv) that lie strictly within the radius, row by row;
@@ -146,8 +160,8 @@ __device__ __forceinline__ double dot3(const double a[3], const double b[3]) {
 template <int D>
 __host__ __device__ constexpr int mono(int a, int b) { return a * (D + 1) - a * (a - 1) / 2 + b; }
 
-template <int ORDER>
-__global__ void __launch_bounds__(128) k_mls(MlsParams P) {
+template <int ORDER, bool RECORDS>
+__global__ void __launch_bounds__(128) k_mls(MlsParams P, MlsRecords Q) {
   pdl_prologue();
   constexpr int NC = (ORDER + 1) * (ORDER + 2) / 2;   // coefficients (10 at order 3)
   constexpr int D2 = ORDER > 1 ? 2 * ORDER : 0;
@@ -163,8 +177,9 @@ __global__ void __launch_bounds__(128) k_mls(MlsParams P) {
     qx = p.x; qy = p.y; qz = p.z;
     row = __float_as_int(p.w);
     valid = P.choice == nullptr || __ldg(P.choice + row) == P.my_proj;
+    if (RECORDS && Q.nmap) valid = valid && __ldg(Q.nmap + row) >= 0;   // halo copies are candidates, never queries
   }
-  if (P.choice && !__any_sync(0xffffffffu, valid)) return;
+  if ((P.choice || (RECORDS && Q.nmap)) && !__any_sync(0xffffffffu, valid)) return;
   int cu = 0, cv = 0;
   if (valid) {
     cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
@@ -329,6 +344,19 @@ __global__ void __launch_bounds__(128) k_mls(MlsParams P) {
       }
     }
   }
+  if constexpr (RECORDS) {   // every query's record is written, so nothing of an earlier call survives in the buffer
+    if (!valid) return;
+    PPP_DEV_ASSERT(row >= 0);
+    float o[8];
+    if (emit) {
+      o[0] = (float)outp[0]; o[1] = (float)outp[1]; o[2] = (float)outp[2]; o[3] = 1.0f;
+      o[4] = (float)outn[0]; o[5] = (float)outn[1]; o[6] = (float)outn[2]; o[7] = (float)curvature;
+    } else {
+      mls_no_row(o);
+    }
+    store_mls_record(Q.rec, Q.nmap, row, o, Q.route);
+    return;
+  }
   if (!emit) return;
   PPP_DEV_ASSERT(row >= 0);
   P.xyz_out[row] = make_float4((float)outp[0], (float)outp[1], (float)outp[2], 0.0f);
@@ -336,48 +364,93 @@ __global__ void __launch_bounds__(128) k_mls(MlsParams P) {
   P.emit[row] = 1;
 }
 
-// Compaction: row o = pos[i] of the output gets point i's results (pos = exclusive scan of emit).
+// Compaction: row row_base + pos[i] of the output gets point i's results (pos = exclusive scan of emit).  Inputs
+// xyz (x, y, z) and nrm (nx, ny, nz, curvature) are read as float4 at a stride of in_sf floats; output points are
+// records of out_sf floats whose other fields come from the source records src_rec (nullptr: x, y, z only).
 __global__ void __launch_bounds__(256) k_mls_scatter(const int32_t* __restrict__ emit, const int32_t* __restrict__ pos,
-                                                     int64_t n, const float4* __restrict__ xyz, const float4* __restrict__ nrm,
-                                                     float* __restrict__ xyz_c, float4* __restrict__ nrm_c,
-                                                     int32_t* __restrict__ src_c) {
+                                                     int64_t n, const float* __restrict__ xyz, const float* __restrict__ nrm, int in_sf,
+                                                     const float* __restrict__ src_rec, int out_sf, float* __restrict__ xyz_c,
+                                                     float4* __restrict__ nrm_c, int32_t* __restrict__ src_c, int64_t row_base,
+                                                     int32_t idx_base) {
   pdl_prologue();
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n || !__ldg(emit + i)) return;
-  const int32_t o = __ldg(pos + i);
-  PPP_DEV_ASSERT(o >= 0 && o < __ldg(pos + n) && (int64_t)o <= i);
-  const float4 p = __ldg(xyz + i);
-  xyz_c[3 * (int64_t)o] = p.x; xyz_c[3 * (int64_t)o + 1] = p.y; xyz_c[3 * (int64_t)o + 2] = p.z;
-  if (nrm_c) nrm_c[o] = __ldg(nrm + i);
-  src_c[o] = (int32_t)i;
+  const int32_t at = __ldg(pos + i);
+  PPP_DEV_ASSERT(at >= 0 && at < __ldg(pos + n) && (int64_t)at <= i);
+  const int64_t o = row_base + at;
+  const float4 p = __ldg(reinterpret_cast<const float4*>(xyz + i * in_sf));
+  float* d = xyz_c + o * out_sf;
+  if (src_rec)
+    for (int k = 3; k < out_sf; k++) d[k] = __ldg(src_rec + i * out_sf + k);
+  d[0] = p.x; d[1] = p.y; d[2] = p.z;
+  if (nrm_c) nrm_c[o] = __ldg(reinterpret_cast<const float4*>(nrm + i * in_sf));
+  src_c[o] = idx_base + (int32_t)i;
 }
 
-template <int ORDER>
-int launch_mls_order(ppp_ctx* ctx, const MlsParams& P) {
+// Output flags of n records: emit[i] = 1 where record i has a row.
+__global__ void __launch_bounds__(256) k_mls_flags(const float* __restrict__ rec, int64_t n, int32_t* __restrict__ emit) {
+  pdl_prologue();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) emit[i] = __ldg(rec + i * 8 + 3) == 1.0f ? 1 : 0;
+}
+
+// Records of the points that are not indexed (a non-finite coordinate): no row.
+__global__ void __launch_bounds__(256) k_mls_default_rows(const float4* __restrict__ xyz4, int64_t n, float* rec,
+                                                          const int32_t* __restrict__ nmap, const NormalRoute* __restrict__ route) {
+  pdl_prologue();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float4 p = __ldg(xyz4 + i);
+  if (p.w == p.w) return;
+  float o[8];
+  mls_no_row(o);
+  store_mls_record(rec, nmap, i, o, route);
+}
+
+template <int ORDER, bool RECORDS>
+int launch_mls_order(ppp_ctx* ctx, const MlsParams& P, const MlsRecords& Q) {
   static const char* names[4] = {"mls_plane", "mls_plane", "mls_order2", "mls_order3"};
-  auto kern = k_mls<ORDER>;
+  auto kern = k_mls<ORDER, RECORDS>;
   const unsigned blocks = (unsigned)((P.nq + 127) / 128);
-  PPP_LAUNCH(ctx, names[ORDER], kern, blocks, 128, 0, P);
+  PPP_LAUNCH(ctx, names[ORDER], kern, blocks, 128, 0, P, Q);
   PPP_CHECK_LAUNCH();
   return PPP_OK;
 }
 
+// out: the output fields of MlsParams (xyz_out ... route); the rest is filled in here.
+template <bool RECORDS>
 int launch_mls(ppp_ctx* ctx, const GridStore& gs, double radius, int order, const unsigned char* choice, int my_proj,
-               float4* xyz, float4* nrm, int32_t* emit) {
+               const MlsParams& out, const MlsRecords& Q) {
   if (gs.v.n_sorted <= 0) return PPP_OK;
-  MlsParams P{};
+  MlsParams P = out;
   P.g = gs.v;
   P.nq = gs.v.n_sorted;
   P.r2 = (float)(radius * radius);   // [upstream] pcl::KdTreeFLANN::radiusSearch
   P.R = radius_rings(gs.v, std::sqrt((double)P.r2));
   P.inv_sq_radius = 1.0 / (radius * radius);
   P.choice = choice; P.my_proj = my_proj;
-  P.xyz_out = xyz; P.nrm_out = nrm; P.emit = emit;
   switch (order) {
-    case 0: case 1: return launch_mls_order<1>(ctx, P);
-    case 2: return launch_mls_order<2>(ctx, P);
-    default: return launch_mls_order<3>(ctx, P);
+    case 0: case 1: return launch_mls_order<1, RECORDS>(ctx, P, Q);
+    case 2: return launch_mls_order<2, RECORDS>(ctx, P, Q);
+    default: return launch_mls_order<3, RECORDS>(ctx, P, Q);
   }
+}
+
+// k_mls over every indexed point of the cloud (through the multi-projection index where the cloud needs it).
+template <bool RECORDS>
+int mls_over_cloud(ppp_cloud* c, double radius, int order, const MlsParams& out, const MlsRecords& Q) {
+  const double h = cloud_cell_for_radius(c, radius);
+  GridStore* g;
+  PPP_TRY(cloud_get_grid(c, h, &g));
+  PPP_TRY(cloud_decide_projection(c, *g));
+  if (c->mp_state == 1) {
+    // not a height field: every point is answered through the projection that spreads its block out best
+    MPSet* mp;
+    PPP_TRY(cloud_get_mp(c, h, 2, &mp));   // cloud_cell_for_radius sizes the cells so that two rings cover the radius
+    for (int p = 0; p < 3; p++) PPP_TRY(launch_mls<RECORDS>(c->ctx, *mp->g[p], radius, order, mp->choice, p, out, Q));
+    return PPP_OK;
+  }
+  return launch_mls<RECORDS>(c->ctx, *g, radius, order, nullptr, 0, out, Q);
 }
 
 }  // namespace
@@ -390,10 +463,6 @@ int mls_smooth_launch(ppp_cloud* c, double radius, int order, float* xyz_c, floa
     return PPP_ERR_UNSUPPORTED;
   }
   if (c->n == 0) return PPP_OK;
-  const double h = cloud_cell_for_radius(c, radius);
-  GridStore* g;
-  PPP_TRY(cloud_get_grid(c, h, &g));
-  PPP_TRY(cloud_decide_projection(c, *g));
   float4 *xyz = nullptr, *nrm = nullptr;
   int32_t *emit = nullptr, *pos = nullptr;
   PPP_TRY(dev_alloc(ctx, &xyz, (size_t)c->n));
@@ -401,19 +470,15 @@ int mls_smooth_launch(ppp_cloud* c, double radius, int order, float* xyz_c, floa
   PPP_TRY(dev_alloc(ctx, &emit, (size_t)c->n));
   PPP_TRY(dev_alloc(ctx, &pos, (size_t)c->n + 1));
   PPP_CUDA(cudaMemsetAsync(emit, 0, (size_t)c->n * sizeof(int32_t), ctx->stream));
-  if (c->mp_state == 1) {
-    // not a height field: every point is answered through the projection that spreads its block out best
-    MPSet* mp;
-    PPP_TRY(cloud_get_mp(c, h, 2, &mp));   // cloud_cell_for_radius sizes the cells so that two rings cover the radius
-    for (int p = 0; p < 3; p++) PPP_TRY(launch_mls(ctx, *mp->g[p], radius, order, mp->choice, p, xyz, nrm, emit));
-  } else {
-    PPP_TRY(launch_mls(ctx, *g, radius, order, nullptr, 0, xyz, nrm, emit));
-  }
+  MlsParams out{};
+  out.xyz_out = xyz; out.nrm_out = nrm; out.emit = emit;
+  PPP_TRY(mls_over_cloud<false>(c, radius, order, out, MlsRecords{}));
   PPP_TRY(scan_exclusive_i32(ctx, emit, pos, c->n));
   {
     const unsigned blocks = (unsigned)((c->n + 255) / 256);
     PPP_LAUNCH(ctx, "mls_scatter", k_mls_scatter, blocks, 256, 0, (const int32_t*)emit, (const int32_t*)pos, c->n,
-               (const float4*)xyz, (const float4*)nrm, xyz_c, nrm_c, src_c);
+               (const float*)xyz, (const float*)nrm, 4, (const float*)nullptr, 3, xyz_c, nrm_c, src_c, (int64_t)0,
+               (int32_t)0);
     PPP_CHECK_LAUNCH();
   }
   int32_t total = 0;
@@ -422,4 +487,73 @@ int mls_smooth_launch(ppp_cloud* c, double radius, int order, float* xyz_c, floa
   dev_free(ctx, xyz); dev_free(ctx, nrm); dev_free(ctx, emit); dev_free(ctx, pos);
   *n_rows = total;
   return PPP_OK;
+}
+
+int mls_smooth_records(ppp_cloud* c, double radius, int order, float* rec) {
+  ppp_ctx* ctx = c->ctx;
+  if (c->n == 0) return PPP_OK;
+  MlsRecords out{};
+  out.rec = rec; out.nmap = c->nmap; out.route = c->nmap ? c->route : nullptr;
+  PPP_TRY(mls_over_cloud<true>(c, radius, order, MlsParams{}, out));
+  if (c->n_finite < c->n) {   // non-finite points are not indexed: their records are written here
+    const unsigned blocks = (unsigned)((c->n + 255) / 256);
+    PPP_LAUNCH(ctx, "mls_default_rows", k_mls_default_rows, blocks, 256, 0, (const float4*)c->xyz4, c->n, rec, out.nmap, out.route);
+    PPP_CHECK_LAUNCH();
+  }
+  return PPP_OK;
+}
+
+int mls_compact_launch(ppp_ctx* ctx, const float* rec, int64_t n, const float* src_rec, int out_sf, int32_t idx_base,
+                       int64_t row_base, float* points_out, float4* normals_out, int32_t* src_out, int64_t cap_rows,
+                       int64_t* n_rows) {
+  *n_rows = 0;
+  if (n == 0) return PPP_OK;
+  int32_t *emit = nullptr, *pos = nullptr;
+  PPP_TRY(dev_alloc(ctx, &emit, (size_t)n));
+  PPP_TRY(dev_alloc(ctx, &pos, (size_t)n + 1));
+  const unsigned blocks = (unsigned)((n + 255) / 256);
+  PPP_LAUNCH(ctx, "mls_flags", k_mls_flags, blocks, 256, 0, rec, n, emit);
+  PPP_CHECK_LAUNCH();
+  PPP_TRY(scan_exclusive_i32(ctx, emit, pos, n));
+  int32_t total = 0;
+  PPP_TRY(fetch_small(ctx, pos + n, sizeof(int32_t), &total));
+  *n_rows = total;
+  if (points_out) {
+    if (row_base + total > cap_rows) {
+      ppp_set_error("ppp_dev_mls_compact: the output holds %lld rows, rows up to %lld are needed", (long long)cap_rows,
+                    (long long)(row_base + total));
+      dev_free(ctx, emit); dev_free(ctx, pos);
+      return PPP_ERR_CAPACITY;
+    }
+    PPP_LAUNCH(ctx, "mls_scatter", k_mls_scatter, blocks, 256, 0, (const int32_t*)emit, (const int32_t*)pos, n, rec, rec + 4, 8,
+               src_rec, out_sf, points_out, normals_out, src_out, row_base, idx_base);
+    PPP_CHECK_LAUNCH();
+  }
+  dev_free(ctx, emit); dev_free(ctx, pos);
+  return PPP_OK;
+}
+
+// The exchange halo that keeps every MLS neighbour of an owned point in that point's slab (ppp_mls_halo).
+//
+// A candidate c is a neighbour of the query q when d2 = fl(fl(fl(dx^2) + fl(dy^2)) + fl(dz^2)) < r2, with
+// dx = fl(q.x - c.x) and r2 = (float)(r * r) (d2_flann_x2, MlsParams::r2).
+//  1. Rounding is monotone and the added terms are >= 0, so d2 >= fl(dx^2).  Let t be the smallest float with
+//     fl(t * t) >= r2.  |dx| >= t would give fl(dx^2) >= fl(t * t) >= r2: a neighbour has |dx| < t.
+//  2. t is a float and float subtraction is monotone, so |fl(q.x - c.x)| < t needs |q.x - c.x| < t exactly.
+//  3. The exchange (exchange.cu, ex_dest_mask) owns a point by its histogram bin and copies c into slab o when
+//     (double)c.x < fl(cut[o+1] + halo) or (double)c.x >= fl(cut[o] - halo).  The bin, fl((x - gmin) * inv), and
+//     the cut, fl(gmin + span * bin / 1024), are each a few double roundings of quantities no larger than
+//     M + span <= 3 M (M = largest finite |x|), so an owned q lies within 12 * 2^-53 * M of its slab's limits,
+//     and fl(cut +- halo) moves the limit by at most 2^-53 * (M + halo).
+// So halo = t + 2^-44 * (M + t + 1) (2^-44 = 512 * 2^-53, the 1 covers the span floor of 1e-9 and M = 0) puts
+// every neighbour of every owned point into its slab.
+double mls_halo(double radius, double x_abs_max) {
+  if (!(radius > 0) || !std::isfinite((float)(radius * radius)) || !(x_abs_max >= 0) || !std::isfinite(x_abs_max))
+    return std::nan("");
+  const float r2 = (float)(radius * radius);
+  auto sq = [](float v) { return (float)((double)v * (double)v); };   // the product is exact in double: fl32(v * v)
+  float t = (float)std::sqrt((double)r2);
+  while (t > 0.0f && sq(std::nextafter(t, 0.0f)) >= r2) t = std::nextafter(t, 0.0f);
+  while (sq(t) < r2) t = std::nextafter(t, INFINITY);
+  return (double)t + 0x1p-44 * (x_abs_max + (double)t + 1.0);
 }

@@ -262,6 +262,32 @@ __device__ __forceinline__ void store_normal(float* base, const int32_t* __restr
   }
 }
 
+// MLS result record (ppp_dev_mls_smooth) of a point without an output row: flag 0, every other field NaN.
+__device__ __forceinline__ void mls_no_row(float o[8]) {
+#pragma unroll
+  for (int k = 0; k < 8; k++) o[k] = CUDART_NAN_F;
+  o[3] = 0.0f;
+}
+
+// Store one 32-byte MLS result record {x, y, z, flag, nx, ny, nz, curvature}: at base + 8 * row, or, with a map,
+// at the record of global index map[row] (negative: not stored) in its home rank's buffer when a route is given.
+__device__ __forceinline__ void store_mls_record(float* base, const int32_t* __restrict__ map, int64_t row, const float o[8],
+                                                 const NormalRoute* __restrict__ route) {
+  if (map) {
+    row = __ldg(map + row);
+    if (row < 0) return;
+  }
+  if (route) {
+    int r = 0;
+    while (r + 1 < route->world && row >= route->start[r + 1]) r++;
+    base = route->base[r];
+    row -= route->start[r];
+  }
+  float4* p = reinterpret_cast<float4*>(base + row * 8);
+  p[0] = make_float4(o[0], o[1], o[2], o[3]);
+  p[1] = make_float4(o[4], o[5], o[6], o[7]);
+}
+
 // Visit every indexed point whose cell lies in the square annulus R_prev < max(|du|,|dv|) <= R
 // around (cu, cv)  (R_prev = -1: the whole (2R+1)^2 block).  [ulo, uhi] optionally restricts the
 // visited cell columns (callers that only want points of an x-interval).

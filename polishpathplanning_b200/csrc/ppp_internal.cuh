@@ -178,6 +178,10 @@ struct ppp_cloud {
   int64_t* ext_off = nullptr;      // ppp_dev_set_contour_offsets_buffer
   int64_t ext_off_cap = 0;
   double *out_y = nullptr, *out_x = nullptr, *out_z = nullptr;  // where the last call wrote the nodes
+  // an exchange slab (ppp_exch_attach): the halo it was cut with, the largest finite |x| of the whole cloud and the
+  // record stride of the home buffers, which ppp_dev_mls_smooth checks before it delivers records there
+  double ex_halo = 0, ex_xmag = 0;
+  int ex_home_bytes = 0;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -362,6 +366,16 @@ int coverage_mark_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, 
 // ppp_mls_smooth's device part: compacted rows (xyz_c: 3 floats per row; nrm_c nullable: nx ny nz curvature;
 // src_c: source index) for every finite point with >= 3 neighbours, in ascending source order.  Synchronises.
 int mls_smooth_launch(ppp_cloud* c, double radius, int order, float* xyz_c, float4* nrm_c, int32_t* src_c, int64_t* n_rows);
+// ppp_dev_mls_smooth's device part: one 32-byte record per point (by original index into rec, or to the home ranks
+// through c->route on an exchange slab, where only owned rows are queries).  Does not synchronise.
+int mls_smooth_records(ppp_cloud* c, double radius, int order, float* rec);
+// ppp_dev_mls_compact's device part: *n_rows = rows of the n records; with points_out, rows [row_base, row_base +
+// *n_rows) are written (PPP_ERR_CAPACITY past cap_rows).  Synchronises once.
+int mls_compact_launch(ppp_ctx* ctx, const float* rec, int64_t n, const float* src_rec, int out_sf, int32_t idx_base,
+                       int64_t row_base, float* points_out, float4* normals_out, int32_t* src_out, int64_t cap_rows,
+                       int64_t* n_rows);
+// The exchange halo an MLS call of this radius needs (ppp_mls_halo).
+double mls_halo(double radius, double x_abs_max);
 
 // slices.cu
 int bands_launch(ppp_cloud* c, const float* plane_x_host, int S, float half_width, int truncate_center, int sort_bands,

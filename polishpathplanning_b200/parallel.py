@@ -305,6 +305,74 @@ class Exchange:
             self._h = None
 
 
+# -------------------------------------------------------------------------------------------------
+# MLS smooth() over the exchange: halo = the MLS radius (mls_halo), every rank smooths the points it owns, each record
+# travels to its home rank, and the home ranks compact their index ranges into one result in source order.
+# -------------------------------------------------------------------------------------------------
+MLS_RECORD_BYTES = 32   # {x, y, z, flag, nx, ny, nz, curvature}: the exchange must be created with normal_stride_bytes=32
+
+
+def mls_halo(radius, x_abs_max):
+    """The exchange halo an MLS call of `radius` needs on a cloud whose finite x lie within +-x_abs_max (ppp_mls_halo:
+    the float32 reach of the radius plus the double rounding of the cut positions; derivation in csrc/mls.cu).  The
+    library refuses an MLS call on a slab cut with a narrower halo."""
+    from . import _lib
+    return float(_lib.load().ppp_mls_halo(float(radius), float(x_abs_max)))
+
+
+def mls_smooth_sharded(exs, chunk_ptrs, stride_bytes, radius, order, halo, outputs, dist=None, device=None):
+    """One MLS step for the ranks this process drives (exs: their Exchange objects, one under torchrun, every rank with
+    Exchange.connect_local; chunk_ptrs: each rank's chunk, device records of stride_bytes, its index range).
+
+    exchange -> attach -> ppp_dev_mls_smooth (records to the home ranks) -> results signal / wait -> count -> share the
+    counts (dist.all_gather across processes, the list itself when every rank lives here) -> compact.
+    outputs[i] = (points_ptr, normals_ptr or None, src_index_ptr, cap_rows, shared) for exs[i]: shared=True: one
+    buffer every rank writes (device or mapped host memory, e.g. SharedHost.dev_base sections), the rank's rows start at
+    the rows of the lower ranks; shared=False: a buffer of this rank's own, its rows from row 0.  Points are records of
+    stride_bytes: x, y, z smoothed, every other field from the source record.  Nothing is synchronised at the end:
+    call ctx.sync() (and meet the other processes) before reading.
+
+    Returns (counts, row_bases): rows of every rank and where each rank's rows start in the whole result.  The rows
+    themselves are what Cloud.mls_smooth returns for the whole cloud -- (points, src_index, normals) in ascending
+    source order -- written into the caller's buffers rather than returned: under torchrun the result is one shared
+    host buffer (or one device buffer per rank) that a returned copy would have to duplicate; mls_rows() views it."""
+    for p in range(4):                                   # phase by phase over the ranks of this process
+        for ex, ptr in zip(exs, chunk_ptrs):
+            ex.phase(p, ptr, ex.home_rows, stride_bytes, halo)
+    clouds = []
+    for ex in exs:
+        assert ex.normal_stride_bytes == MLS_RECORD_BYTES
+        clouds.append(ex.finish_attach(to_rank0=False)[1])
+        clouds[-1].dev_mls_smooth(radius, order)
+        ex.results_signal(ex.NORMALS)
+    for ex in exs:
+        ex.results_wait(ex.NORMALS)
+    mine = [ex.ctx.dev_mls_compact(ex.home_normals_ptr, ex.home_rows) for ex in exs]
+    world = exs[0].world
+    if dist is not None and len(exs) < world:
+        import torch
+        t = [torch.zeros(1, dtype=torch.int64, device=device) for _ in range(world)]
+        dist.all_gather(t, torch.tensor(mine, dtype=torch.int64, device=device))
+        counts = [int(v.item()) for v in t]
+    else:
+        assert len(exs) == world
+        counts = mine
+    bases = np.concatenate([[0], np.cumsum(counts)]).astype(np.int64)
+    for ex, ptr, (pts, nrm, src, cap, shared) in zip(exs, chunk_ptrs, outputs):
+        ex.ctx.dev_mls_compact(ex.home_normals_ptr, ex.home_rows, ptr, stride_bytes, int(ex.starts[ex.rank]),
+                               int(bases[ex.rank]) if shared else 0, pts, stride_bytes, nrm, src, cap)
+    for c in clouds:
+        c.close()
+    return counts, bases[:-1]
+
+
+def mls_rows(points, src_index, normals, counts):
+    """The (points, src_index, normals) tuple of Cloud.mls_smooth as views of shared output buffers (numpy arrays of
+    n_total rows that mls_smooth_sharded filled with shared=True); normals may be None."""
+    m = int(sum(int(c) for c in counts))
+    return points[:m], src_index[:m], (normals[:m] if normals is not None else None)
+
+
 def host_region_layout(world, n_total, normal_stride_bytes, S_cap, node_cap):
     """Byte layout of the ONE host result buffer (every section 256-byte aligned):
     [normals n_total x stride][rank 0: offsets (S_cap + 1) int64 | y | x | z (node_cap doubles each)] ... [rank world-1]."""
