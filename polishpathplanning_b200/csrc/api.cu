@@ -440,7 +440,7 @@ int ppp_dev_normals_knn(ppp_cloud* c, int k, const float vp[3], unsigned flags, 
     // not a height field: one grid per axis pair, every point searched in the projection that spreads its
     // neighbourhood out best (three launches, each warp leaves at once unless some of its points are its own)
     MPSet* mp;
-    PPP_TRY(cloud_get_mp(c, h, knn_block_rings(), &mp));
+    PPP_TRY(cloud_get_mp(c, h, PPP_KNN_RINGS, &mp));
     for (int p = 0; p < 3; p++)
       PPP_TRY(knn_launch(c, *mp->g[p], nullptr, count, 0, 0, k, knn_idx_dev, knn_d2_dev, normals_dev != nullptr, vp, flags,
                          normals_dev, (int)(normal_stride_bytes / 4), mp->choice, p));
@@ -494,7 +494,7 @@ int ppp_dev_slice_contours(ppp_cloud* c, const float* plane_x_host, int S, float
   PPP_TRY(pick_any_grid(c, &g));
   PPP_TRY(cloud_decide_projection(c, *g));
   MPSet* mp = nullptr;
-  if (c->mp_state == 1) PPP_TRY(cloud_get_mp(c, g->h, knn_block_rings(), &mp));
+  if (c->mp_state == 1) PPP_TRY(cloud_get_mp(c, g->h, PPP_KNN_RINGS, &mp));
   int st;
   int64_t M = 0, total = 0;
   {
@@ -885,7 +885,7 @@ int ppp_insert_point(ppp_cloud* c, const int32_t* indices, int64_t m, float plan
   PPP_TRY(pick_any_grid(c, &g));
   PPP_TRY(cloud_decide_projection(c, *g));
   MPSet* mp = nullptr;
-  if (c->mp_state == 1) PPP_TRY(cloud_get_mp(c, g->h, knn_block_rings(), &mp));
+  if (c->mp_state == 1) PPP_TRY(cloud_get_mp(c, g->h, PPP_KNN_RINGS, &mp));
   int64_t total = 0;
   PPP_TRY(contours_from_indices_launch(c, *g, indices, m, plane_x, pairing_mode, &total, mp));
   *n_nodes = total;

@@ -463,16 +463,6 @@ int cloud_ingest_ex(ppp_cloud* c, const void* pts_dev, size_t stride_bytes, int6
   return PPP_OK;
 }
 
-// Rings of cells in the fixed candidate block of the fast k-nearest kernels (2: a 5 x 5 block).
-int knn_block_rings() {
-  static int r0 = [] {
-    int v = 2;
-    if (const char* e = getenv("PPP_KNN_R0")) { int t = atoi(e); if (t >= 1 && t <= 4) v = t; }  // tuning aid
-    return v;
-  }();
-  return r0;
-}
-
 // Cell size for a k-search: 2 rings of cells should cover the expected k-th neighbour distance
 // with ~35% head room (queries that need more simply expand further rings).
 double cloud_cell_for_k(const ppp_cloud* c, int k) {
@@ -481,7 +471,7 @@ double cloud_cell_for_k(const ppp_cloud* c, int k) {
   double rk = std::sqrt((double)std::max(k, 1) / (3.14159265358979 * rho));
   double f = 1.35;
   if (const char* e = getenv("PPP_CELL_FACTOR")) { double v = atof(e); if (v > 0.5 && v < 4.0) f = v; }  // tuning aid
-  return f * rk / (double)knn_block_rings();
+  return f * rk / (double)PPP_KNN_RINGS;
 }
 // Cell size for a radius search: R = 2 rings cover r exactly (plus rounding slack).
 double cloud_cell_for_radius(const ppp_cloud* c, double r) {

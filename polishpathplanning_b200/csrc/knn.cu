@@ -169,498 +169,27 @@ __global__ void __launch_bounds__(128) k_search(SearchParams P) {
 
 
 // ---------------------------------------------------------------------------------------------
-// Fast k-nearest path (k <= 32): fixed (2*R0+1)^2 cell block, warp-uniform candidate loops,
-// accepted candidates buffered per thread in shared memory and merged K at a time into a sorted
-// register list with sorting networks (Batcher odd-even merge sort + bitonic merge).  No
-// data-dependent branches inside the selection: the only divergence left is the row ranges.
-// A candidate is accepted only if d2 < ring_bound2(R0) (beyond that the block is not a superset
-// of the neighbourhood), so a query that does not collect k candidates is handed to the generic
-// ring-expanding kernel through redo_list; everything it does finish is exact.
-// ---------------------------------------------------------------------------------------------
-// K = list length kept in registers (8, 16, 32, 64), PB = pending batch merged per flush.
-// RADIUS = true: fixed-radius mode (NormalEstimation::setRadiusSearch): every candidate with
-// d2 < r2 is wanted; a query with more than K of them is handed over to the generic kernel.
-template <int K, int PB, bool RADIUS>
-__global__ void __launch_bounds__(128, (K <= 16 ? 6 : (K <= 32 ? 3 : 2))) k_knn_fast(SearchParams P) {
-  pdl_prologue();
-  extern __shared__ u64 s_keys[];
-  constexpr int BD = 128;  // launch block size (immediate shared-memory offsets)
-  const int64_t t = (int64_t)blockIdx.x * BD + threadIdx.x;
-  const GridView& g = P.g;
-  bool valid = t < P.nq;
-  float qx = 0.f, qy = 0.f, qz = 0.f;
-  int64_t row = 0;
-  if (valid) {
-    if (P.q) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
-  }
-  const bool self = P.q == nullptr;
-  valid = query_is_mine(P, valid, row);
-  if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
-  const bool fin = valid && finite3(qx, qy, qz);
-  const bool act = fin && g.n_sorted > 0;
-  u64* pend_s = s_keys + threadIdx.x;
-  u64 best[K];
-#pragma unroll
-  for (int i = 0; i < K; i++) best[i] = PPP_KEY_INF;
-  int pc = 0;
-  int nacc = 0;  // RADIUS: number of in-radius candidates seen (overflow detection)
-  const int R = P.R0;
-  int cu = 0, cv = 0;
-  u64 tau = 0;  // inactive lanes accept nothing
-  if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
-    tau = RADIUS ? make_key(P.r2, 0) : make_key(ring_bound2(g, R, cu, cv), 0);
-  }
-
-  // Merge the pending batch into `best`: INF-padded load, sort network on PB keys, half-cleaner
-  // against the top PB entries of `best`, bitonic merge of all K.  One straight-line copy of the
-  // networks only: duplicated copies thrash the instruction cache.
-  auto flush = [&]() {
-    u64 pend[PB];
-#pragma unroll
-    for (int i = 0; i < PB; i++) {
-      u64 v = pend_s[i * BD];  // unconditional load (stale slots are ignored), then pad
-      pend[i] = i < pc ? v : PPP_KEY_INF;
-    }
-    SortNet<PB>::sort(pend);
-#pragma unroll
-    for (int i = 0; i < PB; i++) {
-      u64 o = pend[PB - 1 - i];
-      best[K - PB + i] = o < best[K - PB + i] ? o : best[K - PB + i];
-    }
-    SortNet<K>::bitonic_merge(best);
-    pc = 0;
-    if (!RADIUS && best[K - 1] < tau) tau = best[K - 1];
-  };
-
-  // rows dv = -R..R, plus one pseudo-row (dv = R+1) whose single empty iteration drains the
-  // pending buffers: one flush site keeps the unrolled networks in the instruction cache once.
-  // U candidates per iteration: the loads are issued together, then consumed.
-  constexpr int U = 4;
-  u64* wptr = pend_s;  // next free pending slot of this thread (= pend_s + pc * BD)
-#pragma unroll 1
-  for (int j = 0; j <= 2 * R + 1; j++) {
-    // rows nearest first: 0, -1, +1, -2, +2, ... so the first merge already yields a tight k-th
-    // distance and the outer rows add few candidates
-    const int dv = (j & 1) ? -((j + 1) >> 1) : (j >> 1);
-    int s = 0, e = 0;
-    int v = cv + dv;
-    const bool drain = j == 2 * R + 1;
-    if (!drain && act && v >= 0 && v < g.nv) {
-      int a = max(cu - R, 0), b = min(cu + R, g.nu - 1);
-      if (a <= b) {
-        const int32_t* rowp = g.cell_start + (int64_t)v * g.nu;
-        s = __ldg(rowp + a);
-        e = __ldg(rowp + b + 1);
-      }
-    }
-    // drain row: one empty iteration with trigger level 0.  Written arithmetically (no select on
-    // `drain`) so the compiler does not clone the loop body, and with it the flush networks.
-    const int n_it = (__reduce_max_sync(0xffffffffu, e - s) + U - 1) / U + (j - 2 * R > 0 ? 1 : 0);
-    const int trig = min(PB - U, (2 * R + 1 - j) * PB);  // flush when some lane could overflow next iteration
-#pragma unroll 1
-    for (int it = 0; it < n_it; it++) {
-      float4 c[U];
-      bool in[U];
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        int i = s + it * U + u;
-        in[u] = i < e;
-        c[u] = __ldg(g.sorted + (in[u] ? i : 0));
-      }
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        float d2 = d2_flann_x2(pack2(qx, qy), qz, c[u]);
-        u64 key = make_key(d2, __float_as_int(c[u].w));
-        if (in[u] && key < tau) {
-          *wptr = key;
-          wptr += BD;
-        }
-      }
-      const int pc_new = (int)(wptr - pend_s) / BD;
-      nacc += pc_new - pc;
-      pc = pc_new;
-      if (__any_sync(0xffffffffu, pc > trig)) { flush(); wptr = pend_s; }
-    }
-  }
-  if (!valid) return;
-
-  bool complete;
-  int m;  // neighbours found
-  if (RADIUS) {
-    complete = nacc <= K;
-    m = nacc;
-  } else {
-    // complete iff kk candidates were found inside the bound (then the kk-th is < bound by construction)
-    const int kk = P.kk;
-    complete = !act || kk == 0;
-    if (!complete) {
-      u64 kth = PPP_KEY_INF;
-#pragma unroll
-      for (int i = 0; i < K; i++) if (i == kk - 1) kth = best[i];
-      complete = kth != PPP_KEY_INF;
-    }
-    m = 0;
-#pragma unroll
-    for (int j = 0; j < K; j++) m += (j < P.cap && best[j] != PPP_KEY_INF) ? 1 : 0;
-  }
-  if (!complete) {
-    int slot = atomicAdd(P.redo_count, 1);
-    P.redo_list[slot] = (int32_t)t;
-    return;
-  }
-  const int k = P.cap;
-  float o[4];
-  if (K <= 16 && !RADIUS) {
-    // short lists: everything from registers, all gathers in flight at once
-    if (P.idx_out) {
-      int32_t* io = P.idx_out + row * (int64_t)k;
-      float* dout = P.d2_out ? P.d2_out + row * (int64_t)k : nullptr;
-#pragma unroll
-      for (int j = 0; j < K; j++) {
-        if (j < k) {
-          bool has = best[j] != PPP_KEY_INF;
-          io[j] = has ? key_idx(best[j]) : -1;
-          if (dout) dout[j] = has ? key_d2(best[j]) : CUDART_INF_F;
-        }
-      }
-    }
-    if (P.normals) {
-      if (!fin || m < 3) {
-        o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-      } else {
-        float4 nb[K];
-#pragma unroll
-        for (int j = 0; j < K; j++)
-          if (j < m) nb[j] = __ldg(P.xyz4 + key_idx(best[j]));
-        float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-        float kx = shifted ? nb[0].x : 0.f, ky = shifted ? nb[0].y : 0.f, kz = shifted ? nb[0].z : 0.f;
-#pragma unroll
-        for (int j = 0; j < K; j++) {
-          if (j < m) {
-            float x = nb[j].x, y = nb[j].y, z = nb[j].z;
-            if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-            accumulate_point(acc, x, y, z);
-          }
-        }
-        normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-      }
-      store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-    }
-  } else {
-    // long lists: park the sorted keys in this thread's shared-memory column (K slots) and walk
-    // them with rolled loops, which bounds registers and code size
-    __syncwarp();
-#pragma unroll
-    for (int j = 0; j < K; j++) pend_s[j * BD] = best[j];
-    if (P.idx_out && !RADIUS) {
-      int32_t* io = P.idx_out + row * (int64_t)k;
-      float* dout = P.d2_out ? P.d2_out + row * (int64_t)k : nullptr;
-      if ((k & 3) == 0 && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 15) == 0) {
-        // rows are 16-byte aligned: 128-bit stores (a lane's row is contiguous, the rows of a warp are not)
-        for (int j = 0; j < k; j += 4) {
-          u64 k0 = pend_s[j * BD], k1 = pend_s[(j + 1) * BD], k2 = pend_s[(j + 2) * BD], k3 = pend_s[(j + 3) * BD];
-          reinterpret_cast<int4*>(io)[j >> 2] = make_int4(k0 != PPP_KEY_INF ? key_idx(k0) : -1, k1 != PPP_KEY_INF ? key_idx(k1) : -1,
-                                                          k2 != PPP_KEY_INF ? key_idx(k2) : -1, k3 != PPP_KEY_INF ? key_idx(k3) : -1);
-          if (dout)
-            reinterpret_cast<float4*>(dout)[j >> 2] =
-                make_float4(k0 != PPP_KEY_INF ? key_d2(k0) : CUDART_INF_F, k1 != PPP_KEY_INF ? key_d2(k1) : CUDART_INF_F,
-                            k2 != PPP_KEY_INF ? key_d2(k2) : CUDART_INF_F, k3 != PPP_KEY_INF ? key_d2(k3) : CUDART_INF_F);
-        }
-      } else {
-        for (int j = 0; j < k; j++) {
-          u64 key = pend_s[j * BD];
-          bool has = key != PPP_KEY_INF;
-          io[j] = has ? key_idx(key) : -1;
-          if (dout) dout[j] = has ? key_d2(key) : CUDART_INF_F;
-        }
-      }
-    }
-    if (P.normals) {
-      if (!fin || m < 3) {
-        o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-      } else {
-        float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-        const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-        float kx = 0.f, ky = 0.f, kz = 0.f;
-        if (shifted) {
-          float4 f = __ldg(P.xyz4 + key_idx(pend_s[0]));
-          kx = f.x; ky = f.y; kz = f.z;
-        }
-        int j = 0;
-        for (; j + 4 <= m; j += 4) {
-          float4 a0 = __ldg(P.xyz4 + key_idx(pend_s[(j + 0) * BD]));
-          float4 a1 = __ldg(P.xyz4 + key_idx(pend_s[(j + 1) * BD]));
-          float4 a2 = __ldg(P.xyz4 + key_idx(pend_s[(j + 2) * BD]));
-          float4 a3 = __ldg(P.xyz4 + key_idx(pend_s[(j + 3) * BD]));
-          if (shifted) {
-            a0.x = __fsub_rn(a0.x, kx); a0.y = __fsub_rn(a0.y, ky); a0.z = __fsub_rn(a0.z, kz);
-            a1.x = __fsub_rn(a1.x, kx); a1.y = __fsub_rn(a1.y, ky); a1.z = __fsub_rn(a1.z, kz);
-            a2.x = __fsub_rn(a2.x, kx); a2.y = __fsub_rn(a2.y, ky); a2.z = __fsub_rn(a2.z, kz);
-            a3.x = __fsub_rn(a3.x, kx); a3.y = __fsub_rn(a3.y, ky); a3.z = __fsub_rn(a3.z, kz);
-          }
-          accumulate_point(acc, a0.x, a0.y, a0.z);
-          accumulate_point(acc, a1.x, a1.y, a1.z);
-          accumulate_point(acc, a2.x, a2.y, a2.z);
-          accumulate_point(acc, a3.x, a3.y, a3.z);
-        }
-        for (; j < m; j++) {
-          float4 a = __ldg(P.xyz4 + key_idx(pend_s[j * BD]));
-          if (shifted) { a.x = __fsub_rn(a.x, kx); a.y = __fsub_rn(a.y, ky); a.z = __fsub_rn(a.z, kz); }
-          accumulate_point(acc, a.x, a.y, a.z);
-        }
-        normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-      }
-      store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// k <= 16 variant with 32-bit COMPOSITE sort keys.  Accepted candidates are parked, unmoved, in a
-// 32-slot shared-memory store per thread (full 64-bit keys).  A flush sorts the 32 composite keys
-//     c = (bits(d2) & ~31) | slot
-// with a Batcher network whose compare-exchange is one unsigned min + one unsigned max (2
-// instructions instead of 6 for 64-bit keys), keeps the 16 smallest, moves their full keys to
-// slots 0..15 and tightens the acceptance threshold to the exact key of the 16th.
-// Dropping 5 mantissa bits can only misorder two candidates whose d2 agree in the upper 27 bits;
-// any such pair among the 17 smallest marks the query for the exact hand-over kernel instead
-// (measured: well under 0.1 % of the queries), so every delivered list is in the exact
-// (d2, index) order.  For the same reason the low word of a parked key need not be the point index:
-// it is the candidate's position in the sorted array, which the final gather reads back.
-// ---------------------------------------------------------------------------------------------
-constexpr int C_SLOTS = 32;   // keys ordered per network pass
-constexpr int C_STORE = 36;   // storage slots: U spare ones, so a pass is only forced beyond 32 occupied
-
-template <int BD>
-__device__ __forceinline__ void knn16c_body(const SearchParams& P, const int64_t t, bool valid) {
-  extern __shared__ u64 s_keys[];
-  constexpr int K = 16;
-  const GridView& g = P.g;
-  float qx = 0.f, qy = 0.f, qz = 0.f;
-  int64_t row = 0;
-  if (valid) {
-    if (P.q) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
-  }
-  valid = query_is_mine(P, valid, row);
-  if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
-  const bool fin = valid && finite3(qx, qy, qz);
-  const bool act = fin && g.n_sorted > 0;
-  u64* store = s_keys + threadIdx.x;  // slot j of this thread at store[j * BD]
-  // 32-bit shared-window address of slot 0: the candidate loop advances a 32-bit cursor (one
-  // predicated add per accepted candidate) instead of a 64-bit generic pointer
-  const unsigned store_sa = (unsigned)__cvta_generic_to_shared(store);
-  constexpr unsigned SLOT_B = BD * 8;
-  const int R = P.R0;
-  int cu = 0, cv = 0;
-  // Acceptance threshold on d2 alone, INCLUSIVE: a candidate that ties the current K-th distance is
-  // parked too, and the tie then shows up as an ambiguous pair in the next pass (-> exact hand-over).
-  // The low key word is the candidate's SORTED POSITION, not its index: the final gather reads
-  // g.sorted[pos] (coordinates + original index in one record, from lines this warp has just used).
-  float tau = -1.0f;  // inactive lanes accept nothing
-  if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
-    tau = ring_bound2(g, R, cu, cv);
-  }
-  int ns = 0;            // occupied slots
-  bool ambiguous = false;
-  const int last = max(g.n_sorted - 1, 0);
-
-  auto flush = [&]() {
-    unsigned c[C_SLOTS];
-#pragma unroll
-    for (int i = 0; i < C_SLOTS; i++) {
-      unsigned hi = (unsigned)(store[i * BD] >> 32);   // stale slots are masked below
-      c[i] = i < ns ? ((hi & 0xFFFFFFE0u) | (unsigned)i) : 0xFFFFFFFFu;
-    }
-    SortNetU32<C_SLOTS>::sort(c);
-    // two of the 17 smallest with equal upper 27 bits: their order (or the cut between the 16th and
-    // the 17th) is not decided by the composite key
-#pragma unroll
-    for (int i = 0; i < K; i++) ambiguous |= (i + 1 < ns) && ((c[i] ^ c[i + 1]) < 32u);
-    // the K smallest, in order, to slots 0..K-1 (INF padded while fewer than K are known)
-    u64 keep[K];
-#pragma unroll
-    for (int i = 0; i < K; i++) keep[i] = i < ns ? store[(c[i] & 31u) * BD] : PPP_KEY_INF;
-#pragma unroll
-    for (int i = 0; i < K; i++) store[i * BD] = keep[i];
-    if (ns >= K) tau = fminf(tau, key_d2(keep[K - 1]));
-    ns = min(ns, K);
-  };
-
-  constexpr int U = 4;
-#pragma unroll 1
-  for (int j = 0; j <= 2 * R + 1; j++) {
-    const int dv = (j & 1) ? -((j + 1) >> 1) : (j >> 1);  // rows nearest first
-    int s = 0, e = 0;
-    int v = cv + dv;
-    const bool drain = j == 2 * R + 1;
-    if (!drain && act && v >= 0 && v < g.nv) {
-      int a = max(cu - R, 0), b = min(cu + R, g.nu - 1);
-      if (a <= b) {
-        const int32_t* rowp = g.cell_start + (int64_t)v * g.nu;
-        s = __ldg(rowp + a);
-        e = __ldg(rowp + b + 1);
-      }
-    }
-    const int n_it = (__reduce_max_sync(0xffffffffu, e - s) + U - 1) / U + (j - 2 * R > 0 ? 1 : 0);
-    // flush when some lane could run out of slots in the next iteration; the drain row flushes once
-    const int trig = min(C_SLOTS - U, (2 * R + 1 - j) * C_SLOTS - 1);
-    unsigned wsa = store_sa + (unsigned)ns * SLOT_B;
-    const unsigned trig_sa = store_sa + (unsigned)trig * SLOT_B;
-    int i0 = s;
-#pragma unroll 1
-    for (int it = 0; it < n_it; it++, i0 += U) {
-      float4 c4[U];
-#pragma unroll
-      for (int u = 0; u < U; u++) c4[u] = __ldg(g.sorted + min(i0 + u, last));   // clamped: always a valid record
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        float d2 = d2_flann_x2(pack2(qx, qy), qz, c4[u]);
-        if (i0 + u < e && d2 <= tau) {
-          asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(wsa), "r"(i0 + u), "r"(__float_as_uint(d2)) : "memory");
-          wsa += SLOT_B;
-        }
-      }
-      if (__any_sync(0xffffffffu, wsa > trig_sa)) {
-        ns = (int)((wsa - store_sa) / SLOT_B);
-        flush();
-        wsa = store_sa + (unsigned)ns * SLOT_B;
-      }
-    }
-    ns = (int)((wsa - store_sa) / SLOT_B);
-  }
-  if (!valid) return;
-  // slots 0..15 now hold the 16 smallest keys in order (INF padded)
-  const int kk = P.kk;
-  bool complete = !act || kk == 0;
-  if (!complete) complete = store[(kk - 1) * BD] != PPP_KEY_INF;
-  if (!complete || ambiguous) {
-    P.redo_list[atomicAdd(P.redo_count, 1)] = (int32_t)t;
-    return;
-  }
-  const int k = P.cap;
-  int m = 0;  // neighbours found (the list is sorted and INF padded)
-#pragma unroll
-  for (int j = 0; j < K; j++) m += (act && j < k && (unsigned)(store[j * BD] >> 32) != 0xFFFFFFFFu) ? 1 : 0;
-  int32_t* io = P.idx_out ? P.idx_out + row * (int64_t)k : nullptr;
-  float* dout = (P.idx_out && P.d2_out) ? P.d2_out + row * (int64_t)k : nullptr;
-  const bool al32 = k == K && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 31) == 0;
-  const bool al16 = (k & 3) == 0 && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 15) == 0;
-  const bool want_n = P.normals && fin && m >= 3;
-  const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-  float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  float kx = 0.f, ky = 0.f, kz = 0.f;
-  // Eight neighbours at a time: ONE gather of the neighbour's sorted record serves both outputs (its
-  // coordinates for the covariance, its original index for the id list); eight records in flight keep
-  // the register count where the candidate loop wants it.
-#pragma unroll
-  for (int jb = 0; jb < K; jb += 8) {
-    if (jb >= k) break;
-    float4 nb[8];
-    float dd[8];
-#pragma unroll
-    for (int u = 0; u < 8; u++) {
-      const u64 key = store[(jb + u) * BD];
-      const bool has = jb + u < m;
-      nb[u] = has ? __ldg(g.sorted + key_idx(key)) : make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
-      dd[u] = has ? key_d2(key) : CUDART_INF_F;
-    }
-    if (io) {
-      if (al32) {
-        // a full row is 64 contiguous, 32-byte aligned bytes: two 256-bit stores instead of sixteen 32-bit ones
-        st_global_256(io + jb, nb[0].w, nb[1].w, nb[2].w, nb[3].w, nb[4].w, nb[5].w, nb[6].w, nb[7].w);
-        if (dout) {
-          reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-          reinterpret_cast<float4*>(dout + jb)[1] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        }
-      } else if (al16) {
-        // k = 4, 8, 12: rows are still 16-byte aligned
-        reinterpret_cast<float4*>(io + jb)[0] = make_float4(nb[0].w, nb[1].w, nb[2].w, nb[3].w);
-        if (dout) reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        if (jb + 4 < k) {
-          reinterpret_cast<float4*>(io + jb)[1] = make_float4(nb[4].w, nb[5].w, nb[6].w, nb[7].w);
-          if (dout) reinterpret_cast<float4*>(dout + jb)[1] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        }
-      } else {
-#pragma unroll
-        for (int u = 0; u < 8; u++) {
-          if (jb + u < k) {
-            io[jb + u] = __float_as_int(nb[u].w);
-            if (dout) dout[jb + u] = dd[u];
-          }
-        }
-      }
-    }
-    if (want_n) {
-      if (jb == 0 && shifted) { kx = nb[0].x; ky = nb[0].y; kz = nb[0].z; }
-#pragma unroll
-      for (int u = 0; u < 8; u++) {
-        if (jb + u < m) {
-          float x = nb[u].x, y = nb[u].y, z = nb[u].z;
-          if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-          accumulate_point(acc, x, y, z);
-        }
-      }
-    }
-  }
-  if (P.normals) {
-    float o[4];
-    if (want_n) normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    else o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-  }
-}
-
-template <int BD>
-__global__ void __launch_bounds__(BD, (BD == 128 ? 7 : (BD == 96 ? 9 : 13))) k_knn16c(SearchParams P) {
-  pdl_prologue();
-  const int64_t t = (int64_t)blockIdx.x * BD + threadIdx.x;
-  knn16c_body<BD>(P, t, t < P.nq);
-}
-
-// ---------------------------------------------------------------------------------------------
-// k <= 16, the cloud's own points as queries: 32-bit FIXED-POINT keys.
+// k <= 16: 32-bit FIXED-POINT keys.  The queries are the cloud's own points in cell order or, with EXT, a query
+// array (its row t is the query's position); only the load of the query differs.
 //     key = floor(d2 * scale) << 10 | ordinal         scale = (2^22 - margin) / (ring bound)^2  per query
 // Candidates arrive uniformly in d2 (area), so 22 bits of fixed point over [0, bound^2] resolve the k-th
 // neighbourhood nearly as finely as the float itself does (2.2e-6 mm^2 at cfg2 against an ulp of 4.8e-7), where a
 // truncated float spends its bits on the nearest neighbours.  The ordinal names the candidate by (row of the
 // block, slot in the row); its sorted position is rebuilt from the row start at the very end, and the exact d2
 // -- needed only if the caller asked for distances -- is recomputed from the gathered record with the same
-// arithmetic.  Consequences against the composite-key kernel above: the per-thread store is 4 bytes per slot
-// instead of 8 (half the shared-memory wave fronts, which with the scattered 128-bit candidate loads made the L1
-// data pipe the busiest unit of that kernel: 69 % under ncu), the sorted words ARE the result (no composite
-// construction, no second gather through the slot number), and from the second flush on slots 0..15 are already
-// in order, so a flush is a 16-input sort of the newcomers, one row of minima and a 16-input bitonic merge.
-// Two candidates whose keys agree in the upper 22 bits (including the best one just dropped) leave the order to
-// the exact hand-over kernel, exactly like the composite keys do.  floor(d2 * scale) is one FFMA.RZ against
+// arithmetic.  So the per-thread store is 4 bytes per slot, the sorted words ARE the result, and from the second
+// flush on slots 0..15 are already in order, so a flush is a 16-input sort of the newcomers, one row of minima and
+// a 16-input bitonic merge.  Two candidates whose keys agree in the upper 22 bits (including the best one just
+// dropped) leave their order to the exact hand-over kernel k_knn_warp.  floor(d2 * scale) is one FFMA.RZ against
 // 2^23 (exact floor of the real product: monotone in d2).
 // ---------------------------------------------------------------------------------------------
 constexpr int F_SLOTS = 32;
 constexpr int F_MAXR = 3;
+static_assert(PPP_KNN_RINGS <= F_MAXR, "the ordinal names the block row in 3 bits: 2 R0 + 1 <= 7");
 // RB (template parameter of k_knn16f): bits of the ordinal that name the slot inside a cell row (3 more name the row,
 // 2R+1 <= 7).  RB = 7: rows of up to 128 candidates, 22 bits of d2.
 
-template <int BD, int MB, int F_RB>
+template <int BD, int MB, int F_RB, bool EXT>
 __global__ void __launch_bounds__(BD, MB) k_knn16f(SearchParams P) {
   pdl_prologue();
   extern __shared__ __align__(128) unsigned s_fkeys[];
@@ -682,9 +211,15 @@ __global__ void __launch_bounds__(BD, MB) k_knn16f(SearchParams P) {
   float qx = 0.f, qy = 0.f, qz = 0.f;
   int64_t row = 0;
   if (valid) {
-    float4 p = __ldg(g.sorted + P.first + t);
-    qx = p.x; qy = p.y; qz = p.z;
-    row = __float_as_int(p.w);
+    if (EXT) {
+      const float* qp = P.q + t * P.q_sf;
+      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
+      row = t;
+    } else {
+      float4 p = __ldg(g.sorted + P.first + t);
+      qx = p.x; qy = p.y; qz = p.z;
+      row = __float_as_int(p.w);
+    }
   }
   valid = query_is_mine(P, valid, row);
   if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
@@ -890,209 +425,15 @@ __global__ void __launch_bounds__(BD, MB) k_knn16f(SearchParams P) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// 16 < k <= 32 with the same composite keys and a MERGE instead of a full sort: slots 0..31 of the
-// per-thread store hold the 32 best so far in order, slots 32..47 take up to 16 newly accepted candidates.
-// A flush sorts the 16 new composite keys  (bits(d2) & ~63) | slot  (63 exchanges), folds them into the
-// kept 32 with one row of minima (the half-cleaner of a bitonic merge whose other inputs are +inf) and a
-// 32-input bitonic merge (80 exchanges), every exchange one unsigned min + one unsigned max, then moves
-// the full keys of the survivors to slots 0..31.  Dropping 6 mantissa bits leaves the order of two
-// candidates open only if their d2 agree in the upper 26 bits; such a pair among the 33 smallest sends the
-// query to the exact hand-over kernel.  (The 64-bit-key kernel this replaces kept 32 + 16 keys in 96
-// registers and spilled 304 bytes per thread.)
+// 16 < k <= 64: the fixed-point keys of k_knn16f (queries from the cloud or, with EXT, from a query array) with a
+// MERGE instead of a full sort.  Slots 0..K-1 hold the K best so far in order (free values behind the keys), slots
+// K..K+NEW-1 take the newcomers; a flush sorts the newcomers, folds them into the kept K with one row of minima (the
+// half-cleaner of a bitonic merge) and a K-input bitonic merge, every exchange one unsigned min + one unsigned max,
+// and writes the K words back.  K = 32: 16 newcomers (63 + 80 exchanges per flush), ordinals of 3 + 6 bits, 23 bits
+// of d2.  K = 64: 32 newcomers (191 + 192 exchanges), ordinals of 3 + 7 bits (rows of up to 128 candidates), 22 bits
+// of d2 -- the list lives in 96 registers during a flush.
 // ---------------------------------------------------------------------------------------------
-template <int BD>
-__global__ void __launch_bounds__(BD, (BD == 64 ? 8 : 4)) k_knn32c(SearchParams P) {
-  pdl_prologue();
-  extern __shared__ u64 s_keys[];
-  constexpr int K = 32, NEW = 16, SLOTS = K + NEW;
-  constexpr unsigned SMASK = 63u;   // slot bits of a composite key
-  const int64_t t = (int64_t)blockIdx.x * BD + threadIdx.x;
-  const GridView& g = P.g;
-  bool valid = t < P.nq;
-  float qx = 0.f, qy = 0.f, qz = 0.f;
-  int64_t row = 0;
-  if (valid) {
-    if (P.q) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
-  }
-  valid = query_is_mine(P, valid, row);
-  if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
-  const bool fin = valid && finite3(qx, qy, qz);
-  const bool act = fin && g.n_sorted > 0;
-  u64* store = s_keys + threadIdx.x;
-  const unsigned store_sa = (unsigned)__cvta_generic_to_shared(store);
-  constexpr unsigned SLOT_B = BD * 8;
-  const int R = P.R0;
-  const int kk = P.kk;       // neighbours wanted (<= 32)
-  int cu = 0, cv = 0;
-  float tau = -1.0f;         // inclusive d2 threshold; inactive lanes accept nothing
-  if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
-    tau = ring_bound2(g, R, cu, cv);
-  }
-  int nk = 0;                // kept (slots 0..nk-1, sorted)
-  bool ambiguous = false;
-  const int last = max(g.n_sorted - 1, 0);
-  unsigned wsa = store_sa + (unsigned)K * SLOT_B;     // cursor in the "new" region
-
-  auto flush = [&]() {
-    const int nn = (int)((wsa - store_sa) / SLOT_B) - K;
-    unsigned b[NEW];
-#pragma unroll
-    for (int i = 0; i < NEW; i++) {
-      unsigned hi = (unsigned)(store[(K + i) * BD] >> 32);   // stale slots are masked below
-      b[i] = i < nn ? ((hi & ~SMASK) | (unsigned)(K + i)) : 0xFFFFFFFFu;
-    }
-    SortNetU32<NEW>::sort(b);
-    unsigned a[K];
-#pragma unroll
-    for (int i = 0; i < K; i++) {
-      unsigned hi = (unsigned)(store[i * BD] >> 32);
-      a[i] = i < nk ? ((hi & ~SMASK) | (unsigned)i) : 0xFFFFFFFFu;
-    }
-    // kept (ascending) ++ new (descending, +inf padded in front) is bitonic: its half-cleaner leaves the 32
-    // smallest in a[]; the smallest of what it discards is the 33rd of the union
-    unsigned next = 0xFFFFFFFFu;
-#pragma unroll
-    for (int i = K - NEW; i < K; i++) {
-      const unsigned o = b[K - 1 - i];
-      next = min(next, max(a[i], o));
-      a[i] = min(a[i], o);
-    }
-    SortNetU32<K>::bitonic_merge(a);
-    const int tot = min(nk + nn, K);
-#pragma unroll
-    for (int i = 0; i + 1 < K; i++) ambiguous |= (i + 1 < tot) && ((a[i] ^ a[i + 1]) <= SMASK);
-    ambiguous |= (nk + nn > K) && ((a[K - 1] ^ next) <= SMASK);
-    u64 keep[K];
-#pragma unroll
-    for (int i = 0; i < K; i++) keep[i] = i < tot ? store[(a[i] & SMASK) * BD] : PPP_KEY_INF;
-#pragma unroll
-    for (int i = 0; i < K; i++) store[i * BD] = keep[i];
-    nk = tot;
-    wsa = store_sa + (unsigned)K * SLOT_B;
-    if (nk >= kk && kk > 0) tau = fminf(tau, key_d2(store[(kk - 1) * BD]));
-  };
-
-  constexpr int U = 4;
-  const unsigned trig_sa = store_sa + (unsigned)(K + NEW - U) * SLOT_B;   // room for one more iteration?
-#pragma unroll 1
-  for (int j = 0; j <= 2 * R + 1; j++) {
-    const int dv = (j & 1) ? -((j + 1) >> 1) : (j >> 1);  // rows nearest first
-    int s = 0, e = 0;
-    int v = cv + dv;
-    const bool drain = j == 2 * R + 1;
-    if (!drain && act && v >= 0 && v < g.nv) {
-      int a0 = max(cu - R, 0), b0 = min(cu + R, g.nu - 1);
-      if (a0 <= b0) {
-        const int32_t* rowp = g.cell_start + (int64_t)v * g.nu;
-        s = __ldg(rowp + a0);
-        e = __ldg(rowp + b0 + 1);
-      }
-    }
-    // the drain pseudo-row runs one empty iteration whose flush is unconditional
-    const int n_it = (__reduce_max_sync(0xffffffffu, e - s) + U - 1) / U + (j - 2 * R > 0 ? 1 : 0);
-    const unsigned trig = drain ? 0u : trig_sa;
-    int i0 = s;
-#pragma unroll 1
-    for (int it = 0; it < n_it; it++, i0 += U) {
-      float4 c4[U];
-#pragma unroll
-      for (int u = 0; u < U; u++) c4[u] = __ldg(g.sorted + min(i0 + u, last));
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        float d2 = d2_flann_x2(pack2(qx, qy), qz, c4[u]);
-        if (i0 + u < e && d2 <= tau) {
-          asm volatile("st.shared.v2.b32 [%0], {%1, %2};" ::"r"(wsa), "r"(i0 + u), "r"(__float_as_uint(d2)) : "memory");
-          wsa += SLOT_B;
-        }
-      }
-      if (__any_sync(0xffffffffu, wsa > trig)) flush();
-    }
-  }
-  if (!valid) return;
-  const bool complete = !act || kk == 0 || nk >= kk;
-  if (!complete || ambiguous) {
-    int slot = atomicAdd(P.redo_count, 1);
-    P.redo_list[slot] = (int32_t)t;
-    return;
-  }
-  const int k = P.cap;
-  const int m = act ? min(nk, k) : 0;
-  int32_t* io = P.idx_out ? P.idx_out + row * (int64_t)k : nullptr;
-  float* dout = (P.idx_out && P.d2_out) ? P.d2_out + row * (int64_t)k : nullptr;
-  const bool al32 = (k & 7) == 0 && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 31) == 0;
-  const bool want_n = P.normals && fin && m >= 3;
-  const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-  float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  float kx = 0.f, ky = 0.f, kz = 0.f;
-#pragma unroll 1
-  for (int jb = 0; jb < k; jb += 8) {
-    float4 nb[8];
-    float dd[8];
-#pragma unroll
-    for (int u = 0; u < 8; u++) {
-      const bool has = jb + u < m;
-      const u64 key = has ? store[(jb + u) * BD] : 0ull;
-      nb[u] = has ? __ldg(g.sorted + key_idx(key)) : make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
-      dd[u] = has ? key_d2(key) : CUDART_INF_F;
-    }
-    if (io) {
-      if (al32) {
-        st_global_256(io + jb, nb[0].w, nb[1].w, nb[2].w, nb[3].w, nb[4].w, nb[5].w, nb[6].w, nb[7].w);
-        if (dout) {
-          reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-          reinterpret_cast<float4*>(dout + jb)[1] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        }
-      } else {
-#pragma unroll
-        for (int u = 0; u < 8; u++) {
-          if (jb + u < k) {
-            io[jb + u] = __float_as_int(nb[u].w);
-            if (dout) dout[jb + u] = dd[u];
-          }
-        }
-      }
-    }
-    if (want_n) {
-      if (jb == 0 && shifted) { kx = nb[0].x; ky = nb[0].y; kz = nb[0].z; }
-#pragma unroll
-      for (int u = 0; u < 8; u++) {
-        if (jb + u < m) {
-          float x = nb[u].x, y = nb[u].y, z = nb[u].z;
-          if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-          accumulate_point(acc, x, y, z);
-        }
-      }
-    }
-  }
-  if (P.normals) {
-    float o[4];
-    if (want_n) normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    else o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-  }
-}
-
-// ---------------------------------------------------------------------------------------------
-// 16 < k <= 64, the cloud's own points as queries: the fixed-point keys of k_knn16f with the merge scheme of
-// k_knn32c.  Slots 0..K-1 hold the K best so far in order (free values behind the keys), slots K..K+NEW-1 take the
-// newcomers; a flush sorts the newcomers, folds them into the kept K with one row of minima and a K-input bitonic
-// merge and writes the K words back: no composite construction, no gather of 64-bit keys through the slot number,
-// 4 bytes of shared memory per slot instead of 8.  K = 32: 16 newcomers (63 + 80 exchanges per flush), ordinals of
-// 3 + 6 bits, 23 bits of d2.  K = 64: 32 newcomers (191 + 192 exchanges), ordinals of 3 + 7 bits (rows of up to 128
-// candidates), 22 bits of d2 -- the list lives in 96 registers during a flush where the 64-bit-key kernel it
-// replaces (k_knn_fast<64,16>) needed 198.
-// ---------------------------------------------------------------------------------------------
-template <int K, int NEW, int RB, int BD, int MB>
+template <int K, int NEW, int RB, int BD, int MB, bool EXT>
 __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   pdl_prologue();
   extern __shared__ __align__(128) unsigned s_fkeys[];
@@ -1112,9 +453,15 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   float qx = 0.f, qy = 0.f, qz = 0.f;
   int64_t row = 0;
   if (valid) {
-    float4 p = __ldg(g.sorted + P.first + t);
-    qx = p.x; qy = p.y; qz = p.z;
-    row = __float_as_int(p.w);
+    if (EXT) {
+      const float* qp = P.q + t * P.q_sf;
+      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
+      row = t;
+    } else {
+      float4 p = __ldg(g.sorted + P.first + t);
+      qx = p.x; qy = p.y; qz = p.z;
+      row = __float_as_int(p.w);
+    }
   }
   valid = query_is_mine(P, valid, row);
   if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
@@ -1301,11 +648,18 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
 
 // ---------------------------------------------------------------------------------------------
 // Fixed-radius normals (NormalEstimation::setRadiusSearch, the reference's default r = 2.5) with
-// the same composite-key idea: every candidate with d2 < r2 is parked in one of 32 slots, ONE
-// 32-input network on 32-bit composite keys orders them at the end, and the covariance is
-// accumulated by walking the sorted slots.  A query with more than 32 - U neighbours, or with two
-// neighbours whose d2 agree in the upper 27 bits, goes to the generic kernel (exact for any count).
+// 32-bit COMPOSITE sort keys.  Every candidate with d2 < r2 is parked, unmoved, in a shared-memory
+// store per thread (full 64-bit keys).  At the end ONE 32-input Batcher network sorts the composite keys
+//     c = (bits(d2) & ~31) | slot
+// (a compare-exchange is one unsigned min + one unsigned max: 2 instructions instead of 6 for 64-bit
+// keys), and the covariance is accumulated by walking the slots in that order.  Dropping 5 mantissa
+// bits can only misorder two candidates whose d2 agree in the upper 27 bits; a query with such a pair,
+// or with more than C_SLOTS neighbours, goes to the hand-over kernels (exact for any count), so every
+// accumulation runs in the exact (d2, index) order.
 // ---------------------------------------------------------------------------------------------
+constexpr int C_SLOTS = 32;   // keys ordered per network pass
+constexpr int C_STORE = 36;   // storage slots: U spare ones, so a query overflows only beyond 32 neighbours
+
 __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
   pdl_prologue();
   extern __shared__ u64 s_keys[];
@@ -1423,8 +777,8 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Ring-expanding k-nearest search, one WARP per query: the hand-over path of k_knn_fast (sparse
-// regions, cloud borders; typically well under 1% of the queries).  The 32 lanes stride over the
+// Ring-expanding k-nearest search, one WARP per query: the hand-over path of k_knn16f and k_knnf (sparse
+// regions, cloud borders, near-ties, dense rows; typically well under 1% of the queries).  The 32 lanes stride over the
 // candidates of each ring (coalesced), each lane keeps its own sorted list of at most k keys in
 // shared memory, and after every ring the k smallest of the 32 lists are extracted with warp-wide
 // 64-bit min reductions to test the exactness bound.  A thread-per-query kernel is latency-bound
@@ -1931,19 +1285,6 @@ static int launch_search(ppp_cloud* c, SearchParams& P) {
   return PPP_OK;
 }
 
-template <int K, int PB, bool RADIUS>
-static int launch_knn_fast_k(ppp_cloud* c, SearchParams& P) {
-  ppp_ctx* ctx = c->ctx;
-  auto kern = k_knn_fast<K, PB, RADIUS>;
-  const int block = 128;
-  size_t smem = (size_t)((K > 16 || RADIUS) ? (K > PB ? K : PB) : PB) * 8 * block;
-  if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  unsigned blocks = (unsigned)((P.nq + block - 1) / block);
-  PPP_LAUNCH(ctx, RADIUS ? "radius_normals" : (P.normals ? "knn_normals" : "knn"), kern, blocks, block, smem, P);
-  PPP_CHECK_LAUNCH();
-  return PPP_OK;
-}
-
 static int prepare_fast(ppp_cloud* c, SearchParams& P, int32_t** redo_out) {
   ppp_ctx* ctx = c->ctx;
   int32_t* redo = nullptr;
@@ -1961,69 +1302,30 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
   ppp_ctx* ctx = c->ctx;
   int32_t* redo = nullptr;
   PPP_TRY(prepare_fast(c, P, &redo));
-  int st;
-  if (P.cap <= 16) {
-    // block size: 96 threads hold 27 warps per SM (24 KB of candidate store per block), 128 hold 24.
-    // (Tried and rejected on measurements: a second pass of this kernel with a 7 x 7 block over the ~0.2 % of
-    // queries the 5 x 5 block cannot finish, before the one-warp-per-query kernel: each extra launch costs the
-    // life time of one block, 30-50 us, whatever the number of queries -- 0.308 ms against 0.266 ms for the stage.)
-    // the cloud's own points (cell order): fixed-point keys; external queries keep the composite-key kernel
-    static const bool old16 = getenv("PPP_KNN16_OLD") != nullptr;   // tuning / comparison aid
-    const bool fixed = !P.q && P.R0 <= F_MAXR && !old16;
-    int block = fixed ? 128 : 96;   // measured: 0.196 / 0.198 / 0.201 ms with 128 / 64 / 96 threads (fixed-point kernel)
-    if (const char* e = getenv("PPP_KNN_BD")) { int v = atoi(e); if (v == 64 || v == 96 || v == 128) block = v; }
-    size_t smem = fixed ? (size_t)(F_SLOTS + 2 * P.R0 + 1) * 4 * block : (size_t)C_SLOTS * 8 * block;
-    static const bool more_regs = getenv("PPP_KNN16_REGS72") != nullptr;   // 72 instead of 64 registers per thread
-    // (RB = 9 -- rows of up to 512 candidates -- for workpieces with walls was measured and rejected: box with walls
-    // search 0.41 -> 0.72 ms for a hand-over kernel that only went 0.73 -> 0.53 ms: the warp-uniform row loops of the
-    // thread-per-query kernel pay for the longest row of 32 queries.)
-    auto kern = fixed ? (block == 128 ? (more_regs ? k_knn16f<128, 7, 7> : k_knn16f<128, 8, 7>)
-                                      : (block == 96 ? (more_regs ? k_knn16f<96, 9, 7> : k_knn16f<96, 10, 7>)
-                                                     : (more_regs ? k_knn16f<64, 14, 7> : k_knn16f<64, 16, 7>)))
-                      : (block == 128 ? k_knn16c<128> : (block == 96 ? k_knn16c<96> : k_knn16c<64>));
-    PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    unsigned blocks = (unsigned)((P.nq + block - 1) / block);
+  // measured with the cloud's own points (1M points, ms): k = 16 0.196 / 0.198 / 0.201 with 128 / 64 / 96 threads;
+  // k = 32 128 threads x 6 blocks (80 registers) 0.351, x 5 (93) 0.359, 64 threads x 12 / 10 / 8 0.354 / 0.365 / 0.359;
+  // k = 64 0.789 with 128 threads x 4 blocks, 0.829 with 64 x 8.
+  // (Tried and rejected on measurements: a second pass of the k <= 16 kernel with a 7 x 7 block over the ~0.2 % of
+  // queries the 5 x 5 block cannot finish, before the one-warp-per-query kernel: each extra launch costs the life
+  // time of one block, 30-50 us, whatever the number of queries -- 0.308 ms against 0.266 ms for the stage.  RB = 9
+  // -- rows of up to 512 candidates -- for workpieces with walls: box with walls search 0.41 -> 0.72 ms for a
+  // hand-over kernel that only went 0.73 -> 0.53 ms: the warp-uniform row loops of the thread-per-query kernel pay
+  // for the longest row of 32 queries.)
+  constexpr int block = 128;
+  const unsigned blocks = (unsigned)((P.nq + block - 1) / block);
+  const bool ext = P.q != nullptr;   // a query array instead of the cloud's own points in cell order
+  // per thread: `slots` key words, then the first sorted position of each of the 2 R0 + 1 block rows
+  auto launch = [&](auto kern, int slots) -> int {
+    const size_t smem = (size_t)(slots + 2 * P.R0 + 1) * 4 * block;
+    if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     PPP_LAUNCH(ctx, P.normals ? "knn_normals" : "knn", kern, blocks, block, smem, P);
     PPP_CHECK_LAUNCH();
-    st = PPP_OK;
-  }
-  else if (P.cap <= 32 && !P.q && P.R0 <= F_MAXR && !getenv("PPP_KNN32_OLD")) {
-    // measured (1M points, k = 32, ms): 128 threads x 6 blocks (80 registers) 0.351, x 5 (93) 0.359, 64 threads x 12 / 10 / 8: 0.354 / 0.365 / 0.359
-    int block = 128;
-    if (const char* e = getenv("PPP_KNN_BD")) { int v = atoi(e); if (v == 64 || v == 128) block = v; }
-    size_t smem = (size_t)(32 + 16 + 2 * P.R0 + 1) * 4 * block;
-    static const int regs = getenv("PPP_KNNF_REGS") ? atoi(getenv("PPP_KNNF_REGS")) : 0;   // tuning aid: +1 more registers, fewer blocks
-    auto kern = block == 128 ? (regs > 0 ? k_knnf<32, 16, 6, 128, 5> : k_knnf<32, 16, 6, 128, 6>)
-                             : (regs > 0 ? k_knnf<32, 16, 6, 64, 10> : k_knnf<32, 16, 6, 64, 12>);
-    unsigned blocks = (unsigned)((P.nq + block - 1) / block);
-    PPP_LAUNCH(ctx, P.normals ? "knn_normals" : "knn", kern, blocks, block, smem, P);
-    PPP_CHECK_LAUNCH();
-    st = PPP_OK;
-  }
-  else if (P.cap > 32 && P.cap <= 64 && !P.q && P.R0 <= F_MAXR && !getenv("PPP_KNN64_OLD")) {
-    int block = 128;   // measured (1M points, k = 64): 0.789 ms with 128 threads x 4 blocks, 0.829 with 64 x 8
-    if (const char* e = getenv("PPP_KNN_BD")) { int v = atoi(e); if (v == 64 || v == 128) block = v; }
-    size_t smem = (size_t)(64 + 32 + 2 * P.R0 + 1) * 4 * block;
-    static const int regs = getenv("PPP_KNNF_REGS") ? atoi(getenv("PPP_KNNF_REGS")) : 0;
-    auto kern = block == 128 ? (regs > 0 ? k_knnf<64, 32, 7, 128, 3> : k_knnf<64, 32, 7, 128, 4>)
-                             : (regs > 0 ? k_knnf<64, 32, 7, 64, 6> : k_knnf<64, 32, 7, 64, 8>);
-    PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    unsigned blocks = (unsigned)((P.nq + block - 1) / block);
-    PPP_LAUNCH(ctx, P.normals ? "knn_normals" : "knn", kern, blocks, block, smem, P);
-    PPP_CHECK_LAUNCH();
-    st = PPP_OK;
-  }
-  else if (P.cap <= 32) {   // external query arrays (not in cell order), or PPP_KNN32_OLD: composite keys
-    const int block = 64;
-    size_t smem = (size_t)48 * 8 * block;
-    auto kern = k_knn32c<64>;
-    unsigned blocks = (unsigned)((P.nq + block - 1) / block);
-    PPP_LAUNCH(ctx, P.normals ? "knn_normals" : "knn", kern, blocks, block, smem, P);
-    PPP_CHECK_LAUNCH();
-    st = PPP_OK;
-  }
-  else st = launch_knn_fast_k<64, 16, false>(c, P);   // external query arrays with 32 < k <= 64, or PPP_KNN64_OLD: 64-bit keys
-  if (st == PPP_OK) {
+    return PPP_OK;
+  };
+  if (P.cap <= 16) PPP_TRY(launch(ext ? k_knn16f<128, 8, 7, true> : k_knn16f<128, 8, 7, false>, F_SLOTS));
+  else if (P.cap <= 32) PPP_TRY(launch(ext ? k_knnf<32, 16, 6, 128, 6, true> : k_knnf<32, 16, 6, 128, 6, false>, 32 + 16));
+  else PPP_TRY(launch(ext ? k_knnf<64, 32, 7, 128, 4, true> : k_knnf<64, 32, 7, 128, 4, false>, 64 + 32));
+  {
     // hand-over queries: one warp each, persistent warps (their number is only known on the device)
     P.use_redo = 1;
     size_t smem = (size_t)WARPQ_WARPS * 32 * P.cap * 8;
@@ -2034,14 +1336,14 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
     PPP_LAUNCH(ctx, "knn_redo", k_knn_warp, blocks, WARPQ_WARPS * 32, smem, P);
     PPP_CHECK_LAUNCH();
   }
-  if (st == PPP_OK && getenv("PPP_DEBUG")) {
+  if (getenv("PPP_DEBUG")) {
     int32_t n_redo = 0;
     fetch_small(ctx, redo, 4, &n_redo);
     fprintf(stderr, "[ppp] knn fast path: %lld queries, %d handed to the ring-expanding kernel (h=%g, R0=%d)\n",
             (long long)P.nq, n_redo, (double)P.g.h, P.R0);
   }
   dev_free(ctx, redo);
-  return st;
+  return PPP_OK;
 }
 
 int knn_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f, int64_t first, int k,
@@ -2050,7 +1352,7 @@ int knn_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq
   ppp_ctx* ctx = c->ctx;
   SearchParams P{};
   P.g = gs.v; P.xyz4 = c->xyz4; P.q = q_dev; P.q_sf = q_stride_f; P.nq = nq; P.first = first;
-  P.cap = k; P.kk = (int)std::min<int64_t>(k, c->n_finite); P.mode = 0; P.R0 = knn_block_rings(); P.r2 = 0;
+  P.cap = k; P.kk = (int)std::min<int64_t>(k, c->n_finite); P.mode = 0; P.R0 = PPP_KNN_RINGS; P.r2 = 0;
   P.idx_out = idx_dev; P.d2_out = d2_dev; P.offsets = nullptr;
   P.normals = with_normals ? normals_dev : nullptr; P.nsf = normal_stride_f; P.nmap = c->nmap; P.route = c->route;
   P.vpx = vp ? vp[0] : 0; P.vpy = vp ? vp[1] : 0; P.vpz = vp ? vp[2] : 0; P.flags = flags;
@@ -2061,7 +1363,7 @@ int knn_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq
                P.normals, normal_stride_f, c->nmap, c->route);
     PPP_CHECK_LAUNCH();
   }
-  if (k <= 64 && nq > 0 && !getenv("PPP_KNN_GENERIC")) return launch_knn_fast(c, P);
+  if (k <= 64 && nq > 0) return launch_knn_fast(c, P);
   return launch_search(c, P);
 }
 
@@ -2123,7 +1425,7 @@ int normals_radius_launch(ppp_cloud* c, const GridStore& gs, int64_t first, int6
   // expected neighbours per query from the surface density; the fixed-capacity fast kernel pays
   // off while most queries stay within its 32-entry lists
   const double expect = c->density * 3.14159265358979 * (double)r2;
-  const bool fast = expect <= 24.0 && !getenv("PPP_KNN_GENERIC");
+  const bool fast = expect <= 24.0;
   int32_t* redo = nullptr;
   int n_redo = 0;
   if (fast) {

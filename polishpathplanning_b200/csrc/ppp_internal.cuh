@@ -102,6 +102,9 @@ struct NormalRoute {
 // the range test), at most PPP_SORTED_PAD - 1 records beyond the end of a row.
 constexpr int PPP_SORTED_PAD = 160;
 
+// Rings of cells in the fixed candidate block of the fast k-nearest kernels (2: a 5 x 5 block).
+constexpr int PPP_KNN_RINGS = 2;
+
 struct GridStore {
   GridView v{};
   int drop = 2;              // the axis this grid does NOT span (2: cells over x, y)
@@ -336,7 +339,6 @@ int cloud_decide_projection(ppp_cloud* c, const GridStore& g);
 // The three grids of cell size h and the per-point choice for candidate blocks of (2*R0+1)^2 cells.
 int cloud_get_mp(ppp_cloud* c, double h, int R0, MPSet** out);
 double cloud_cell_for_k(const ppp_cloud* c, int k);
-int knn_block_rings();
 double cloud_cell_for_radius(const ppp_cloud* c, double r);
 
 // knn.cu
