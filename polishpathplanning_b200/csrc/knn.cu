@@ -48,6 +48,21 @@ struct SearchParams {
   int my_proj;
 };
 
+// Query t: row t of the query array P.q (ext), or the t-th of the cloud's own points in cell order, whose row is its
+// original index.
+__device__ __forceinline__ void load_query(const SearchParams& P, bool ext, int64_t t, float& qx, float& qy, float& qz,
+                                           int64_t& row) {
+  if (ext) {
+    const float* qp = P.q + t * P.q_sf;
+    qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
+    row = t;
+  } else {
+    float4 p = __ldg(P.g.sorted + P.first + t);
+    qx = p.x; qy = p.y; qz = p.z;
+    row = __float_as_int(p.w);
+  }
+}
+
 // Self-query `row` belongs to this launch?  (Warps none of whose lanes do leave at once.)
 __device__ __forceinline__ bool query_is_mine(const SearchParams& P, bool valid, int64_t row) {
   return valid && (P.choice == nullptr || __ldg(P.choice + row) == P.my_proj);
@@ -78,15 +93,7 @@ __global__ void __launch_bounds__(128) k_search(SearchParams P) {
   const GridView& g = P.g;
   float qx, qy, qz;
   int64_t row;
-  if (P.q) {
-    const float* qp = P.q + t * P.q_sf;
-    qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-    row = t;
-  } else {
-    float4 p = __ldg(g.sorted + P.first + t);
-    qx = p.x; qy = p.y; qz = p.z;
-    row = __float_as_int(p.w);
-  }
+  load_query(P, P.q != nullptr, t, qx, qy, qz, row);
   if (!P.use_redo && P.choice && __ldg(P.choice + row) != P.my_proj) return;
   u64* L = s_keys + threadIdx.x;
   int cnt = 0;
@@ -169,272 +176,41 @@ __global__ void __launch_bounds__(128) k_search(SearchParams P) {
 
 
 // ---------------------------------------------------------------------------------------------
-// k <= 16: 32-bit FIXED-POINT keys.  The queries are the cloud's own points in cell order or, with EXT, a query
+// k <= 64: 32-bit FIXED-POINT keys.  The queries are the cloud's own points in cell order or, with EXT, a query
 // array (its row t is the query's position); only the load of the query differs.
-//     key = floor(d2 * scale) << 10 | ordinal         scale = (2^22 - margin) / (ring bound)^2  per query
+//     key = floor(d2 * scale) << SH | ordinal         scale = (2^(32 - SH) - margin) / (ring bound)^2  per query
 // Candidates arrive uniformly in d2 (area), so 22 bits of fixed point over [0, bound^2] resolve the k-th
 // neighbourhood nearly as finely as the float itself does (2.2e-6 mm^2 at cfg2 against an ulp of 4.8e-7), where a
-// truncated float spends its bits on the nearest neighbours.  The ordinal names the candidate by (row of the
-// block, slot in the row); its sorted position is rebuilt from the row start at the very end, and the exact d2
-// -- needed only if the caller asked for distances -- is recomputed from the gathered record with the same
-// arithmetic.  So the per-thread store is 4 bytes per slot, the sorted words ARE the result, and from the second
-// flush on slots 0..15 are already in order, so a flush is a 16-input sort of the newcomers, one row of minima and
-// a 16-input bitonic merge.  Two candidates whose keys agree in the upper 22 bits (including the best one just
-// dropped) leave their order to the exact hand-over kernel k_knn_warp.  floor(d2 * scale) is one FFMA.RZ against
-// 2^23 (exact floor of the real product: monotone in d2).
+// truncated float spends its bits on the nearest neighbours.  The ordinal (SH = 3 + RB bits) names the candidate by
+// (row of the block, slot in the row); its sorted position is rebuilt from the row start at the very end, and the
+// exact d2 -- needed only if the caller asked for distances -- is recomputed from the gathered record with the same
+// arithmetic.  So the per-thread store is 4 bytes per slot and the sorted words ARE the result.  floor(d2 * scale) is
+// one FFMA.RZ against 2^23 (exact floor of the real product: monotone in d2).
+// Slots 0..K-1 hold the K best so far in order (free values behind the keys), slots K..K+NEW-1 take the newcomers; a
+// flush sorts the newcomers, folds them into the kept K with one row of minima (the half-cleaner of a bitonic merge)
+// and a K-input bitonic merge, every exchange one unsigned min + one unsigned max, and writes the K words back.
+// Before the first flush the newcomers start at slot FIRST: FIRST = K leaves slots 0..K-1 to the free values, which
+// are in order from the start; FIRST = 0 uses all K + NEW slots for them, and the first flush sorts slots 0..K-1 too.
+// Two candidates whose keys agree in the fixed-point bits (including the best one just dropped) leave their order to
+// the exact hand-over kernel k_knn_warp.
+//   K = 16: 16 newcomers, FIRST = 0, ordinals of 3 + 7 bits (rows of up to 128 candidates), 22 bits of d2.
+//   K = 32: 16 newcomers (63 + 80 exchanges per flush), ordinals of 3 + 6 bits, 23 bits of d2.
+//   K = 64: 32 newcomers (191 + 192 exchanges), ordinals of 3 + 7 bits, 22 bits of d2 -- the list lives in 96
+//   registers during a flush.
 // ---------------------------------------------------------------------------------------------
-constexpr int F_SLOTS = 32;
 constexpr int F_MAXR = 3;
 static_assert(PPP_KNN_RINGS <= F_MAXR, "the ordinal names the block row in 3 bits: 2 R0 + 1 <= 7");
-// RB (template parameter of k_knn16f): bits of the ordinal that name the slot inside a cell row (3 more name the row,
-// 2R+1 <= 7).  RB = 7: rows of up to 128 candidates, 22 bits of d2.
 
-template <int BD, int MB, int F_RB, bool EXT>
-__global__ void __launch_bounds__(BD, MB) k_knn16f(SearchParams P) {
-  pdl_prologue();
-  extern __shared__ __align__(128) unsigned s_fkeys[];
-  constexpr int K = 16;
-  constexpr int PPP_ASSERT_SLOTS = F_SLOTS;
-  constexpr int F_ROWCAP = 1 << F_RB;      // candidates per cell row an ordinal can name; denser rows take the exact path
-  constexpr int F_SH = 3 + F_RB;
-  constexpr unsigned F_OMASK = (1u << F_SH) - 1u;
-  constexpr unsigned F_FIXTOP = 1u << (32 - F_SH);   // fixed-point values stay below F_FIXTOP - 608
-  static_assert(F_ROWCAP + 4 <= PPP_SORTED_PAD, "unclamped candidate loads run up to F_ROWCAP + 3 records past a row");
-  // A free slot j holds FREE(j): above every key (fixed-point values stop 608 below F_FIXTOP), and distinct in the
-  // fixed-point bits from every other free slot, so free slots never look like an undecided pair.  Slots fill in
-  // order, a flush keeps the smallest free values FREE(ns..15) exactly where they were: the invariant holds.
-#define F_FREE(j) (((F_FIXTOP - 128u + (unsigned)(j)) << F_SH) | F_OMASK)
-  constexpr unsigned FREE0 = F_FREE(0);
-  const GridView& g = P.g;
-  const int64_t t = (int64_t)blockIdx.x * BD + threadIdx.x;
-  bool valid = t < P.nq;
-  float qx = 0.f, qy = 0.f, qz = 0.f;
-  int64_t row = 0;
-  if (valid) {
-    if (EXT) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
-  }
-  valid = query_is_mine(P, valid, row);
-  if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
-  const bool fin = valid && finite3(qx, qy, qz);
-  const bool act = fin && g.n_sorted > 0;
-  unsigned* keys = s_fkeys + threadIdx.x;                       // slot j of this thread at keys[j * BD]
-  int* rows = (int*)(s_fkeys + F_SLOTS * BD) + threadIdx.x;     // first sorted position of block row j at rows[j * BD]
-  const unsigned keys_sa = (unsigned)__cvta_generic_to_shared(keys);
-  constexpr unsigned SLOT_B = BD * 4;
-  const int R = P.R0;
-  int cu = 0, cv = 0;
-  float tau = -1.0f, scale = 0.0f;   // inactive lanes accept nothing
-  if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
-    tau = ring_bound2(g, R, cu, cv);
-    // d2 <= tau  =>  d2 * scale < F_FIXTOP - 608
-    scale = tau > 0.0f ? fminf(__fdiv_rd((float)(F_FIXTOP - 608u), tau), 3.0e38f) : 0.0f;
-  }
-#pragma unroll
-  for (int i = 0; i < F_SLOTS; i++) keys[i * BD] = F_FREE(i);   // a flush needs no masks
-  const u64 qxy = pack2(qx, qy);
-  int ns = 0;              // next slot to fill
-  bool ambiguous = false, overflow = false;
-  bool in_order = false;   // slots 0..15 are sorted (warp-uniform: flushes are)
-
-  auto flush = [&]() {
-    unsigned a[16], b[16];
-#pragma unroll
-    for (int i = 0; i < 16; i++) { a[i] = keys[i * BD]; b[i] = keys[(16 + i) * BD]; }
-    if (!in_order) SortNetU32<16>::sort(a);
-    SortNetU32<16>::sort(b);
-    // half-cleaner of the bitonic merge: the 16 smallest end up in a (bitonic), the others in b
-    unsigned drop = 0xFFFFFFFFu;
-#pragma unroll
-    for (int i = 0; i < 16; i++) {
-      const unsigned lo = min(a[i], b[15 - i]);
-      drop = min(drop, max(a[i], b[15 - i]));
-      a[i] = lo;
-    }
-    SortNetU32<16>::bitonic_merge(a);
-    // equal upper 23 bits among the kept 16 or between the 16th and the best one dropped: the fixed-point key does
-    // not decide their order
-    ambiguous |= (a[15] ^ drop) <= F_OMASK;
-#pragma unroll
-    for (int i = 0; i + 1 < 16; i++) ambiguous |= (a[i] ^ a[i + 1]) <= F_OMASK;
-#pragma unroll
-    for (int i = 0; i < 16; i++) { keys[i * BD] = a[i]; keys[(16 + i) * BD] = F_FREE(16 + i); }
-    // every d2 whose key could still sort at or before the 16th: floor(d2 * scale) <= F  =>  d2 < (F + 1) / scale
-    if (a[15] < FREE0) tau = fminf(tau, __fdiv_ru((float)((a[15] >> F_SH) + 1u), scale));
-    // newcomers go to slots 16.. from now on, also when fewer than 16 slots hold keys: slots 0..15 (keys, then free
-    // values) stay in order
-    ns = K;
-    in_order = true;
-  };
-
-  constexpr int U = 4;
-#pragma unroll 1
-  for (int j = 0; j <= 2 * R + 1; j++) {
-    const int dv = (j & 1) ? -((j + 1) >> 1) : (j >> 1);  // rows nearest first
-    int s = 0, cnt = 0;
-    const int v = cv + dv;
-    const bool drain = j == 2 * R + 1;
-    if (!drain && act && v >= 0 && v < g.nv) {
-      int a = max(cu - R, 0), b = min(cu + R, g.nu - 1);
-      if (a <= b) {
-        const int32_t* rowp = g.cell_start + (int64_t)v * g.nu;
-        s = __ldg(rowp + a);
-        cnt = __ldg(rowp + b + 1) - s;
-      }
-    }
-    if (!drain) rows[j * BD] = s;
-    if (cnt > F_ROWCAP) { overflow = true; cnt = F_ROWCAP; }   // the ordinal cannot name more: exact path
-    const int n_it = (__reduce_max_sync(0xffffffffu, cnt) + U - 1) / U + (drain ? 1 : 0);
-    // flush when some lane could run out of slots in the next iteration; the drain row flushes once
-    const int trig = min(F_SLOTS - U, (2 * R + 1 - j) * F_SLOTS - 1);
-    unsigned wsa = keys_sa + (unsigned)ns * SLOT_B;
-    const unsigned trig_sa = keys_sa + (unsigned)trig * SLOT_B;
-    int i0 = s;
-    int rem = cnt;   // candidates of this lane's row not yet looked at
-    unsigned ord = (unsigned)j << F_RB;
-#pragma unroll 1
-    for (int it = 0; it < n_it; it++, i0 += U, ord += U, rem -= U) {
-      float4 c4[U];
-      PPP_DEV_ASSERT(i0 >= 0 && i0 + U - 1 < g.n_sorted + PPP_SORTED_PAD);
-#pragma unroll
-      for (int u = 0; u < U; u++) c4[u] = __ldg(g.sorted + (i0 + u));   // never clamped: see PPP_SORTED_PAD
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        const float d2 = d2_flann_x2(qxy, qz, c4[u]);
-        if (u < rem && d2 <= tau) {
-          // (bits << F_SH) + ordinal: the exponent bits of 2^23 leave at the top; one IMAD (+ an add of u)
-          const unsigned key = __float_as_uint(__fmaf_rz(d2, scale, 8388608.0f)) * (1u << F_SH) + ord + (unsigned)u;
-          PPP_DEV_ASSERT(wsa >= keys_sa && wsa < keys_sa + (unsigned)(PPP_ASSERT_SLOTS) * SLOT_B);
-          asm volatile("st.shared.b32 [%0], %1;" ::"r"(wsa), "r"(key) : "memory");
-          wsa += SLOT_B;
-        }
-      }
-      if (__any_sync(0xffffffffu, wsa > trig_sa)) {
-        ns = (int)((wsa - keys_sa) / SLOT_B);
-        flush();
-        wsa = keys_sa + (unsigned)ns * SLOT_B;
-      }
-    }
-    ns = (int)((wsa - keys_sa) / SLOT_B);
-  }
-  if (!valid) return;
-  // slots 0..15 now hold the 16 smallest keys in order (padded with free values)
-  const int kk = P.kk;
-  bool complete = !act || kk == 0;
-  if (!complete) complete = keys[(kk - 1) * BD] < FREE0;
-  if (!complete || ambiguous || overflow) {
-    P.redo_list[atomicAdd(P.redo_count, 1)] = (int32_t)t;
-    return;
-  }
-  const int k = P.cap;
-  int m = 0;  // neighbours found: keys come first in slots 0..15, so four probes find their number
-  if (act) {
-    if (keys[15 * BD] < FREE0) {
-      m = 16;
-    } else {
-      if (keys[7 * BD] < FREE0) m = 8;
-      if (keys[(m + 3) * BD] < FREE0) m += 4;
-      if (keys[(m + 1) * BD] < FREE0) m += 2;
-      if (keys[m * BD] < FREE0) m += 1;
-    }
-    m = min(m, k);
-  }
-  int32_t* io = P.idx_out ? P.idx_out + row * (int64_t)k : nullptr;
-  float* dout = (P.idx_out && P.d2_out) ? P.d2_out + row * (int64_t)k : nullptr;
-  const bool al32 = k == K && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 31) == 0;
-  const bool al16 = (k & 3) == 0 && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 15) == 0;
-  const bool want_n = P.normals && fin && m >= 3;
-  const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-  float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  float kx = 0.f, ky = 0.f, kz = 0.f;
-  // eight neighbours at a time; ONE gather of the neighbour's sorted record serves the id list, the covariance
-  // and (if asked for) the exact distance
-#pragma unroll
-  for (int jb = 0; jb < K; jb += 8) {
-    if (jb >= k) break;
-    float4 nb[8];
-#pragma unroll
-    for (int u = 0; u < 8; u++) {
-      const unsigned key = keys[(jb + u) * BD];
-      const bool has = jb + u < m;
-      nb[u] = make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
-      if (has) {   // a free value names no row
-        const int rj = (int)((key >> F_RB) & 7u), pos = rows[rj * BD] + (int)(key & (unsigned)(F_ROWCAP - 1));
-        PPP_DEV_ASSERT(rj <= 2 * R && pos >= 0 && pos < g.n_sorted);
-        nb[u] = __ldg(g.sorted + pos);
-      }
-    }
-    if (io) {
-      float dd[8];
-      if (dout) {
-#pragma unroll
-        for (int u = 0; u < 8; u++) dd[u] = jb + u < m ? d2_flann(qx, qy, qz, nb[u].x, nb[u].y, nb[u].z) : CUDART_INF_F;
-      }
-      if (al32) {
-        // a full row is 64 contiguous, 32-byte aligned bytes: two 256-bit stores instead of sixteen 32-bit ones
-        st_global_256(io + jb, nb[0].w, nb[1].w, nb[2].w, nb[3].w, nb[4].w, nb[5].w, nb[6].w, nb[7].w);
-        if (dout) {
-          reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-          reinterpret_cast<float4*>(dout + jb)[1] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        }
-      } else if (al16) {
-        // k = 4, 8, 12: rows are still 16-byte aligned
-        reinterpret_cast<float4*>(io + jb)[0] = make_float4(nb[0].w, nb[1].w, nb[2].w, nb[3].w);
-        if (dout) reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
-        if (jb + 4 < k) {
-          reinterpret_cast<float4*>(io + jb)[1] = make_float4(nb[4].w, nb[5].w, nb[6].w, nb[7].w);
-          if (dout) reinterpret_cast<float4*>(dout + jb)[1] = make_float4(dd[4], dd[5], dd[6], dd[7]);
-        }
-      } else {
-#pragma unroll
-        for (int u = 0; u < 8; u++) {
-          if (jb + u < k) {
-            io[jb + u] = __float_as_int(nb[u].w);
-            if (dout) dout[jb + u] = dd[u];
-          }
-        }
-      }
-    }
-    if (want_n) {
-      if (jb == 0 && shifted) { kx = nb[0].x; ky = nb[0].y; kz = nb[0].z; }
-#pragma unroll
-      for (int u = 0; u < 8; u++) {
-        if (jb + u < m) {
-          float x = nb[u].x, y = nb[u].y, z = nb[u].z;
-          if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-          accumulate_point(acc, x, y, z);
-        }
-      }
-    }
-  }
-  if (P.normals) {
-    float o[4];
-    if (want_n) normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    else o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-  }
+// Free value of slot j with SH ordinal bits: above every key (fixed-point values stay below 2^(32 - SH) - 608), and
+// distinct in the fixed-point bits from every other free slot, so free slots never look like an undecided pair.
+template <int SH>
+__device__ constexpr unsigned free_word(int j) {
+  return (((1u << (32 - SH)) - 128u + (unsigned)j) << SH) | ((1u << SH) - 1u);
 }
 
-// ---------------------------------------------------------------------------------------------
-// 16 < k <= 64: the fixed-point keys of k_knn16f (queries from the cloud or, with EXT, from a query array) with a
-// MERGE instead of a full sort.  Slots 0..K-1 hold the K best so far in order (free values behind the keys), slots
-// K..K+NEW-1 take the newcomers; a flush sorts the newcomers, folds them into the kept K with one row of minima (the
-// half-cleaner of a bitonic merge) and a K-input bitonic merge, every exchange one unsigned min + one unsigned max,
-// and writes the K words back.  K = 32: 16 newcomers (63 + 80 exchanges per flush), ordinals of 3 + 6 bits, 23 bits
-// of d2.  K = 64: 32 newcomers (191 + 192 exchanges), ordinals of 3 + 7 bits (rows of up to 128 candidates), 22 bits
-// of d2 -- the list lives in 96 registers during a flush.
-// ---------------------------------------------------------------------------------------------
-template <int K, int NEW, int RB, int BD, int MB, bool EXT>
+template <int K, int NEW, int RB, int BD, int MB, int FIRST, bool EXT>
 __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
+  static_assert(FIRST == 0 || FIRST == K, "newcomers start at slot 0 or behind the kept K");
   pdl_prologue();
   extern __shared__ __align__(128) unsigned s_fkeys[];
   constexpr int SLOTS = K + NEW;
@@ -445,24 +221,13 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   constexpr int ROWCAP = 1 << RB;
   static_assert(ROWCAP + 4 <= PPP_SORTED_PAD, "unclamped candidate loads run up to ROWCAP + 3 records past a row");
   static_assert(SLOTS <= 128, "free values are FIXTOP - 128 + slot");
-#define F32_FREE(j) (((FIXTOP - 128u + (unsigned)(j)) << SH) | OMASK)
-  constexpr unsigned FREE0 = F32_FREE(0);
+  constexpr unsigned FREE0 = free_word<SH>(0);
   const GridView& g = P.g;
   const int64_t t = (int64_t)blockIdx.x * BD + threadIdx.x;
   bool valid = t < P.nq;
   float qx = 0.f, qy = 0.f, qz = 0.f;
   int64_t row = 0;
-  if (valid) {
-    if (EXT) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
-  }
+  if (valid) load_query(P, EXT, t, qx, qy, qz, row);
   valid = query_is_mine(P, valid, row);
   if (P.choice && !__any_sync(0xffffffffu, valid)) return;   // none of this warp's points chose this projection
   const bool fin = valid && finite3(qx, qy, qz);
@@ -482,10 +247,11 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
     scale = tau > 0.0f ? fminf(__fdiv_rd((float)(FIXTOP - 608u), tau), 3.0e38f) : 0.0f;   // d2 <= tau  =>  d2 * scale < FIXTOP - 608
   }
 #pragma unroll
-  for (int i = 0; i < SLOTS; i++) keys[i * BD] = F32_FREE(i);   // ascending: slots 0..K-1 are "in order" from the start
+  for (int i = 0; i < SLOTS; i++) keys[i * BD] = free_word<SH>(i);   // ascending: slots 0..K-1 are "in order" from the start
   const u64 qxy = pack2(qx, qy);
   bool ambiguous = false, overflow = false;
-  unsigned wsa = keys_sa + (unsigned)K * SLOT_B;     // cursor in the newcomers' region
+  bool in_order = FIRST == K;   // slots 0..K-1 are sorted (warp-uniform: flushes are)
+  unsigned wsa = keys_sa + (unsigned)FIRST * SLOT_B;   // cursor of the newcomers
 
   auto flush = [&]() {
     unsigned b[NEW];
@@ -495,6 +261,10 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
     unsigned a[K];
 #pragma unroll
     for (int i = 0; i < K; i++) a[i] = keys[i * BD];
+    if constexpr (FIRST == 0) {
+      if (!in_order) SortNetU32<K>::sort(a);
+      in_order = true;
+    }
     // kept (ascending) ++ newcomers (descending) is bitonic: the half-cleaner leaves the K smallest in a[]; the
     // smallest of what it discards is the (K+1)-th of the union
     unsigned next = 0xFFFFFFFFu;
@@ -513,8 +283,10 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
 #pragma unroll
     for (int i = 0; i < K; i++) keys[i * BD] = a[i];
 #pragma unroll
-    for (int i = 0; i < NEW; i++) keys[(K + i) * BD] = F32_FREE(K + i);
+    for (int i = 0; i < NEW; i++) keys[(K + i) * BD] = free_word<SH>(K + i);
+    // newcomers go to slots K.. from now on, also when fewer than K slots hold keys: slots 0..K-1 stay in order
     wsa = keys_sa + (unsigned)K * SLOT_B;
+    // every d2 whose key could still sort at or before the kk-th: floor(d2 * scale) <= F  =>  d2 < (F + 1) / scale
     if (kk > 0) {
       const unsigned kth = keys[(kk - 1) * BD];
       if (kth < FREE0) tau = fminf(tau, __fdiv_ru((float)((kth >> SH) + 1u), scale));
@@ -591,13 +363,18 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
   float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
   float kx = 0.f, ky = 0.f, kz = 0.f;
-#pragma unroll 1
-  for (int jb = 0; jb < k; jb += 8) {
+  // eight neighbours at a time; ONE gather of the neighbour's sorted record serves the id list, the covariance
+  // and (if asked for) the exact distance.  K = 16 unrolls its two blocks of eight (the rolled loop spills twice as
+  // much there); K = 32 / 64 keep one copy of the loop body.
+  constexpr bool UNROLL = K <= 16;
+#pragma unroll (UNROLL ? K / 8 : 1)
+  for (int jb = 0; jb < (UNROLL ? K : k); jb += 8) {
+    if (UNROLL && jb >= k) break;
     float4 nb[8];
 #pragma unroll
     for (int u = 0; u < 8; u++) {
       nb[u] = make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
-      if (jb + u < m) {
+      if (jb + u < m) {   // a free value names no row
         const unsigned key = keys[(jb + u) * BD];
         const int rj = (int)((key >> RB) & 7u), pos = rows[rj * BD] + (int)(key & (unsigned)(ROWCAP - 1));
         PPP_DEV_ASSERT(rj <= 2 * R && pos >= 0 && pos < g.n_sorted);
@@ -611,6 +388,7 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
         for (int u = 0; u < 8; u++) dd[u] = jb + u < m ? d2_flann(qx, qy, qz, nb[u].x, nb[u].y, nb[u].z) : CUDART_INF_F;
       }
       if (al32) {
+        // rows of a multiple of 8 neighbours are 32-byte aligned: one 256-bit store per eight ids instead of eight
         st_global_256(io + jb, nb[0].w, nb[1].w, nb[2].w, nb[3].w, nb[4].w, nb[5].w, nb[6].w, nb[7].w);
         if (dout) {
           reinterpret_cast<float4*>(dout + jb)[0] = make_float4(dd[0], dd[1], dd[2], dd[3]);
@@ -777,7 +555,7 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// Ring-expanding k-nearest search, one WARP per query: the hand-over path of k_knn16f and k_knnf (sparse
+// Ring-expanding k-nearest search, one WARP per query: the hand-over path of k_knnf (sparse
 // regions, cloud borders, near-ties, dense rows; typically well under 1% of the queries).  The 32 lanes stride over the
 // candidates of each ring (coalesced), each lane keeps its own sorted list of at most k keys in
 // shared memory, and after every ring the k smallest of the 32 lists are extracted with warp-wide
@@ -812,15 +590,7 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
   const int64_t t = P.redo_list[slot];
   float qx, qy, qz;
   int64_t row;
-  if (P.q) {
-    const float* qp = P.q + t * P.q_sf;
-    qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-    row = t;
-  } else {
-    float4 p = __ldg(g.sorted + P.first + t);
-    qx = p.x; qy = p.y; qz = p.z;
-    row = __float_as_int(p.w);
-  }
+  load_query(P, P.q != nullptr, t, qx, qy, qz, row);
   const int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
   const int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
   int cnt = 0;
@@ -1054,15 +824,7 @@ __global__ void __launch_bounds__(128) k_radius_count(SearchParams P, int32_t* _
     const GridView& g = P.g;
     float qx, qy, qz;
     int64_t row;
-    if (P.q) {
-      const float* qp = P.q + t * P.q_sf;
-      qx = __ldg(qp); qy = __ldg(qp + 1); qz = __ldg(qp + 2);
-      row = t;
-    } else {
-      float4 p = __ldg(g.sorted + P.first + t);
-      qx = p.x; qy = p.y; qz = p.z;
-      row = __float_as_int(p.w);
-    }
+    load_query(P, P.q != nullptr, t, qx, qy, qz, row);
     const bool mine = P.use_redo || P.choice == nullptr || P.q != nullptr || __ldg(P.choice + row) == P.my_proj;
     if (mine && finite3(qx, qy, qz) && g.n_sorted > 0) {
       int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
@@ -1322,9 +1084,9 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
     PPP_CHECK_LAUNCH();
     return PPP_OK;
   };
-  if (P.cap <= 16) PPP_TRY(launch(ext ? k_knn16f<128, 8, 7, true> : k_knn16f<128, 8, 7, false>, F_SLOTS));
-  else if (P.cap <= 32) PPP_TRY(launch(ext ? k_knnf<32, 16, 6, 128, 6, true> : k_knnf<32, 16, 6, 128, 6, false>, 32 + 16));
-  else PPP_TRY(launch(ext ? k_knnf<64, 32, 7, 128, 4, true> : k_knnf<64, 32, 7, 128, 4, false>, 64 + 32));
+  if (P.cap <= 16) PPP_TRY(launch(ext ? k_knnf<16, 16, 7, 128, 8, 0, true> : k_knnf<16, 16, 7, 128, 8, 0, false>, 16 + 16));
+  else if (P.cap <= 32) PPP_TRY(launch(ext ? k_knnf<32, 16, 6, 128, 6, 32, true> : k_knnf<32, 16, 6, 128, 6, 32, false>, 32 + 16));
+  else PPP_TRY(launch(ext ? k_knnf<64, 32, 7, 128, 4, 64, true> : k_knnf<64, 32, 7, 128, 4, 64, false>, 64 + 32));
   {
     // hand-over queries: one warp each, persistent warps (their number is only known on the device)
     P.use_redo = 1;

@@ -1,7 +1,7 @@
 """External-query searches and the kernels built on them, against the brute-force numpy references
 (tests/golden/query_numpy.py) and the CPU oracle.
 
-- kNN with a query array through every route: k_knn16f (k <= 16), k_knnf<32,16> (17..32), k_knnf<64,32> (33..64),
+- kNN with a query array through every route: k_knnf<16,16> (k <= 16), k_knnf<32,16> (17..32), k_knnf<64,32> (33..64),
   k_search (k > 64) and the one-warp-per-query hand-over kernel; index lists and d² bits must be identical, for
   every query stride.
 - Radius search with a query array, counts-only against fill, strict d² < r², the fill call's list limit.
