@@ -310,8 +310,8 @@ struct G3 { GridView g[3]; };
 
 // Points in the (2R+1)^2 cell block around p in grid g.
 __device__ __forceinline__ int block_population(const GridView& g, float x, float y, float z, int R) {
-  const int cu = cell_coord_raw(axis_of(x, y, z, g.au), g.min_u, g.inv_h);
-  const int cv = cell_coord_raw(axis_of(x, y, z, g.av), g.min_v, g.inv_h);
+  int cu, cv;
+  query_cell(g, x, y, z, cu, cv);
   const int a = max(cu - R, 0), b = min(cu + R, g.nu - 1);
   if (a > b) return 0;
   int cnt = 0;

@@ -99,8 +99,8 @@ __global__ void __launch_bounds__(128) k_search(SearchParams P) {
   int cnt = 0;
   const bool fin = finite3(qx, qy, qz);
   if (fin && g.n_sorted > 0) {
-    int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+    int cu, cv;
+    query_cell(g, qx, qy, qz, cu, cv);
     if (P.mode == 1) {
       u64 tau = make_key(P.r2, 0);
       visit_annulus(g, cu, cv, -1, P.R0, [&](float4 c) {
@@ -151,26 +151,9 @@ __global__ void __launch_bounds__(128) k_search(SearchParams P) {
     }
   }
   if (P.normals) {
-    float o[4];
-    if (!fin || cnt < 3) {
-      o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    } else {
-      float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      float kx = 0.f, ky = 0.f, kz = 0.f;
-      const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-      if (shifted) {
-        float4 f = __ldg(P.xyz4 + key_idx(L[0]));
-        kx = f.x; ky = f.y; kz = f.z;
-      }
-      for (int j = 0; j < cnt; j++) {
-        float4 a = __ldg(P.xyz4 + key_idx(L[j * BD]));
-        float x = a.x, y = a.y, z = a.z;
-        if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-        accumulate_point(acc, x, y, z);
-      }
-      normal_from_accumulators(acc, cnt, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    }
-    store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
+    CovAcc cov(P.flags);
+    for (int j = 0; j < cnt; j++) cov.add(__ldg(P.xyz4 + key_idx(L[j * BD])));
+    cov.finish(P, fin, row, qx, qy, qz);
   }
 }
 
@@ -241,8 +224,7 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   int cu = 0, cv = 0;
   float tau = -1.0f, scale = 0.0f;   // inactive lanes accept nothing
   if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+    query_cell(g, qx, qy, qz, cu, cv);
     tau = ring_bound2(g, R, cu, cv);
     scale = tau > 0.0f ? fminf(__fdiv_rd((float)(FIXTOP - 608u), tau), 3.0e38f) : 0.0f;   // d2 <= tau  =>  d2 * scale < FIXTOP - 608
   }
@@ -360,9 +342,7 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
   float* dout = (P.idx_out && P.d2_out) ? P.d2_out + row * (int64_t)k : nullptr;
   const bool al32 = (k & 7) == 0 && (((uintptr_t)P.idx_out | (uintptr_t)P.d2_out) & 31) == 0;
   const bool want_n = P.normals && fin && m >= 3;
-  const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-  float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  float kx = 0.f, ky = 0.f, kz = 0.f;
+  CovAcc cov(P.flags);
   // eight neighbours at a time; ONE gather of the neighbour's sorted record serves the id list, the covariance
   // and (if asked for) the exact distance.  K = 16 unrolls its two blocks of eight (the rolled loop spills twice as
   // much there); K = 32 / 64 keep one copy of the loop body.
@@ -405,23 +385,17 @@ __global__ void __launch_bounds__(BD, MB) k_knnf(SearchParams P) {
       }
     }
     if (want_n) {
-      if (jb == 0 && shifted) { kx = nb[0].x; ky = nb[0].y; kz = nb[0].z; }
 #pragma unroll
       for (int u = 0; u < 8; u++) {
         if (jb + u < m) {
-          float x = nb[u].x, y = nb[u].y, z = nb[u].z;
-          if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-          accumulate_point(acc, x, y, z);
+          // adds come in slot order: telling the compiler so lets the unrolled loop drop the origin test
+          if (UNROLL) __builtin_assume(cov.m == jb + u);
+          cov.add(nb[u]);
         }
       }
     }
   }
-  if (P.normals) {
-    float o[4];
-    if (want_n) normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    else o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
-  }
+  if (P.normals) cov.finish(P, fin, row, qx, qy, qz);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -448,11 +422,7 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
   bool valid = t < P.nq;
   float qx = 0.f, qy = 0.f, qz = 0.f;
   int64_t row = 0;
-  if (valid) {
-    float4 p = __ldg(g.sorted + P.first + t);
-    qx = p.x; qy = p.y; qz = p.z;
-    row = __float_as_int(p.w);
-  }
+  if (valid) load_query(P, false, t, qx, qy, qz, row);
   valid = query_is_mine(P, valid, row);
   if (P.choice && !__any_sync(0xffffffffu, valid)) return;
   const bool act = valid && g.n_sorted > 0;  // self queries are finite by construction
@@ -461,8 +431,7 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
   int cu = 0, cv = 0;
   u64 tau = 0;
   if (act) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+    query_cell(g, qx, qy, qz, cu, cv);
     tau = make_key(P.r2, 0);
   }
   int ns = 0;
@@ -520,18 +489,9 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
     P.redo_list[slot] = (int32_t)t;
     return;
   }
-  float o[4];
   const int m = ns;
-  if (!act || m < 3) {
-    o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-  } else {
-    float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-    float kx = 0.f, ky = 0.f, kz = 0.f;
-    if (shifted) {
-      float4 f = __ldg(P.xyz4 + key_idx(store[(c[0] & 31u) * BD]));
-      kx = f.x; ky = f.y; kz = f.z;
-    }
+  CovAcc cov(P.flags);
+  if (act && m >= 3) {
 #pragma unroll
     for (int jb = 0; jb < C_SLOTS; jb += 4) {
       if (jb < m) {
@@ -540,18 +500,12 @@ __global__ void __launch_bounds__(128, 6) k_radius_normals32(SearchParams P) {
         for (int u = 0; u < 4; u++)
           if (jb + u < m) a[u] = __ldg(P.xyz4 + key_idx(store[(c[jb + u] & 31u) * BD]));
 #pragma unroll
-        for (int u = 0; u < 4; u++) {
-          if (jb + u < m) {
-            float x = a[u].x, y = a[u].y, z = a[u].z;
-            if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-            accumulate_point(acc, x, y, z);
-          }
-        }
+        for (int u = 0; u < 4; u++)
+          if (jb + u < m) cov.add(a[u]);
       }
     }
-    normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
   }
-  store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
+  cov.finish(P, act, row, qx, qy, qz);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -573,7 +527,7 @@ __device__ __forceinline__ u64 warp_min_u64(u64 v) {
 
 constexpr int WARPQ_WARPS = 4;
 
-constexpr int WQ_SEG_MAX = 128;   // cell ranges of one ring handled in the flattened way (rings up to 31)
+constexpr int WQ_SEG_MAX = 128;   // cell ranges of a ring looked up at once (the ranges of 64 rows)
 
 __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
   pdl_prologue();
@@ -591,8 +545,8 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
   float qx, qy, qz;
   int64_t row;
   load_query(P, P.q != nullptr, t, qx, qy, qz, row);
-  const int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-  const int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+  int cu, cv;
+  query_cell(g, qx, qy, qz, cu, cv);
   int cnt = 0;
   u64 tau = PPP_KEY_INF;  // warp-uniform acceptance threshold (k-th best after the last ring)
   u64 mine = PPP_KEY_INF;  // lane j ends up holding the j-th nearest key ...
@@ -602,19 +556,22 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
   int R_prev = -1;
   while (true) {
     // annulus R_prev < max(|du|,|dv|) <= R.  Its cell ranges (one per row, two for the rows that only add the
-    // two outer column strips) are looked up by all lanes at once, then the lanes stride over the CONCATENATION
-    // of the ranges with four candidates in flight each: a query costs a couple of dependent memory latencies
-    // per ring instead of two per row (this kernel is latency-bound: a few hundred queries, one warp each).
-    const int v0 = max(cv - R, 0), v1 = min(cv + R, g.nv - 1);
-    const int nseg = 2 * (v1 - v0 + 1);
-    if (nseg > 0 && nseg <= WQ_SEG_MAX) {
-      int* seg_s = s_seg[w];
-      int* seg_p = s_pre[w];
+    // two outer column strips) are looked up by all lanes at once, WQ_SEG_MAX of them at a time, then the lanes
+    // stride over the CONCATENATION of the ranges with four candidates in flight each: a query costs a couple of
+    // dependent memory latencies per ring instead of two per row (this kernel is latency-bound: a few hundred
+    // queries, one warp each).  The visiting order cannot change the result: keys are unique, and both the
+    // acceptance test and the k smallest taken after the ring are the same for any order.
+    int* seg_s = s_seg[w];
+    int* seg_p = s_pre[w];
+    const int v1 = min(cv + R, g.nv - 1);
+    for (int vb = max(cv - R, 0); vb <= v1; vb += WQ_SEG_MAX / 2) {
+      const int nseg = 2 * (min(v1 - vb + 1, WQ_SEG_MAX / 2));
+      __syncwarp();   // the previous batch has been read
       for (int sg0 = 0; sg0 < nseg; sg0 += 32) {
         const int sg = sg0 + lane;
         int s0 = 0, len = 0;
         if (sg < nseg) {
-          const int v = v0 + (sg >> 1), part = sg & 1;
+          const int v = vb + (sg >> 1), part = sg & 1;
           const bool full = abs(v - cv) > R_prev;
           int a, b;
           if (full) { a = max(cu - R, 0); b = part == 0 ? min(cu + R, g.nu - 1) : -1; }
@@ -655,25 +612,6 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
           if (key < tau && (cnt < k || key < L[(k - 1) * 32])) list_insert(L, 32, cnt, k, key);
         }
       }
-    } else {
-    for (int v = v0; v <= v1; v++) {
-      const int32_t* rowp = g.cell_start + (int64_t)v * g.nu;
-      const bool full = abs(v - cv) > R_prev;
-      for (int part = 0; part < (full ? 1 : 2); part++) {
-        int a, b;
-        if (full) { a = max(cu - R, 0); b = min(cu + R, g.nu - 1); }
-        else if (part == 0) { a = max(cu - R, 0); b = min(cu - R_prev - 1, g.nu - 1); }
-        else { a = max(cu + R_prev + 1, 0); b = min(cu + R, g.nu - 1); }
-        if (a > b) continue;
-        const int s = __ldg(rowp + a), e = __ldg(rowp + b + 1);
-        for (int i = s + lane; i < e; i += 32) {
-          float4 c = __ldg(g.sorted + i);
-          u64 key = make_key(d2_flann(qx, qy, qz, c.x, c.y, c.z), __float_as_int(c.w));
-          // a full lane list only takes keys below its own last entry (list_insert overwrites it)
-          if (key < tau && (cnt < k || key < L[(k - 1) * 32])) list_insert(L, 32, cnt, k, key);
-        }
-      }
-    }
     }
     __syncwarp();
     // k smallest of the 32 sorted lists
@@ -706,14 +644,9 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
     if (P.d2_out) P.d2_out[row * (int64_t)k + 32 + lane] = mine2 != PPP_KEY_INF ? key_d2(mine2) : CUDART_INF_F;
   }
   if (P.normals) {
-    float o[4];
-    if (have < 3) {
-      o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    } else {
-      // sequential accumulation in list order, computed redundantly by every lane
-      float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-      float kx = 0.f, ky = 0.f, kz = 0.f;
+    // sequential accumulation in list order, computed redundantly by every lane
+    CovAcc cov(P.flags);
+    if (have >= 3) {
       // every lane fetches ITS neighbour's record (one memory latency for all of them); the accumulation then walks
       // the list through shuffles -- sixteen dependent loads in a row were a third of this latency-bound kernel
       float4 rec = make_float4(0.f, 0.f, 0.f, 0.f), rec2 = rec;
@@ -725,14 +658,10 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_knn_warp(SearchParams P) {
         a.x = __shfl_sync(0xffffffffu, lo32 ? rec.x : rec2.x, j & 31);
         a.y = __shfl_sync(0xffffffffu, lo32 ? rec.y : rec2.y, j & 31);
         a.z = __shfl_sync(0xffffffffu, lo32 ? rec.z : rec2.z, j & 31);
-        if (shifted && j == 0) { kx = a.x; ky = a.y; kz = a.z; }
-        float x = a.x, y = a.y, z = a.z;
-        if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-        accumulate_point(acc, x, y, z);
+        cov.add(a);
       }
-      normal_from_accumulators(acc, have, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
     }
-    if (lane == 0) store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
+    cov.finish(P, true, row, qx, qy, qz, lane == 0);
   }
   __syncwarp();
   }  // slot loop
@@ -759,11 +688,11 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_radius_warp(SearchParams P
   const u64 tau = make_key(P.r2, 0);
   for (int64_t slot = (int64_t)blockIdx.x * WARPQ_WARPS + w; slot < n_redo; slot += (int64_t)gridDim.x * WARPQ_WARPS) {
     const int64_t t = P.redo_list[slot];
-    float4 p = __ldg(g.sorted + P.first + t);
-    const float qx = p.x, qy = p.y, qz = p.z;
-    const int64_t row = __float_as_int(p.w);
-    const int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    const int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+    float qx, qy, qz;
+    int64_t row;
+    load_query(P, false, t, qx, qy, qz, row);
+    int cu, cv;
+    query_cell(g, qx, qy, qz, cu, cv);
     const int R = P.R0;
     int cnt = 0;
     bool over = false;
@@ -787,26 +716,16 @@ __global__ void __launch_bounds__(WARPQ_WARPS * 32) k_radius_warp(SearchParams P
       if (lane == 0) redo2_list[atomicAdd(redo2_count, 1)] = (int32_t)t;
       continue;
     }
-    float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    const bool shifted = (P.flags & PPP_COV_SHIFTED) != 0;
-    float kx = 0.f, ky = 0.f, kz = 0.f;
-    int head = 0, m = 0;
+    CovAcc cov(P.flags);
+    int head = 0;
     while (true) {
       u64 h = head < cnt ? L[head * 32] : PPP_KEY_INF;
       u64 mn = warp_min_u64(h);
       if (mn == PPP_KEY_INF) break;
       if (h == mn) head++;
-      float4 a = __ldg(P.xyz4 + key_idx(mn));
-      if (shifted && m == 0) { kx = a.x; ky = a.y; kz = a.z; }
-      float x = a.x, y = a.y, z = a.z;
-      if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
-      accumulate_point(acc, x, y, z);
-      m++;
+      cov.add(__ldg(P.xyz4 + key_idx(mn)));
     }
-    float o[4];
-    if (m < 3) o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
-    else normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
-    if (lane == 0) store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
+    cov.finish(P, true, row, qx, qy, qz, lane == 0);
     __syncwarp();
   }
 }
@@ -827,8 +746,8 @@ __global__ void __launch_bounds__(128) k_radius_count(SearchParams P, int32_t* _
     load_query(P, P.q != nullptr, t, qx, qy, qz, row);
     const bool mine = P.use_redo || P.choice == nullptr || P.q != nullptr || __ldg(P.choice + row) == P.my_proj;
     if (mine && finite3(qx, qy, qz) && g.n_sorted > 0) {
-      int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-      int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+      int cu, cv;
+      query_cell(g, qx, qy, qz, cu, cv);
       const float r2 = P.r2;
       visit_annulus(g, cu, cv, -1, P.R0, [&](float4 c) {
         cnt += d2_flann(qx, qy, qz, c.x, c.y, c.z) < r2 ? 1 : 0;
@@ -933,11 +852,12 @@ __global__ void __launch_bounds__(128) k_coverage_mark(SearchParams P, unsigned 
   int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= P.nq) return;
   const GridView& g = P.g;
-  const float* qp = P.q + t * P.q_sf;
-  const float qx = __ldg(qp), qy = __ldg(qp + 1), qz = __ldg(qp + 2);
+  float qx, qy, qz;
+  int64_t row;
+  load_query(P, true, t, qx, qy, qz, row);
   if (!finite3(qx, qy, qz) || g.n_sorted == 0) return;
-  int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-  int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+  int cu, cv;
+  query_cell(g, qx, qy, qz, cu, cv);
   const float r2 = r2_per_query ? __ldg(r2_per_query + t) : P.r2;   // the block radius R0 covers the largest of them
   if (!(r2 > 0.0f)) return;                                        // NaN / zero radius: nothing is strictly inside
   visit_annulus(g, cu, cv, -1, P.R0, [&](float4 c) {
@@ -1028,6 +948,40 @@ int radius_rings(const GridView& g, double r) {
   return std::max(R, 0);
 }
 
+// The fields every search launch shares: the grid, the cloud and the queries (q == nullptr: the cloud's own points
+// from sorted position `first` on).
+static SearchParams search_params(const ppp_cloud* c, const GridStore& gs, const float* q, int64_t nq, int q_sf,
+                                  int64_t first) {
+  SearchParams P{};
+  P.g = gs.v; P.xyz4 = c->xyz4; P.q = q; P.q_sf = q_sf; P.nq = nq; P.first = first;
+  return P;
+}
+
+// The normal outputs: records of stride nsf (nullptr: none) through the cloud's row map and route, flipped towards
+// vp, and the projection whose self-queries this launch answers (choice == nullptr: all of them).
+static void set_normal_outputs(SearchParams& P, const ppp_cloud* c, float* normals, int nsf, const float vp[3],
+                               unsigned flags, const unsigned char* choice, int my_proj) {
+  P.normals = normals; P.nsf = nsf; P.nmap = c->nmap; P.route = c->route;
+  P.vpx = vp ? vp[0] : 0; P.vpy = vp ? vp[1] : 0; P.vpz = vp ? vp[2] : 0; P.flags = flags;
+  P.choice = P.q ? nullptr : choice; P.my_proj = my_proj;
+}
+
+// Self-queries cover the indexed points only: the rows of the non-finite points get their defaults (idx -1, d2 inf,
+// NaN normals) from the launch that starts at the first sorted position.
+static int launch_default_rows(ppp_cloud* c, const SearchParams& P) {
+  if (P.q || P.first != 0 || c->n_finite == c->n) return PPP_OK;
+  unsigned blocks = (unsigned)((c->n + 255) / 256);
+  PPP_LAUNCH(c->ctx, "default_rows", k_default_rows, blocks, 256, 0, (const float4*)c->xyz4, c->n, P.cap, P.idx_out,
+             P.d2_out, P.normals, P.nsf, P.nmap, P.route);
+  PPP_CHECK_LAUNCH();
+  return PPP_OK;
+}
+
+// Grid of the persistent one-warp-per-query hand-over kernels (the number of queries is only known on the device).
+static unsigned handover_blocks(const ppp_ctx* ctx, int64_t nq) {
+  return (unsigned)std::min<int64_t>((nq + WARPQ_WARPS - 1) / WARPQ_WARPS, (int64_t)ctx->sm_count * 8);
+}
+
 static int launch_search(ppp_cloud* c, SearchParams& P) {
   ppp_ctx* ctx = c->ctx;
   int block; size_t smem;
@@ -1036,8 +990,7 @@ static int launch_search(ppp_cloud* c, SearchParams& P) {
     block = 32;
     smem = (size_t)std::max(P.cap, 1) * 8 * block;
   }
-  if (smem > 40 * 1024)
-    PPP_CUDA(cudaFuncSetAttribute(k_search, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PPP_TRY(smem_optin(k_search, smem));
   if (P.nq > 0) {
     unsigned blocks = (unsigned)((P.nq + block - 1) / block);
     PPP_LAUNCH(ctx, P.use_redo ? "knn_redo" : P.mode == 0 ? (P.normals ? "knn_normals" : "knn") : (P.normals ? "radius_normals" : "radius_fill"),
@@ -1045,6 +998,30 @@ static int launch_search(ppp_cloud* c, SearchParams& P) {
     PPP_CHECK_LAUNCH();
   }
   return PPP_OK;
+}
+
+// Radius neighbours of P's queries (counts[row], optional) and the largest count, fetched to the host.
+static int radius_count_max(ppp_cloud* c, const SearchParams& P, int32_t* counts, int* max_out) {
+  ppp_ctx* ctx = c->ctx;
+  int32_t* mx = nullptr;
+  PPP_TRY(dev_alloc(ctx, &mx, 1));
+  PPP_CUDA(cudaMemsetAsync(mx, 0, 4, ctx->stream));
+  if (P.nq > 0) {
+    unsigned blocks = (unsigned)((P.nq + 127) / 128);
+    PPP_LAUNCH(ctx, "radius_count", k_radius_count, blocks, 128, 0, P, counts, mx);
+    PPP_CHECK_LAUNCH();
+  }
+  PPP_TRY(fetch_small(ctx, mx, 4, max_out));
+  dev_free(ctx, mx);
+  return PPP_OK;
+}
+
+// Radius lists of unknown length: k_search with lists as long as the largest neighbour count.
+static int launch_search_at_max_count(ppp_cloud* c, SearchParams P) {
+  int mx = 0;
+  PPP_TRY(radius_count_max(c, P, nullptr, &mx));
+  P.cap = std::max(mx, 1);
+  return launch_search(c, P);
 }
 
 static int prepare_fast(ppp_cloud* c, SearchParams& P, int32_t** redo_out) {
@@ -1079,7 +1056,7 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
   // per thread: `slots` key words, then the first sorted position of each of the 2 R0 + 1 block rows
   auto launch = [&](auto kern, int slots) -> int {
     const size_t smem = (size_t)(slots + 2 * P.R0 + 1) * 4 * block;
-    if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    PPP_TRY(smem_optin(kern, smem));
     PPP_LAUNCH(ctx, P.normals ? "knn_normals" : "knn", kern, blocks, block, smem, P);
     PPP_CHECK_LAUNCH();
     return PPP_OK;
@@ -1088,14 +1065,11 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
   else if (P.cap <= 32) PPP_TRY(launch(ext ? k_knnf<32, 16, 6, 128, 6, 32, true> : k_knnf<32, 16, 6, 128, 6, 32, false>, 32 + 16));
   else PPP_TRY(launch(ext ? k_knnf<64, 32, 7, 128, 4, 64, true> : k_knnf<64, 32, 7, 128, 4, 64, false>, 64 + 32));
   {
-    // hand-over queries: one warp each, persistent warps (their number is only known on the device)
+    // hand-over queries: one warp each
     P.use_redo = 1;
-    size_t smem = (size_t)WARPQ_WARPS * 32 * P.cap * 8;
-    // (opt in from 40 KB of dynamic shared memory on: the kernels carry static arrays too -- k = 48 asks for exactly
-    // 48 KB here and was refused by the launch without it)
-    if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(k_knn_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    unsigned blocks = (unsigned)std::min<int64_t>((P.nq + WARPQ_WARPS - 1) / WARPQ_WARPS, (int64_t)ctx->sm_count * 8);
-    PPP_LAUNCH(ctx, "knn_redo", k_knn_warp, blocks, WARPQ_WARPS * 32, smem, P);
+    const size_t smem = (size_t)WARPQ_WARPS * 32 * P.cap * 8;
+    PPP_TRY(smem_optin(k_knn_warp, smem));
+    PPP_LAUNCH(ctx, "knn_redo", k_knn_warp, handover_blocks(ctx, P.nq), WARPQ_WARPS * 32, smem, P);
     PPP_CHECK_LAUNCH();
   }
   if (getenv("PPP_DEBUG")) {
@@ -1111,143 +1085,89 @@ static int launch_knn_fast(ppp_cloud* c, SearchParams& P) {
 int knn_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f, int64_t first, int k,
                int32_t* idx_dev, float* d2_dev, bool with_normals, const float vp[3], unsigned flags,
                float* normals_dev, int normal_stride_f, const unsigned char* choice, int my_proj) {
-  ppp_ctx* ctx = c->ctx;
-  SearchParams P{};
-  P.g = gs.v; P.xyz4 = c->xyz4; P.q = q_dev; P.q_sf = q_stride_f; P.nq = nq; P.first = first;
-  P.cap = k; P.kk = (int)std::min<int64_t>(k, c->n_finite); P.mode = 0; P.R0 = PPP_KNN_RINGS; P.r2 = 0;
-  P.idx_out = idx_dev; P.d2_out = d2_dev; P.offsets = nullptr;
-  P.normals = with_normals ? normals_dev : nullptr; P.nsf = normal_stride_f; P.nmap = c->nmap; P.route = c->route;
-  P.vpx = vp ? vp[0] : 0; P.vpy = vp ? vp[1] : 0; P.vpz = vp ? vp[2] : 0; P.flags = flags;
-  P.choice = q_dev ? nullptr : choice; P.my_proj = my_proj;
-  if (!q_dev && c->n_finite < c->n && first == 0) {
-    unsigned blocks = (unsigned)((c->n + 255) / 256);
-    PPP_LAUNCH(ctx, "default_rows", k_default_rows, blocks, 256, 0, (const float4*)c->xyz4, c->n, k, idx_dev, d2_dev,
-               P.normals, normal_stride_f, c->nmap, c->route);
-    PPP_CHECK_LAUNCH();
-  }
+  SearchParams P = search_params(c, gs, q_dev, nq, q_stride_f, first);
+  set_normal_outputs(P, c, with_normals ? normals_dev : nullptr, normal_stride_f, vp, flags, choice, my_proj);
+  P.mode = 0; P.R0 = PPP_KNN_RINGS;
+  P.cap = k; P.kk = (int)std::min<int64_t>(k, c->n_finite);
+  P.idx_out = idx_dev; P.d2_out = d2_dev;
+  PPP_TRY(launch_default_rows(c, P));
   if (k <= 64 && nq > 0) return launch_knn_fast(c, P);
   return launch_search(c, P);
 }
 
 int radius_count_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f,
                         int64_t first, float r2, int32_t* counts_dev) {
-  ppp_ctx* ctx = c->ctx;
-  SearchParams P{};
-  P.g = gs.v; P.xyz4 = c->xyz4; P.q = q_dev; P.q_sf = q_stride_f; P.nq = nq; P.first = first;
+  SearchParams P = search_params(c, gs, q_dev, nq, q_stride_f, first);
   P.mode = 1; P.r2 = r2; P.R0 = radius_rings(gs.v, std::sqrt((double)r2));
-  int32_t* mx = nullptr;
-  PPP_TRY(dev_alloc(ctx, &mx, 1));
-  PPP_CUDA(cudaMemsetAsync(mx, 0, 4, ctx->stream));
   if (!q_dev && c->n_finite < c->n && counts_dev) {
     unsigned blocks = (unsigned)((c->n + 255) / 256);
-    PPP_LAUNCH(ctx, "fill_i32", k_fill_i32, blocks, 256, 0, counts_dev, c->n, 0);
+    PPP_LAUNCH(c->ctx, "fill_i32", k_fill_i32, blocks, 256, 0, counts_dev, c->n, 0);
     PPP_CHECK_LAUNCH();
   }
-  if (nq > 0) {
-    unsigned blocks = (unsigned)((nq + 127) / 128);
-    PPP_LAUNCH(ctx, "radius_count", k_radius_count, blocks, 128, 0, P, counts_dev, mx);
-    PPP_CHECK_LAUNCH();
-  }
-  int hmx = 0;
-  PPP_TRY(fetch_small(ctx, mx, 4, &hmx));
-  dev_free(ctx, mx);
-  return hmx;  // >= 0: maximum neighbour count (used to size the fill pass)
+  int mx = 0;
+  PPP_TRY(radius_count_max(c, P, counts_dev, &mx));
+  return mx;  // >= 0: maximum neighbour count (used to size the fill pass)
 }
 
 int radius_fill_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f,
                        int64_t first, float r2, const int64_t* offsets_dev, int32_t* idx_dev, float* d2_dev) {
-  // the caller has run radius_count_launch and passes the maximum count through d2-independent path:
-  // recompute it here (cheap) so this entry stays self-contained.
-  int mx = radius_count_launch(c, gs, q_dev, nq, q_stride_f, first, r2, nullptr);
-  if (mx < 0) return mx;
-  SearchParams P{};
-  P.g = gs.v; P.xyz4 = c->xyz4; P.q = q_dev; P.q_sf = q_stride_f; P.nq = nq; P.first = first;
-  P.cap = std::max(mx, 1); P.mode = 1; P.r2 = r2; P.R0 = radius_rings(gs.v, std::sqrt((double)r2));
+  SearchParams P = search_params(c, gs, q_dev, nq, q_stride_f, first);
+  P.mode = 1; P.r2 = r2; P.R0 = radius_rings(gs.v, std::sqrt((double)r2));
   P.idx_out = idx_dev; P.d2_out = d2_dev; P.offsets = offsets_dev;
-  return launch_search(c, P);
+  return launch_search_at_max_count(c, P);
 }
 
 int normals_radius_launch(ppp_cloud* c, const GridStore& gs, int64_t first, int64_t count, float r2,
                           const float vp[3], unsigned flags, float* normals_dev, int normal_stride_f,
                           const unsigned char* choice, int my_proj) {
   ppp_ctx* ctx = c->ctx;
-  SearchParams P{};
-  P.g = gs.v; P.xyz4 = c->xyz4; P.q = nullptr; P.nq = count; P.first = first;
+  SearchParams P = search_params(c, gs, nullptr, count, 0, first);
+  set_normal_outputs(P, c, normals_dev, normal_stride_f, vp, flags, choice, my_proj);
   P.mode = 1; P.r2 = r2; P.R0 = radius_rings(gs.v, std::sqrt((double)r2));
-  P.normals = normals_dev; P.nsf = normal_stride_f; P.nmap = c->nmap; P.route = c->route;
-  P.vpx = vp ? vp[0] : 0; P.vpy = vp ? vp[1] : 0; P.vpz = vp ? vp[2] : 0; P.flags = flags;
-  P.choice = choice; P.my_proj = my_proj;
-  if (c->n_finite < c->n && first == 0) {
-    unsigned blocks = (unsigned)((c->n + 255) / 256);
-    PPP_LAUNCH(ctx, "default_rows", k_default_rows, blocks, 256, 0, (const float4*)c->xyz4, c->n, 0, (int32_t*)nullptr,
-               (float*)nullptr, normals_dev, normal_stride_f, c->nmap, c->route);
-    PPP_CHECK_LAUNCH();
-  }
+  PPP_TRY(launch_default_rows(c, P));
   if (count <= 0) return PPP_OK;
   // expected neighbours per query from the surface density; the fixed-capacity fast kernel pays
   // off while most queries stay within its 32-entry lists
   const double expect = c->density * 3.14159265358979 * (double)r2;
-  const bool fast = expect <= 24.0;
+  if (expect > 24.0) return launch_search_at_max_count(c, P);
   int32_t* redo = nullptr;
+  PPP_TRY(prepare_fast(c, P, &redo));
+  P.cap = 32;
+  {
+    const size_t smem = (size_t)C_STORE * 8 * 128;
+    PPP_TRY(smem_optin(k_radius_normals32, smem));
+    unsigned blocks = (unsigned)((P.nq + 127) / 128);
+    PPP_LAUNCH(ctx, "radius_normals", k_radius_normals32, blocks, 128, smem, P);
+    PPP_CHECK_LAUNCH();
+  }
+  // hand-over queries: one warp each; what even that cannot hold goes on to the generic kernel through a second list
+  int32_t* redo2 = nullptr;
+  PPP_TRY(dev_alloc(ctx, &redo2, (size_t)P.nq + 1));
+  PPP_CUDA(cudaMemsetAsync(redo2, 0, sizeof(int32_t), ctx->stream));
+  PPP_LAUNCH(ctx, "radius_redo", k_radius_warp, handover_blocks(ctx, P.nq), WARPQ_WARPS * 32, 0, P, redo2, redo2 + 1);
+  PPP_CHECK_LAUNCH();
   int n_redo = 0;
-  if (fast) {
-    PPP_TRY(prepare_fast(c, P, &redo));
-    P.cap = 32;
-    {
-      size_t smem = (size_t)C_STORE * 8 * 128;
-      PPP_CUDA(cudaFuncSetAttribute(k_radius_normals32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      unsigned blocks = (unsigned)((P.nq + 127) / 128);
-      PPP_LAUNCH(ctx, "radius_normals", k_radius_normals32, blocks, 128, smem, P);
-      PPP_CHECK_LAUNCH();
-    }
-    // hand-over queries: one warp each (persistent warps); what even that cannot hold goes on to the
-    // generic kernel through a second list
-    int32_t* redo2 = nullptr;
-    PPP_TRY(dev_alloc(ctx, &redo2, (size_t)P.nq + 1));
-    PPP_CUDA(cudaMemsetAsync(redo2, 0, sizeof(int32_t), ctx->stream));
-    {
-      unsigned blocks = (unsigned)std::min<int64_t>((P.nq + WARPQ_WARPS - 1) / WARPQ_WARPS, (int64_t)ctx->sm_count * 8);
-      PPP_LAUNCH(ctx, "radius_redo", k_radius_warp, blocks, WARPQ_WARPS * 32, 0, P, redo2, redo2 + 1);
-      PPP_CHECK_LAUNCH();
-    }
-    PPP_TRY(fetch_small(ctx, redo2, 4, &n_redo));
-    dev_free(ctx, redo);
-    redo = redo2;
-    if (n_redo == 0) { dev_free(ctx, redo); return PPP_OK; }
+  PPP_TRY(fetch_small(ctx, redo2, 4, &n_redo));
+  dev_free(ctx, redo);
+  int st = PPP_OK;
+  if (n_redo > 0) {
+    P.nq = n_redo;
     P.redo_count = redo2;
     P.redo_list = redo2 + 1;
     P.use_redo = 1;
+    st = launch_search_at_max_count(c, P);
   }
-  // generic path: all queries, or only the ones the fast kernel handed over
-  const int64_t nq = fast ? n_redo : count;
-  SearchParams C = P;
-  C.nq = nq;
-  int32_t* mx = nullptr;
-  PPP_TRY(dev_alloc(ctx, &mx, 1));
-  PPP_CUDA(cudaMemsetAsync(mx, 0, 4, ctx->stream));
-  {
-    unsigned blocks = (unsigned)((nq + 127) / 128);
-    PPP_LAUNCH(ctx, "radius_count", k_radius_count, blocks, 128, 0, C, (int32_t*)nullptr, mx);
-    PPP_CHECK_LAUNCH();
-  }
-  int hmx = 0;
-  PPP_TRY(fetch_small(ctx, mx, 4, &hmx));
-  dev_free(ctx, mx);
-  C.cap = std::max(hmx, 1);
-  int st = launch_search(c, C);
-  dev_free(ctx, redo);
+  dev_free(ctx, redo2);
   return st;
 }
 
 int coverage_mark_launch(ppp_cloud* c, const GridStore& gs, const float* q_dev, int64_t nq, int q_stride_f, float r2,
                          unsigned char* flags_dev, const float* r2_per_query_dev) {
-  ppp_ctx* ctx = c->ctx;
   if (nq <= 0) return PPP_OK;
-  SearchParams P{};
-  P.g = gs.v; P.xyz4 = c->xyz4; P.q = q_dev; P.q_sf = q_stride_f; P.nq = nq;
+  SearchParams P = search_params(c, gs, q_dev, nq, q_stride_f, 0);
   P.mode = 1; P.r2 = r2; P.R0 = radius_rings(gs.v, std::sqrt((double)r2));
   unsigned blocks = (unsigned)((nq + 127) / 128);
-  PPP_LAUNCH(ctx, "coverage_mark", k_coverage_mark, blocks, 128, 0, P, flags_dev, r2_per_query_dev);
+  PPP_LAUNCH(c->ctx, "coverage_mark", k_coverage_mark, blocks, 128, 0, P, flags_dev, r2_per_query_dev);
   PPP_CHECK_LAUNCH();
   return PPP_OK;
 }

@@ -182,8 +182,7 @@ __global__ void __launch_bounds__(128) k_mls(MlsParams P, MlsRecords Q) {
   if ((P.choice || (RECORDS && Q.nmap)) && !__any_sync(0xffffffffu, valid)) return;
   int cu = 0, cv = 0;
   if (valid) {
-    cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-    cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+    query_cell(g, qx, qy, qz, cu, cv);
   }
   const double qd[3] = {(double)qx, (double)qy, (double)qz};
 

@@ -72,6 +72,12 @@ __device__ __forceinline__ int cell_coord_raw(float a, float amin, float inv_h) 
 
 __device__ __forceinline__ float axis_of(float x, float y, float z, int a) { return a == 0 ? x : (a == 1 ? y : z); }
 
+// The (clamped, possibly outside the grid) cell of a query.
+__device__ __forceinline__ void query_cell(const GridView& g, float qx, float qy, float qz, int& cu, int& cv) {
+  cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
+  cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+}
+
 // Squared lower bound on the distance from a query in cell (cu,cv) to any point whose cell lies
 // outside the (2R+1)x(2R+1) block around it: (R*h - slack)^2, rounded down, shrunk by 1e-6 so a
 // float32 d2 (relative error <= 3*2^-24) of an unseen point can never tie or beat an accepted one.
@@ -261,6 +267,33 @@ __device__ __forceinline__ void store_normal(float* base, const int32_t* __restr
     p[0] = o[0]; p[1] = o[1]; p[2] = o[2]; p[3] = o[3];
   }
 }
+
+// The PCL normal of one query from its neighbour records, added in list order: pcl::NormalEstimation's contract.
+// Under PPP_COV_SHIFTED the first record is the origin every record is taken relative to.
+struct CovAcc {
+  float acc[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float kx = 0.f, ky = 0.f, kz = 0.f;
+  int m = 0;
+  bool shifted;
+  __device__ __forceinline__ explicit CovAcc(unsigned flags) : shifted((flags & PPP_COV_SHIFTED) != 0) {}
+  __device__ __forceinline__ void add(float4 rec) {
+    float x = rec.x, y = rec.y, z = rec.z;
+    if (m == 0) { kx = x; ky = y; kz = z; }
+    if (shifted) { x = __fsub_rn(x, kx); y = __fsub_rn(y, ky); z = __fsub_rn(z, kz); }
+    accumulate_point(acc, x, y, z);
+    m++;
+  }
+  // NaN for a non-finite query or fewer than 3 neighbours; the record of `row` is stored if `store` (the lanes of a
+  // warp that all computed it leave the store to one of them).  P: the search parameters.
+  template <class Params>
+  __device__ __forceinline__ void finish(const Params& P, bool fin, int64_t row, float qx, float qy, float qz,
+                                         bool store = true) {
+    float o[4];
+    if (!fin || m < 3) o[0] = o[1] = o[2] = o[3] = CUDART_NAN_F;
+    else normal_from_accumulators(acc, m, qx, qy, qz, P.vpx, P.vpy, P.vpz, o);
+    if (store) store_normal(P.normals, P.nmap, row, P.nsf, o, P.route);
+  }
+};
 
 // MLS result record (ppp_dev_mls_smooth) of a point without an output row: flag 0, every other field NaN.
 __device__ __forceinline__ void mls_no_row(float o[8]) {

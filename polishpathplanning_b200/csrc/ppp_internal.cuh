@@ -264,6 +264,16 @@ bool ppp_pdl_enabled();
 
 #define PPP_CHECK_LAUNCH() PPP_CUDA(cudaGetLastError())
 
+// Lets `kern` launch with `bytes` of dynamic shared memory.  Past 48 KB a kernel has to opt in, and the limit applies
+// to its static arrays plus the dynamic memory: the opt-in starts at 40 KB of dynamic memory because the kernels
+// carry up to 8 KB of static arrays (k = 48 asked the kNN hand-over kernel for exactly 48 KB and the launch was
+// refused without it).
+template <class K>
+int smem_optin(K kern, size_t bytes) {
+  if (bytes > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  return PPP_OK;
+}
+
 
 // A few bytes of device memory to the host in stream order, then synchronise: a tiny kernel stores
 // them into mapped pinned memory.  Unlike a cudaMemcpyAsync this does not queue behind a large

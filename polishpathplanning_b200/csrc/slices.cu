@@ -331,8 +331,8 @@ __device__ int2 nn_side(const GridView& g, const float4* __restrict__ xyz4, floa
     }
     if (key < best) { best = key; best_pos = pos; }
   };
-  int cu = cell_coord_raw(axis_of(qx, qy, qz, g.au), g.min_u, g.inv_h);
-  int cv = cell_coord_raw(axis_of(qx, qy, qz, g.av), g.min_v, g.inv_h);
+  int cu, cv;
+  query_cell(g, qx, qy, qz, cu, cv);
   // when x is the fast grid axis only the cell columns that overlap the wanted x-interval can
   // hold members (cell coordinates are monotone in x)
   int ulo = -2147483647, uhi = 2147483647;
@@ -1091,8 +1091,9 @@ static int bands_prepare(ppp_cloud* c, const float* plane_x_host, int S, float h
 static int bands_fill(ppp_cloud* c, const BandPrep& bp, int32_t* idx) {
   ppp_ctx* ctx = c->ctx;
   if (bp.n_src <= 0 || bp.Sv <= 0) return PPP_OK;
-  if (bp.use_smem) PPP_CUDA(cudaFuncSetAttribute(k_band_fill, cudaFuncAttributeMaxDynamicSharedMemorySize, BAND_SMEM_BINS * 4));
-  PPP_LAUNCH(ctx, "band_fill", k_band_fill, bp.blocks, 256, bp.use_smem ? (size_t)bp.Sv * 8 : 0, bp.b, bp.src, bp.n_src,
+  const size_t smem = bp.use_smem ? (size_t)bp.Sv * 8 : 0;
+  PPP_TRY(smem_optin(k_band_fill, smem));
+  PPP_LAUNCH(ctx, "band_fill", k_band_fill, bp.blocks, 256, smem, bp.b, bp.src, bp.n_src,
              bp.chunk, bp.use_smem, bp.w_is_flag, bp.counts, (const int64_t*)bp.offsets, idx);
   PPP_CHECK_LAUNCH();
   return PPP_OK;
@@ -1119,8 +1120,7 @@ int bands_launch(ppp_cloud* c, const float* plane_x_host, int S, float half_widt
       int64_t maxB = 0;
       for (int s = 0; s < S; s++) maxB = std::max(maxB, off_h[s + 1] - off_h[s]);
       int smem_cap = (int)std::min<int64_t>(std::max<int64_t>(maxB, 1), 49152);  // <= 192 KB of int32
-      if (smem_cap * 4 > 40 * 1024)
-        PPP_CUDA(cudaFuncSetAttribute(k_band_sort, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap * 4));
+      PPP_TRY(smem_optin(k_band_sort, (size_t)smem_cap * 4));
       PPP_LAUNCH(ctx, "band_sort", k_band_sort, (unsigned)S, 1024, (size_t)smem_cap * 4, (const int64_t*)offsets, idx,
                  smem_cap);
       PPP_CHECK_LAUNCH();
@@ -1165,8 +1165,7 @@ static int launch_slice_order(ppp_ctx* ctx, int S, int64_t band_est, bool expect
   const int64_t cap1 = C == 1 ? (int64_t)smem_cap : (int64_t)chunk_cap * C;
   const bool big = expect_big || band_est > cap1;   // a second launch takes the bands beyond cap1
   if (C == 1) {
-    if ((size_t)smem_cap * 8 > 40 * 1024)
-      PPP_CUDA(cudaFuncSetAttribute(k_slice_order, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_cap * 8));
+    PPP_TRY(smem_optin(k_slice_order, (size_t)smem_cap * 8));
     // short bands: 256 threads sort them with a quarter of the barrier traffic, and more slices share an SM
     const int so_threads = smem_cap <= 4608 ? 256 : SO_THREADS;
     PPP_LAUNCH(ctx, "slice_order", k_slice_order, (unsigned)S, so_threads, (size_t)smem_cap * 8, band_off, band_idx, sorted_if_pos,
@@ -1178,15 +1177,15 @@ static int launch_slice_order(ppp_ctx* ctx, int S, int64_t band_est, bool expect
     const unsigned grid = (unsigned)S * (unsigned)C;
     if (C == 2) {
       auto kern = k_slice_order_cl<2>;
-      if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      PPP_TRY(smem_optin(kern, smem));
       PPP_LAUNCH(ctx, "slice_order", kern, grid, SO_THREADS, smem, band_off, band_idx, sorted_if_pos, keys, ys, zs, scratch, chunk_cap, S, -1, max_B, ty, tz, n_nodes);
     } else if (C == 4) {
       auto kern = k_slice_order_cl<4>;
-      if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      PPP_TRY(smem_optin(kern, smem));
       PPP_LAUNCH(ctx, "slice_order", kern, grid, SO_THREADS, smem, band_off, band_idx, sorted_if_pos, keys, ys, zs, scratch, chunk_cap, S, -1, max_B, ty, tz, n_nodes);
     } else {
       auto kern = k_slice_order_cl<8>;
-      if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      PPP_TRY(smem_optin(kern, smem));
       PPP_LAUNCH(ctx, "slice_order", kern, grid, SO_THREADS, smem, band_off, band_idx, sorted_if_pos, keys, ys, zs, scratch, chunk_cap, S, -1, max_B, ty, tz, n_nodes);
     }
     PPP_CHECK_LAUNCH();
@@ -1195,7 +1194,7 @@ static int launch_slice_order(ppp_ctx* ctx, int S, int64_t band_est, bool expect
   // the bands beyond cap1
   auto kern = k_slice_order_cl<8>;
   const size_t smem = (size_t)SOC_CHUNK_MAX * 8;
-  PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PPP_TRY(smem_optin(kern, smem));
   const unsigned clusters = (unsigned)std::min(S, 16);
   PPP_LAUNCH(ctx, "slice_order_big", kern, clusters * 8u, SO_THREADS, smem, band_off, band_idx, sorted_if_pos, keys, ys, zs, scratch,
              SOC_CHUNK_MAX, S, (int)cap1, 2147483647, ty, tz, n_nodes);
@@ -1296,7 +1295,7 @@ int contours_launch(ppp_cloud* c, const GridStore& gs, const float* planes_dev, 
       int smem_cap = (int)std::min<int64_t>(std::max<int64_t>(maxB, 2), 22000);  // 9 bytes per member, <= 198 KB
       size_t smem = 9 * (size_t)((smem_cap + 1) & ~1) + 16;
       auto kern = member_bits ? k_contour<true> : k_contour<false>;
-      if (smem > 40 * 1024) PPP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      PPP_TRY(smem_optin(kern, smem));
       PPP_LAUNCH(ctx, "contour_gen2", kern, (unsigned)S, 1024, smem, P, smem_cap);
       PPP_CHECK_LAUNCH();
     }
