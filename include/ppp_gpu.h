@@ -236,6 +236,30 @@ int ppp_dev_mls_compact(ppp_ctx* ctx, const void* rows_dev, int64_t n, const voi
  * rounding of the exchange's cut positions (derivation in csrc/mls.cu).  NaN for a radius ppp_mls_smooth refuses. */
 double ppp_mls_halo(double radius, double x_abs_max);
 
+/* voxel_down(): pcl::VoxelGrid<PointXYZRGB> (src/Path_Generation.cpp:53-59) with leaf sizes leaf[0..2] and PCL's
+ * defaults otherwise (min_points_per_voxel 0, downsample_all_data).  Voxel coordinates are computed as PCL 1.10 does,
+ * in float32 from the bounding box of the finite points (ppp_cloud_bbox); non-finite points belong to no voxel.  One
+ * row per occupied voxel, in ascending voxel key order: the centroid of its members.  The caller provides room for n
+ * rows:
+ *   points_out: records of out_stride_bytes (>= 12, multiple of 4) of which only x, y, z (the float32 sum of the
+ *               members in ascending source order, divided by (float)count) and, when the stride is >= 16, the pad
+ *               float 1.0f at byte 12 are written;
+ *   row_offsets (nullable, rows + 1 entries) and members (nullable, one entry per finite point): the members of row r
+ *               are members[row_offsets[r] .. row_offsets[r + 1]), ascending source indices (for averaging other
+ *               fields, e.g. rgba, on the host);
+ *   *n_out: rows written.
+ * A cloud without a finite point has 0 rows (PCL leaves that case undefined).
+ * PPP_ERR_INVALID for a leaf size that is <= 0 or not finite, or whose float inverse is not finite.
+ * PPP_ERR_UNSUPPORTED, with PCL's message "Leaf size is too small for the input dataset. Integer indices would
+ * overflow.", where PCL warns and returns the input unchanged: dx * dy * dz > INT32_MAX, dx = (int64)((max.x -
+ * min.x) * inv.x) + 1 in float32 (an extent whose product with the inverse leaf is not finite included).  Also
+ * PPP_ERR_UNSUPPORTED where floorf(bbox * inv) leaves the int range (PCL's voxel coordinates are undefined there).
+ * Contract: the rows, row offsets and members are those of PCL.  PCL sums each voxel in the order its unstable
+ * std::sort leaves the members, so a centroid coordinate of a voxel with n members of magnitude <= M can differ from
+ * PCL's by at most (2n + 1) * 2^-24 * M; in practice most rows are bit-identical (DESIGN.md §2).          */
+int ppp_voxel_grid(ppp_cloud* cloud, const float leaf[3], void* points_out, size_t out_stride_bytes,
+                   int64_t* row_offsets, int32_t* members, int64_t* n_out);
+
 /* estimate_normal() followed by the plane sweep, as one call: what SectPath-derived GenPath does
  * (src/Path_Alg/path_dynamic_alg.cpp:343-366: estimate_normal(); kdtree.setInputCloud; sweep).
  * Exactly the results of ppp_normals_knn (k >= 1, radius = 0) or ppp_normals_radius (k = 0,

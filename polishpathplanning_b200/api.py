@@ -18,6 +18,18 @@ def _ptr(a):
     return a.ctypes.data_as(_vp) if a is not None else None
 
 
+def _centroid_rgba(words, off, mem):
+    """PCL's AccumulatorRGBA over the rows of a voxel grid: per channel byte, the float32 sum over the row's members in
+    member order, divided by the count and truncated.  words: the source rgba words (n,) float32 bits."""
+    b = words.view(np.uint8).reshape(-1, 4)[mem].astype(np.int64)
+    cnt = np.diff(off)
+    sums = np.add.reduceat(b, off[:-1], axis=0).astype(np.float32)   # exact: integer sums below 2^24
+    for r in np.nonzero(cnt * 255 >= (1 << 24))[0]:   # past 2^24 the float partial sums round: add in member order
+        sums[r] = np.cumsum(b[off[r]:off[r + 1]].astype(np.float32), axis=0, dtype=np.float32)[-1]
+    avg = (sums / cnt.astype(np.float32)[:, None]).astype(np.uint32).astype(np.uint8)
+    return np.ascontiguousarray(avg).view(np.uint32).reshape(-1)
+
+
 class Context:
     def __init__(self, device=0):
         self.lib = _lib.load()
@@ -397,6 +409,34 @@ class Cloud:
         out = recs[src].copy()
         out[:, 0:3] = pts[:m, 0:3]
         return out, src, (nrm[:m].copy() if normals else None)
+
+    def voxel_grid(self, leaf):
+        """voxel_down(): pcl::VoxelGrid with leaf size `leaf` (one float or three).  Returns (records, row_offsets,
+        members): records (m, stride) float32 shaped like the source -- x, y, z the voxel centroids from the device,
+        the pad float 1.0, with a stride of 5 floats or more the rgba bytes averaged per channel as PCL's CentroidPoint
+        does, zeros elsewhere --, row_offsets (m + 1,) int64 and members (n_finite,) int32: the source indices of row r
+        are members[row_offsets[r]:row_offsets[r + 1]], ascending.  Raises PPPError with PPP_ERR_UNSUPPORTED where
+        PCL warns that the leaf is too small and keeps the input."""
+        lf = np.broadcast_to(np.asarray(leaf, np.float32), (3,)).copy()
+        recs = self._records
+        if recs is not None and not isinstance(recs, np.ndarray):   # device-attached cloud: fetch the records once
+            ptr, stride = recs
+            recs = self.ctx.download(ptr, (self.n, stride // 4), np.float32)
+        sf = recs.shape[1] if recs is not None else 4
+        pts = np.empty((max(self.n, 1), sf), np.float32)
+        off = np.empty(self.n + 1, np.int64)
+        mem = np.empty(max(self.n, 1), np.int32)
+        m = C.c_int64(0)
+        check(self.lib.ppp_voxel_grid(self._h, lf.ctypes.data_as(_lib._f32p), _ptr(pts), sf * 4, _ptr(off), _ptr(mem),
+                                      C.byref(m)))
+        m = m.value
+        off = off[:m + 1].copy()
+        mem = mem[:int(off[-1])].copy()
+        out = np.zeros((m, sf), np.float32)
+        out[:, :min(sf, 4)] = pts[:m, :min(sf, 4)]
+        if sf >= 5 and m:
+            out[:, 4] = _centroid_rgba(np.ascontiguousarray(recs[:, 4]), off, mem).view(np.float32)
+        return out, off, mem
 
     # ---- device-resident pipeline ---------------------------------------------------------------
     def dev_index(self, k_hint=16, radius_hint=0.0):

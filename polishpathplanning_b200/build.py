@@ -16,7 +16,7 @@ OUT = os.path.join(HERE, "libppp_gpu.so")
 OUT_CHECK = os.path.join(HERE, "libppp_gpu_check.so")   # -DPPP_CHECK_BOUNDS: device-side index assertions (tests/test_gpu_bounds.py)
 OBJ_DIR = os.path.join(HERE, "csrc", "_obj")
 OBJ_DIR_CHECK = os.path.join(HERE, "csrc", "_obj", "check")
-SOURCES = ["api.cu", "scan.cu", "grid.cu", "knn.cu", "slices.cu", "exchange.cu", "mls.cu"]
+SOURCES = ["api.cu", "scan.cu", "grid.cu", "knn.cu", "slices.cu", "exchange.cu", "mls.cu", "voxel.cu"]
 HEADERS = ["ppp_internal.cuh", "ppp_device.cuh", "sortnet.cuh", os.path.join("..", "..", "include", "ppp_gpu.h")]
 
 NVCC_FLAGS = [

@@ -974,6 +974,45 @@ int ppp_mls_smooth(ppp_cloud* c, double radius, int order, void* points_out, siz
 
 double ppp_mls_halo(double radius, double x_abs_max) { return mls_halo(radius, x_abs_max); }
 
+// voxel_down(): pcl::VoxelGrid with leaf sizes leaf[0..2] (src/Path_Generation.cpp:53-59); contract in the header.
+int ppp_voxel_grid(ppp_cloud* c, const float leaf[3], void* points_out, size_t out_stride_bytes, int64_t* row_offsets,
+                   int32_t* members, int64_t* n_out) {
+  REQUIRE(c && leaf && n_out && (points_out || c->n == 0), "NULL argument");
+  for (int d = 0; d < 3; d++)
+    REQUIRE(leaf[d] > 0 && std::isfinite(leaf[d]) && std::isfinite(1.0f / leaf[d]),
+            "leaf sizes must be > 0 and finite, with a finite float inverse");
+  REQUIRE(out_stride_bytes >= 12 && out_stride_bytes % 4 == 0, "output stride must be >= 12 and a multiple of 4");
+  ppp_ctx* ctx = c->ctx;
+  LOCK(ctx);
+  PPP_CUDA(cudaSetDevice(ctx->device));
+  *n_out = 0;
+  if (c->n_finite == 0) {
+    if (row_offsets) row_offsets[0] = 0;
+    return PPP_OK;
+  }
+  float4* rows_d = nullptr; int64_t* off_d = nullptr; int32_t* mem_d = nullptr;
+  PPP_TRY(dev_alloc(ctx, &rows_d, (size_t)c->n));
+  PPP_TRY(dev_alloc(ctx, &off_d, (size_t)c->n + 1));
+  PPP_TRY(dev_alloc(ctx, &mem_d, (size_t)c->n));
+  int64_t m = 0;
+  int st = voxel_grid_launch(c, leaf, rows_d, off_d, mem_d, &m);
+  std::vector<float4> rows;
+  if (st == PPP_OK) {
+    rows.resize((size_t)m);
+    PPP_CUDA(cudaMemcpyAsync(rows.data(), rows_d, (size_t)m * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    if (row_offsets) PPP_CUDA(cudaMemcpyAsync(row_offsets, off_d, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (members) PPP_CUDA(cudaMemcpyAsync(members, mem_d, (size_t)c->n_finite * 4, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  cudaError_t e = cudaStreamSynchronize(ctx->stream);
+  dev_free(ctx, rows_d); dev_free(ctx, off_d); dev_free(ctx, mem_d);
+  if (st != PPP_OK) return st;
+  PPP_CUDA(e);
+  const size_t put = out_stride_bytes >= 16 ? 16 : 12;   // x, y, z and the pad float where the record has one
+  for (int64_t r = 0; r < m; r++) memcpy((char*)points_out + (size_t)r * out_stride_bytes, &rows[(size_t)r], put);
+  *n_out = m;
+  return PPP_OK;
+}
+
 // ppp_mls_smooth's per-point part with the results left in device memory: one 32-byte record per point, by original
 // index, or on an exchange slab to the home ranks (only owned rows are queries there).  Does not synchronise.
 int ppp_dev_mls_smooth(ppp_cloud* c, double radius, int order, void* rows_dev, size_t row_stride_bytes) {

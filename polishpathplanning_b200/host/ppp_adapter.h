@@ -178,6 +178,40 @@ inline void mls_smooth(ppp_cloud* dc, PointCloudType& cloud, const std::string& 
   if (savePCDFile(out_name, cloud) != 0) fprintf(stderr, "smooth: could not write %s\n", out_name.c_str());
 }
 
+// voxel_down() (src/Path_Generation.cpp:53-59): pcl::VoxelGrid with leaf sizes (lx, ly, lz) on the device.  The cloud
+// is replaced by one point per occupied voxel: x, y, z from the device, r, g, b, a averaged over the voxel's members
+// as PCL's CentroidPoint does (float sums in member order, divided by the count, truncated).  Where PCL warns that the
+// leaf is too small and keeps the input, so does this.  Returns false then.
+inline bool voxel_down(ppp_cloud* dc, PointCloudType& cloud, float lx, float ly, float lz) {
+  const size_t n = cloud.points.size();
+  const float leaf[3] = {lx, ly, lz};
+  std::vector<PointType, decltype(cloud.points.get_allocator())> out(n);
+  std::vector<int64_t> off(n + 1);
+  std::vector<int32_t> members(n);
+  int64_t m = 0;
+  const int st = ppp_voxel_grid(dc, leaf, out.data(), sizeof(PointType), off.data(), members.data(), &m);
+  if (st == PPP_ERR_UNSUPPORTED) {
+    fprintf(stderr, "[pcl::VoxelGrid::applyFilter] %s\n", ppp_last_error());
+    return false;
+  }
+  check(st, "ppp_voxel_grid");
+  out.resize((size_t)m);
+  for (int64_t r = 0; r < m; r++) {
+    float sum[4] = {0.f, 0.f, 0.f, 0.f};   // bytes b, g, r, a of the rgba word
+    for (int64_t j = off[(size_t)r]; j < off[(size_t)r + 1]; j++) {
+      const uint32_t w = cloud.points[(size_t)members[(size_t)j]].rgba;
+      for (int c = 0; c < 4; c++) sum[c] += (float)((w >> (8 * c)) & 0xFFu);
+    }
+    const float cnt = (float)(off[(size_t)r + 1] - off[(size_t)r]);
+    uint32_t w = 0;
+    for (int c = 0; c < 4; c++) w |= ((uint32_t)(sum[c] / cnt) & 0xFFu) << (8 * c);
+    out[(size_t)r].rgba = w;
+  }
+  cloud.points.swap(out);
+  cloud.width = (uint32_t)m; cloud.height = 1;
+  return true;
+}
+
 inline MAP to_map(const Contours& c, int s) {
   MAP m;
   for (int64_t i = c.offsets[s]; i < c.offsets[s + 1]; i++) m[c.y[i]] = {c.x[i], c.z[i]};
@@ -213,6 +247,12 @@ public:
   void smooth() {  // src/Path_Generation.cpp:340-360
     ppp_host::mls_smooth(dev_.get(*cloud), *cloud, file_name);
     dev_.invalidate();
+  }
+
+  // src/Path_Generation.cpp:53-59: VoxelGrid::setLeafSize(lx, ly, lz); filter(*cloud).  The reference's leaf size is
+  // not part of this repository, so it is an argument here.
+  void voxel_down(float lx, float ly, float lz) {
+    if (ppp_host::voxel_down(dev_.get(*cloud), *cloud, lx, ly, lz)) dev_.invalidate();
   }
 
   void estimate_normal() {  // NormalEstimation, setRadiusSearch(2.5), viewpoint (0,0,0)

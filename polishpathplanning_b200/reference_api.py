@@ -451,6 +451,23 @@ class path_generater(_Base):
         self.toolRadius = float(Radius)
         self._load(cloud_name, change_range=True)
 
+    def voxel_down(self, leaf):
+        """voxel_down() (src/Path_Generation.cpp:53-59): pcl::VoxelGrid, filter(*cloud).  The reference's leaf size
+        is not part of this repository, so it is an argument (one float or three).  The cloud becomes one record per
+        occupied voxel (Cloud.voxel_grid) and the device copy is rebuilt on next use.  Where PCL warns that the leaf
+        is too small and keeps the input, so does this (and prints PCL's warning).  Returns the row offsets and
+        members of the voxels, or None when the cloud was kept."""
+        try:
+            recs, off, mem = self._dev().voxel_grid(leaf)
+        except api.PPPError as e:
+            if e.status != api._lib.PPP_ERR_UNSUPPORTED:
+                raise
+            print("[pcl::VoxelGrid::applyFilter] %s" % api._lib.load().ppp_last_error().decode())
+            return None
+        self.cloud = np.ascontiguousarray(recs)
+        self._invalidate()
+        return off, mem
+
     def insert_point(self, indices, PlanePoint):
         """std::map<double, std::vector<double>> insert_point(indices, PlanePoint): returns the map
         as (y, x, z) arrays in ascending y.  `indices`: strictly ascending point indices (every reference
