@@ -259,6 +259,24 @@ double ppp_mls_halo(double radius, double x_abs_max);
  * PCL's by at most (2n + 1) * 2^-24 * M; in practice most rows are bit-identical (DESIGN.md §2).          */
 int ppp_voxel_grid(ppp_cloud* cloud, const float leaf[3], void* points_out, size_t out_stride_bytes,
                    int64_t* row_offsets, int32_t* members, int64_t* n_out);
+/* voxel_down() with the rows left in device memory, as whole records the next cloud can be attached from
+ * (ppp_dev_cloud_attach(ctx, rows_dev, *n_rows, stride_bytes, ...)).  Same leaf validation, refusals (PCL's message
+ * included), rows, row offsets, members and x, y, z as ppp_voxel_grid.  All buffers are device memory:
+ *   rows_dev:        room for ppp_cloud_size(cloud) records of stride_bytes (>= 12, multiple of 4); every word of a
+ *                    row's record is written: x, y, z; the pad float 1.0f at byte 12 (stride >= 16); at byte 16
+ *                    (stride >= 20) PCL's AccumulatorRGBA over the rgba words at byte 16 of the members' source
+ *                    records (per byte channel a float32 sum in ascending source order, divided by the count and
+ *                    truncated); 0 elsewhere.  16-byte stores where the stride is a multiple of 16 and rows_dev is
+ *                    16-byte aligned;
+ *   src_dev:         the cloud's n source records in its index order, of the same stride (the buffer given to
+ *                    ppp_dev_cloud_attach); required when stride_bytes >= 20, ignored below;
+ *   row_offsets_dev: nullable, room for rows + 1 entries (at most the finite points + 1);
+ *   members_dev:     nullable, one entry per finite point (as ppp_voxel_grid's);
+ *   *n_rows:         rows written.
+ * A cloud without a finite point has 0 rows and row_offsets_dev[0] = 0.  On an error rows_dev is untouched and
+ * *n_rows is 0.  Synchronises once: on return the rows are in place. */
+int ppp_dev_voxel_grid(ppp_cloud* cloud, const float leaf[3], const void* src_dev, size_t stride_bytes, void* rows_dev,
+                       int64_t* row_offsets_dev, int32_t* members_dev, int64_t* n_rows);
 
 /* estimate_normal() followed by the plane sweep, as one call: what SectPath-derived GenPath does
  * (src/Path_Alg/path_dynamic_alg.cpp:343-366: estimate_normal(); kdtree.setInputCloud; sweep).

@@ -63,6 +63,7 @@ SIGNATURES = {
     "ppp_coverage_mark_radii": (C.c_int, [_vp, _vp, C.c_size_t, C.c_size_t, _vp, _vp]),
     "ppp_mls_smooth": (C.c_int, [_vp, C.c_double, C.c_int, _vp, C.c_size_t, _vp, _vp, _i64p]),
     "ppp_voxel_grid": (C.c_int, [_vp, _f32p, _vp, C.c_size_t, _vp, _vp, _i64p]),
+    "ppp_dev_voxel_grid": (C.c_int, [_vp, _f32p, _vp, C.c_size_t, _vp, _vp, _vp, _i64p]),
     "ppp_dev_mls_smooth": (C.c_int, [_vp, C.c_double, C.c_int, _vp, C.c_size_t]),
     "ppp_dev_mls_compact": (C.c_int, [_vp, _vp, C.c_int64, _vp, C.c_size_t, C.c_int64, C.c_int64, _vp, C.c_size_t, _vp, _vp,
                                       C.c_int64, _i64p]),

@@ -461,6 +461,22 @@ class Cloud:
         check(self.lib.ppp_dev_mls_smooth(self._h, float(radius), int(order), _vp(rows_ptr) if rows_ptr else None,
                                           int(row_stride_bytes)))
 
+    def dev_voxel_grid(self, leaf, rows_ptr, stride_bytes, src_ptr=None, offsets_ptr=None, members_ptr=None):
+        """ppp_dev_voxel_grid: voxel_down() into the device buffer rows_ptr (room for n records of stride_bytes), whole
+        records as Cloud.voxel_grid returns them, ready for Cloud(ctx, device_ptr=rows_ptr, n=rows, ...).  src_ptr: the
+        source records (needed from 20 bytes on, for the colours); defaults to the records this cloud was attached from
+        when they have the same stride.  offsets_ptr (rows + 1 int64) and members_ptr (one int32 per finite point):
+        optional device buffers.  Synchronises; returns the row count."""
+        lf = np.broadcast_to(np.asarray(leaf, np.float32), (3,)).copy()
+        if src_ptr is None and isinstance(self._records, tuple) and self._records[1] == int(stride_bytes):
+            src_ptr = self._records[0]
+        m = C.c_int64(0)
+        check(self.lib.ppp_dev_voxel_grid(self._h, lf.ctypes.data_as(_lib._f32p), _vp(src_ptr) if src_ptr else None,
+                                          int(stride_bytes), _vp(rows_ptr) if rows_ptr else None,
+                                          _vp(offsets_ptr) if offsets_ptr else None,
+                                          _vp(members_ptr) if members_ptr else None, C.byref(m)))
+        return m.value
+
     def dev_set_normal_row_map(self, map_ptr):
         """Device int32 map row -> record of the normals buffer (negative: skip); None = identity."""
         check(self.lib.ppp_dev_set_normal_row_map(self._h, _vp(map_ptr) if map_ptr else None))

@@ -974,13 +974,17 @@ int ppp_mls_smooth(ppp_cloud* c, double radius, int order, void* points_out, siz
 
 double ppp_mls_halo(double radius, double x_abs_max) { return mls_halo(radius, x_abs_max); }
 
+static bool leaf_ok(const float leaf[3]) {
+  for (int d = 0; d < 3; d++)
+    if (!(leaf[d] > 0 && std::isfinite(leaf[d]) && std::isfinite(1.0f / leaf[d]))) return false;
+  return true;
+}
+
 // voxel_down(): pcl::VoxelGrid with leaf sizes leaf[0..2] (src/Path_Generation.cpp:53-59); contract in the header.
 int ppp_voxel_grid(ppp_cloud* c, const float leaf[3], void* points_out, size_t out_stride_bytes, int64_t* row_offsets,
                    int32_t* members, int64_t* n_out) {
   REQUIRE(c && leaf && n_out && (points_out || c->n == 0), "NULL argument");
-  for (int d = 0; d < 3; d++)
-    REQUIRE(leaf[d] > 0 && std::isfinite(leaf[d]) && std::isfinite(1.0f / leaf[d]),
-            "leaf sizes must be > 0 and finite, with a finite float inverse");
+  REQUIRE(leaf_ok(leaf), "leaf sizes must be > 0 and finite, with a finite float inverse");
   REQUIRE(out_stride_bytes >= 12 && out_stride_bytes % 4 == 0, "output stride must be >= 12 and a multiple of 4");
   ppp_ctx* ctx = c->ctx;
   LOCK(ctx);
@@ -995,7 +999,7 @@ int ppp_voxel_grid(ppp_cloud* c, const float leaf[3], void* points_out, size_t o
   PPP_TRY(dev_alloc(ctx, &off_d, (size_t)c->n + 1));
   PPP_TRY(dev_alloc(ctx, &mem_d, (size_t)c->n));
   int64_t m = 0;
-  int st = voxel_grid_launch(c, leaf, rows_d, off_d, mem_d, &m);
+  int st = voxel_grid_launch(c, leaf, nullptr, 4, (float*)rows_d, off_d, mem_d, &m);
   std::vector<float4> rows;
   if (st == PPP_OK) {
     rows.resize((size_t)m);
@@ -1010,6 +1014,41 @@ int ppp_voxel_grid(ppp_cloud* c, const float leaf[3], void* points_out, size_t o
   const size_t put = out_stride_bytes >= 16 ? 16 : 12;   // x, y, z and the pad float where the record has one
   for (int64_t r = 0; r < m; r++) memcpy((char*)points_out + (size_t)r * out_stride_bytes, &rows[(size_t)r], put);
   *n_out = m;
+  return PPP_OK;
+}
+
+// voxel_down() with the rows left in device memory as whole records of stride_bytes (see the header).  Synchronises once.
+int ppp_dev_voxel_grid(ppp_cloud* c, const float leaf[3], const void* src_dev, size_t stride_bytes, void* rows_dev,
+                       int64_t* row_offsets_dev, int32_t* members_dev, int64_t* n_rows) {
+  REQUIRE(n_rows, "n_rows is NULL");
+  *n_rows = 0;
+  REQUIRE(c && leaf, "NULL argument");
+  REQUIRE(leaf_ok(leaf), "leaf sizes must be > 0 and finite, with a finite float inverse");
+  REQUIRE(stride_bytes >= 12 && stride_bytes % 4 == 0, "stride_bytes must be >= 12 and a multiple of 4");
+  REQUIRE(c->n == 0 || (rows_dev && (uintptr_t)rows_dev % 4 == 0), "rows_dev: room for n 4-byte aligned records");
+  const bool rgba = stride_bytes >= 20;
+  REQUIRE(!rgba || c->n == 0 || (src_dev && (uintptr_t)src_dev % 4 == 0),
+          "records of 20 bytes or more average the rgba word of the source records: src_dev is required");
+  REQUIRE((uintptr_t)row_offsets_dev % 8 == 0 && (uintptr_t)members_dev % 4 == 0, "misaligned row_offsets_dev / members_dev");
+  ppp_ctx* ctx = c->ctx;
+  LOCK(ctx);
+  PPP_CUDA(cudaSetDevice(ctx->device));
+  if (c->n_finite == 0) {
+    if (row_offsets_dev) PPP_CUDA(cudaMemsetAsync(row_offsets_dev, 0, 8, ctx->stream));
+    PPP_CUDA(cudaStreamSynchronize(ctx->stream));
+    return PPP_OK;
+  }
+  int64_t* off_d = row_offsets_dev;
+  int32_t* mem_d = members_dev;
+  if (!off_d) PPP_TRY(dev_alloc(ctx, &off_d, (size_t)c->n_finite + 1));
+  if (!mem_d) PPP_TRY(dev_alloc(ctx, &mem_d, (size_t)c->n_finite));
+  int64_t m = 0;
+  const int st = voxel_grid_launch(c, leaf, rgba ? (const float*)src_dev : nullptr, (int)(stride_bytes / 4), (float*)rows_dev,
+                                   off_d, mem_d, &m);
+  if (!row_offsets_dev) dev_free(ctx, off_d);
+  if (!members_dev) dev_free(ctx, mem_d);
+  if (st != PPP_OK) return st;
+  *n_rows = m;
   return PPP_OK;
 }
 

@@ -390,11 +390,13 @@ int mls_compact_launch(ppp_ctx* ctx, const float* rec, int64_t n, const float* s
 double mls_halo(double radius, double x_abs_max);
 
 // voxel.cu
-// ppp_voxel_grid's device part (leaf already validated): rows_dev {x, y, z, 1} per voxel in ascending key order,
-// row_off_dev (rows + 1) and members_dev (the n_finite source indices grouped by row, ascending within a row); each
-// buffer holds n (+1) entries.  PPP_ERR_UNSUPPORTED where PCL refuses the leaf.  Synchronises.
-int voxel_grid_launch(ppp_cloud* c, const float leaf[3], float4* rows_dev, int64_t* row_off_dev, int32_t* members_dev,
-                      int64_t* n_rows);
+// ppp_voxel_grid's and ppp_dev_voxel_grid's device part (leaf already validated): one record of sf words per voxel in
+// ascending key order into rows_dev (room for n records; x, y, z, 1.0f, the averaged rgba word 4 of the source
+// records src when it is not NULL, zeros elsewhere), row_off_dev (rows + 1) and members_dev (the n_finite source
+// indices grouped by row, ascending within a row).  PPP_ERR_UNSUPPORTED where PCL refuses the leaf, before anything is
+// written.  Synchronises.
+int voxel_grid_launch(ppp_cloud* c, const float leaf[3], const float* src, int sf, float* rows_dev, int64_t* row_off_dev,
+                      int32_t* members_dev, int64_t* n_rows);
 
 // slices.cu
 int bands_launch(ppp_cloud* c, const float* plane_x_host, int S, float half_width, int truncate_center, int sort_bands,

@@ -11,8 +11,9 @@
 //               __match_any_sync.  The input is in ascending point order, so every voxel's members end up in
 //               ascending source index;
 //   segments:   boundary flags -> scan -> voxel ordinals -> row offsets;
-//   centroid:   per voxel, a sequential float32 sum of x, y, z in member order, then a division by (float)count
-//               (the library is built with --fmad=false, and the adds and the division are explicitly rounded).
+//   centroid:   per voxel, a sequential float32 sum of x, y, z (and of the rgba bytes of the source records, when
+//               given) in member order, then a division by (float)count (the library is built with --fmad=false, and
+//               the adds and the divisions are explicitly rounded), written as a whole record of the caller's stride.
 // PCL sums in the order its unstable std::sort leaves each voxel, which only differs in the last bits of the
 // centroids: the tolerance contract is in include/ppp_gpu.h (ppp_voxel_grid) and DESIGN.md §2.
 #include <algorithm>
@@ -125,32 +126,64 @@ __global__ void __launch_bounds__(256) k_voxel_offsets(const int32_t* __restrict
   if (i == 0) row_off[ord[m]] = m;
 }
 
-// One thread per voxel: CentroidPoint's x, y, z (AccumulatorXYZ: a float32 sum in member order divided by the count),
-// and the pad float of a default-constructed point.
+// One thread per voxel: a CentroidPoint record of sf words (row r at out + r * sf).  x, y, z: AccumulatorXYZ, a float32
+// sum in member order divided by (float)count; word 3 (sf >= 4): the pad float 1.0f of a default-constructed point;
+// word 4 (sf >= 5), with source records src of sf words: AccumulatorRGBA over their word 4, per byte channel a float32
+// sum in member order divided by the count and truncated; every other word 0.  vec: sf % 4 == 0 and out 16-byte
+// aligned, so that whole records go out as 16-byte stores.  Records and members index the n points of the cloud.
+// RGBA: src is not NULL (the colour sums live in registers only where they are needed).
+template <bool RGBA>
 __global__ void __launch_bounds__(256) k_voxel_centroid(const int64_t* __restrict__ row_off, const int32_t* __restrict__ rows_dev,
                                                         const int32_t* __restrict__ members, const float4* __restrict__ xyz4,
-                                                        float4* __restrict__ out) {
+                                                        int64_t n, const uint32_t* __restrict__ src, int sf, bool vec,
+                                                        float* __restrict__ out) {
   pdl_prologue();
   const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= *rows_dev) return;
   const int64_t a = row_off[r], b = row_off[r + 1];
   float sx = 0.f, sy = 0.f, sz = 0.f;
+  float c0 = 0.f, c1 = 0.f, c2 = 0.f, c3 = 0.f;   // bytes 0..3 of the rgba word
   for (int64_t j = a; j < b; j++) {
-    const float4 p = xyz4[members[j]];
+    const int32_t i = members[j];
+    PPP_DEV_ASSERT(i >= 0 && i < n);
+    const float4 p = xyz4[i];
     sx = __fadd_rn(sx, p.x);
     sy = __fadd_rn(sy, p.y);
     sz = __fadd_rn(sz, p.z);
+    if (RGBA) {
+      const uint32_t w = src[(int64_t)i * sf + 4];
+      c0 = __fadd_rn(c0, (float)(w & 0xffu));
+      c1 = __fadd_rn(c1, (float)((w >> 8) & 0xffu));
+      c2 = __fadd_rn(c2, (float)((w >> 16) & 0xffu));
+      c3 = __fadd_rn(c3, (float)(w >> 24));
+    }
   }
   const float cnt = (float)(b - a);
-  out[r] = make_float4(__fdiv_rn(sx, cnt), __fdiv_rn(sy, cnt), __fdiv_rn(sz, cnt), 1.0f);
+  const float x = __fdiv_rn(sx, cnt), y = __fdiv_rn(sy, cnt), z = __fdiv_rn(sz, cnt);
+  uint32_t rgba = 0u;
+  if (RGBA)   // past 2^24 a channel sum has rounded and its quotient can reach 256: only the low byte is kept
+    rgba = (__float2uint_rz(__fdiv_rn(c0, cnt)) & 0xffu) | (__float2uint_rz(__fdiv_rn(c1, cnt)) & 0xffu) << 8 |
+           (__float2uint_rz(__fdiv_rn(c2, cnt)) & 0xffu) << 16 | (__float2uint_rz(__fdiv_rn(c3, cnt)) & 0xffu) << 24;
+  PPP_DEV_ASSERT(r < n);
+  float* o = out + r * sf;
+  if (vec) {
+    float4* o4 = reinterpret_cast<float4*>(o);
+    o4[0] = make_float4(x, y, z, 1.0f);
+    for (int q = 1; q < sf / 4; q++) o4[q] = make_float4(q == 1 ? __uint_as_float(rgba) : 0.f, 0.f, 0.f, 0.f);
+  } else {
+    o[0] = x; o[1] = y; o[2] = z;
+    if (sf > 3) o[3] = 1.0f;
+    if (sf > 4) o[4] = __uint_as_float(rgba);
+    for (int k = 5; k < sf; k++) o[k] = 0.f;
+  }
 }
 
 inline unsigned blocks_for(int64_t n, int t) { return (unsigned)((n + t - 1) / t); }
 
 }  // namespace
 
-int voxel_grid_launch(ppp_cloud* c, const float leaf[3], float4* rows_dev, int64_t* row_off_dev, int32_t* members_dev,
-                      int64_t* n_rows) {
+int voxel_grid_launch(ppp_cloud* c, const float leaf[3], const float* src, int sf, float* rows_dev, int64_t* row_off_dev,
+                      int32_t* members_dev, int64_t* n_rows) {
   ppp_ctx* ctx = c->ctx;
   *n_rows = 0;
   const int64_t m = c->n_finite;
@@ -195,19 +228,24 @@ int voxel_grid_launch(ppp_cloud* c, const float leaf[3], float4* rows_dev, int64
 
   const int64_t n = c->n;
   uint32_t *keys[2] = {nullptr, nullptr};
-  int32_t* vals_tmp = nullptr;
+  int32_t *vals_tmp = nullptr, *vals_mid = nullptr;
   int32_t *counts = nullptr, *offsets = nullptr, *flags = nullptr, *ord = nullptr;
   const int n_seg_max = (int)((n + VX_SEG - 1) / VX_SEG);
   PPP_TRY(dev_alloc(ctx, &keys[0], (size_t)n));
   PPP_TRY(dev_alloc(ctx, &keys[1], (size_t)n));
   PPP_TRY(dev_alloc(ctx, &vals_tmp, (size_t)n));
+  if ((passes & 1) == 0) PPP_TRY(dev_alloc(ctx, &vals_mid, (size_t)m));
   PPP_TRY(dev_alloc(ctx, &counts, (size_t)VX_DIGITS * n_seg_max));
   PPP_TRY(dev_alloc(ctx, &offsets, (size_t)VX_DIGITS * n_seg_max + 1));
   PPP_TRY(dev_alloc(ctx, &flags, (size_t)m));
   PPP_TRY(dev_alloc(ctx, &ord, (size_t)m + 1));
-  // stage s (0: key pass, p + 1: sort pass p) writes keys[s & 1] and the values into members_dev for the last stage,
-  // alternating backwards from there
-  auto vals_of = [&](int s) { return ((passes - s) & 1) == 0 ? members_dev : vals_tmp; };
+  // stage s (0: key pass over the n points, p + 1: sort pass p over the m finite ones) writes keys[s & 1] and its values:
+  // the key pass into vals_tmp (n entries), the last stage into members_dev (m entries, so the key pass never goes
+  // there), the stages between alternately into vals_tmp and members_dev backwards from the last; where that would make
+  // the first sort pass write its own input vals_tmp (an even number of passes), it writes vals_mid
+  auto vals_of = [&](int s) {
+    return s == 0 ? vals_tmp : ((passes - s) & 1) == 0 ? members_dev : s == 1 ? vals_mid : vals_tmp;
+  };
   PPP_LAUNCH(ctx, "voxel_keys", k_voxel_keys, blocks_for(n, 256), 256, 0, (const float4*)c->xyz4, n, kp, keys[0], vals_of(0));
   PPP_CHECK_LAUNCH();
   for (int p = 0; p < passes; p++) {
@@ -232,13 +270,16 @@ int voxel_grid_launch(ppp_cloud* c, const float leaf[3], float4* rows_dev, int64
   PPP_LAUNCH(ctx, "voxel_offsets", k_voxel_offsets, blocks_for(m, 256), 256, 0, (const int32_t*)flags, (const int32_t*)ord, m,
              row_off_dev);
   PPP_CHECK_LAUNCH();
-  PPP_LAUNCH(ctx, "voxel_centroid", k_voxel_centroid, blocks_for(m, 256), 256, 0, (const int64_t*)row_off_dev,
-             (const int32_t*)(ord + m), (const int32_t*)members_dev, (const float4*)c->xyz4, rows_dev);
+  const bool vec = sf % 4 == 0 && (uintptr_t)rows_dev % 16 == 0;
+  auto* centroid = src ? k_voxel_centroid<true> : k_voxel_centroid<false>;
+  PPP_LAUNCH(ctx, "voxel_centroid", centroid, blocks_for(m, 256), 256, 0, (const int64_t*)row_off_dev,
+             (const int32_t*)(ord + m), (const int32_t*)members_dev, (const float4*)c->xyz4, n, (const uint32_t*)src, sf, vec,
+             rows_dev);
   PPP_CHECK_LAUNCH();
   int32_t rows = 0;
   PPP_CUDA(cudaMemcpyAsync(&rows, ord + m, 4, cudaMemcpyDeviceToHost, ctx->stream));
   PPP_CUDA(cudaStreamSynchronize(ctx->stream));
-  dev_free(ctx, keys[0]); dev_free(ctx, keys[1]); dev_free(ctx, vals_tmp);
+  dev_free(ctx, keys[0]); dev_free(ctx, keys[1]); dev_free(ctx, vals_tmp); dev_free(ctx, vals_mid);
   dev_free(ctx, counts); dev_free(ctx, offsets); dev_free(ctx, flags); dev_free(ctx, ord);
   *n_rows = rows;
   return PPP_OK;
