@@ -291,7 +291,23 @@ int ppp_normals_and_contours(ppp_cloud* cloud, int k, double radius, const float
 /* ------------------------------------------------------------------------------------------ */
 /* device API (results stay in HBM; used by bench.py's device-resident leg and the multi-GPU
  * sharding in polishpathplanning_b200/parallel.py).  Query sub-ranges are given in SORTED
- * (cell-major) order so that a rank's share is spatially compact: [first, first+count).        */
+ * (cell-major) order so that a rank's share is spatially compact: [first, first+count).
+ *  - ranges: 0 <= first <= (finite points), count < 0 = up to the end, first + count <= (finite points); anything
+ *    else is PPP_ERR_INVALID, with nothing written or launched.  The ranges of ppp_dev_normals_knn(k) refer to the
+ *    order ppp_dev_sorted_order returns after ppp_dev_index(cloud, k, 0), those of ppp_dev_normals_radius(r) to the
+ *    order after ppp_dev_index(cloud, 0, r).  A sub-range is always searched on that (primary) grid; the full range
+ *    of a cloud that is not a height field runs on one grid per axis pair.  The results are the same either way:
+ *    the union of the sub-range calls over [0, finite points) is the full-range call, bit for bit.
+ *  - rows written: those of the range's points (by original index).  The rows of the non-finite points get their
+ *    defaults (ids -1, d2 inf, NaN normal) only from the call whose range starts at 0.  Through a row map
+ *    (ppp_dev_set_normal_row_map) a normal record goes to record map[row] instead, or nowhere for a negative entry;
+ *    ids and d2 are not mapped.
+ *  - normal records: stride 16 {nx, ny, nz, curvature}; stride 32 pcl::Normal {nx, ny, nz, 0, curvature, 0, 0, 0};
+ *    strides 20..28 floats 0..3 = {nx, ny, nz, curvature}; strides above 32 floats 0..4 = {nx, ny, nz, 0, curvature}.
+ *    Every other float of a record is left as it was (the host API zero-fills records wider than 32 bytes).
+ *  - alignment: normals_dev 16 bytes when the stride is a multiple of 16 (16-byte vector stores; 32-byte ones from a
+ *    32-byte aligned buffer at stride 32), 4 otherwise; knn_idx_dev, knn_d2_dev and pts_dev of ppp_dev_cloud_attach
+ *    4 bytes.  Misaligned buffers are PPP_ERR_INVALID.                                                           */
 int ppp_dev_index(ppp_cloud* cloud, int k_hint, double radius_hint); /* (re)build the grid now */
 int ppp_dev_normals_knn(ppp_cloud* cloud, int k, const float viewpoint[3], unsigned flags, int64_t first,
                         int64_t count, float* normals_dev, size_t normal_stride_bytes,
@@ -335,7 +351,8 @@ int ppp_peer_buffer_close(ppp_ctx* ctx, void* dev_ptr);
 int ppp_peer_buffer_free(ppp_ctx* ctx, void* dev_ptr);
 /* stream-ordered device -> host copy of a raw device range, then synchronise */
 int ppp_dev_download(ppp_ctx* ctx, void* host_dst, const void* dev_src, size_t bytes);
-/* original index of the point at sorted position p (device array of n int32) */
+/* original index of the point at sorted position p (device array of one int32 per finite point) of the grid the
+ * last ppp_dev_index built or found; NULL before any ppp_dev_index.  Valid while the cloud lives.              */
 const int32_t* ppp_dev_sorted_order(ppp_cloud* cloud);
 
 /* ------------------------------------------------------------------------------------------ */

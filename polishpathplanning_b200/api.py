@@ -442,6 +442,12 @@ class Cloud:
     def dev_index(self, k_hint=16, radius_hint=0.0):
         check(self.lib.ppp_dev_index(self._h, int(k_hint), float(radius_hint)))
 
+    def dev_sorted_order(self):
+        """Device pointer to the original index of each sorted position (one int32 per finite point) of the grid the
+        last dev_index built or found: the positions dev_normals_knn / dev_normals_radius ranges count.  None before
+        any dev_index."""
+        return self.lib.ppp_dev_sorted_order(self._h)
+
     def dev_normals_knn(self, k, normals_ptr, normal_stride_bytes, idx_ptr=None, d2_ptr=None, first=0, count=-1,
                         viewpoint=(0.0, 0.0, 0.0), flags=PPP_COV_PCL110):
         vp = np.asarray(viewpoint, np.float32)

@@ -227,6 +227,7 @@ int ppp_dev_cloud_attach(ppp_ctx* ctx, const void* pts_dev, size_t n, size_t str
   REQUIRE(ctx && out, "ctx/out is NULL");
   REQUIRE(stride_bytes >= 12 && stride_bytes % 4 == 0, "stride_bytes must be >= 12 and a multiple of 4");
   REQUIRE(n == 0 || pts_dev, "pts is NULL");
+  REQUIRE((uintptr_t)pts_dev % 4 == 0, "pts_dev must be 4-byte aligned");
   REQUIRE(n < 2147483647ull, "at most 2^31-2 points (int32 indices, as PCL)");
   LOCK(ctx);
   PPP_CUDA(cudaSetDevice(ctx->device));
@@ -402,12 +403,15 @@ int ppp_dev_download(ppp_ctx* ctx, void* host_dst, const void* dev_src, size_t b
   return PPP_OK;
 }
 
+// The order of the grid the last ppp_dev_index built or found: the primary grid whose sorted positions the query
+// ranges of ppp_dev_normals_knn / _radius with the same k / radius refer to.  (The most recently created grid is not
+// it: the multi-projection index and calls with other cell sizes add grids of their own.)
 const int32_t* ppp_dev_sorted_order(ppp_cloud* c) {
-  if (!c || c->grids.empty()) return nullptr;
+  if (!c || !c->index_grid) return nullptr;
   ApiScope scope(c->ctx);
   if (cudaSetDevice(c->ctx->device) != cudaSuccess) return nullptr;
-  if (grid_sorted_order(c, c->grids.back()) != PPP_OK) return nullptr;
-  return c->grids.back().order;
+  if (grid_sorted_order(c, *c->index_grid) != PPP_OK) return nullptr;
+  return c->index_grid->order;
 }
 
 int ppp_dev_index(ppp_cloud* c, int k_hint, double radius_hint) {
@@ -416,22 +420,38 @@ int ppp_dev_index(ppp_cloud* c, int k_hint, double radius_hint) {
   PPP_CUDA(cudaSetDevice(c->ctx->device));
   GridStore* g;
   double h = radius_hint > 0 ? cloud_cell_for_radius(c, radius_hint) : cloud_cell_for_k(c, k_hint > 0 ? k_hint : 16);
-  return cloud_get_grid(c, h, &g);
+  PPP_TRY(cloud_get_grid(c, h, &g));
+  c->index_grid = g;
+  return PPP_OK;
 }
 
 // ---------------------------------------------------------------------------------------------
 // device-level pipeline entries
 // ---------------------------------------------------------------------------------------------
+// Normal records of a stride that is a multiple of 16 bytes are written with 16-byte (and, from a 32-byte aligned
+// buffer, 32-byte) vector stores (store_normal); every other record float by float.
+static bool normals_aligned(const float* normals_dev, size_t stride_bytes) {
+  return (uintptr_t)normals_dev % (stride_bytes % 16 == 0 ? 16 : 4) == 0;
+}
+
+// [first, first + *count) within the n_finite sorted positions; a negative count runs to the end.
+static bool query_range(const ppp_cloud* c, int64_t first, int64_t* count) {
+  if (first < 0 || first > c->n_finite) return false;
+  if (*count < 0) *count = c->n_finite - first;
+  return *count <= c->n_finite - first;
+}
+
 int ppp_dev_normals_knn(ppp_cloud* c, int k, const float vp[3], unsigned flags, int64_t first, int64_t count,
                         float* normals_dev, size_t normal_stride_bytes, int32_t* knn_idx_dev, float* knn_d2_dev) {
   REQUIRE(c, "cloud is NULL");
   REQUIRE(k >= 1, "k must be >= 1");
   REQUIRE(normal_stride_bytes >= 16 && normal_stride_bytes % 4 == 0, "normal stride must be >= 16 and a multiple of 4");
   REQUIRE(normals_dev || knn_idx_dev, "nothing to compute");
+  REQUIRE(normals_aligned(normals_dev, normal_stride_bytes), "normals_dev must be 16-byte aligned");
+  REQUIRE((uintptr_t)knn_idx_dev % 4 == 0 && (uintptr_t)knn_d2_dev % 4 == 0, "knn_idx_dev / knn_d2_dev must be 4-byte aligned");
   LOCK(c->ctx);
   PPP_CUDA(cudaSetDevice(c->ctx->device));
-  if (count < 0) count = c->n_finite - first;
-  REQUIRE(first >= 0 && first + count <= c->n_finite, "query range outside the indexed points");
+  REQUIRE(query_range(c, first, &count), "query range outside the indexed points");
   GridStore* g;
   const double h = cloud_cell_for_k(c, k);
   PPP_TRY(cloud_get_grid(c, h, &g));
@@ -455,10 +475,10 @@ int ppp_dev_normals_radius(ppp_cloud* c, double radius, const float vp[3], unsig
   REQUIRE(c && normals_dev, "NULL argument");
   REQUIRE(radius > 0 && std::isfinite(radius), "radius must be > 0");
   REQUIRE(normal_stride_bytes >= 16 && normal_stride_bytes % 4 == 0, "normal stride must be >= 16 and a multiple of 4");
+  REQUIRE(normals_aligned(normals_dev, normal_stride_bytes), "normals_dev must be 16-byte aligned");
   LOCK(c->ctx);
   PPP_CUDA(cudaSetDevice(c->ctx->device));
-  if (count < 0) count = c->n_finite - first;
-  REQUIRE(first >= 0 && first + count <= c->n_finite, "query range outside the indexed points");
+  REQUIRE(query_range(c, first, &count), "query range outside the indexed points");
   GridStore* g;
   const double h = cloud_cell_for_radius(c, radius);
   PPP_TRY(cloud_get_grid(c, h, &g));

@@ -168,6 +168,7 @@ struct ppp_cloud {
   std::vector<MPSet> mps;
   float cell_hint = 0;
   std::vector<GridStore> grids;
+  GridStore* index_grid = nullptr;   // the primary grid of the last ppp_dev_index (ppp_dev_sorted_order)
   // results of the last ppp_dev_slice_contours (owned by the cloud)
   int64_t* c_node_off = nullptr;
   double *c_y = nullptr, *c_x = nullptr, *c_z = nullptr;

@@ -48,16 +48,41 @@ def test_radius_lists_bit_exact(ctx, n, seed):
     gc.close()
 
 
+def _viewpoint(cloud, where):
+    """'origin': PCL's default (0, 0, 0), at a corner of the panels; 'above': the x/y centre of the cloud at z = +100,
+    well off the surface."""
+    if where == "origin":
+        return (0.0, 0.0, 0.0)
+    lo, hi = np.nanmin(cloud[:, :3], axis=0), np.nanmax(cloud[:, :3], axis=0)
+    return (float(lo[0] + hi[0]) / 2, float(lo[1] + hi[1]) / 2, 100.0)
+
+
+def _assert_flip_margin(cloud, o, vp, where):
+    """Normals within the tolerance of each other must not fall on opposite sides of the viewpoint flip: every finite
+    row's |(vp - q).n| clears 1e-3.  The origin lies close to the tangent planes of a few points of the 100000-point
+    panel (|(vp - q).n| down to 1.1e-4 at |vp - q| ~ 160: a normal 7e-7 away, ten float ulps, can have the other
+    sign), so there the comparison holds only while those normals come out as the oracle's; the margin is asserted
+    where the viewpoint is off the surface."""
+    if where == "origin":
+        return
+    ok = ~np.isnan(o[:, 0])
+    w = np.asarray(vp, np.float64) - cloud[ok, :3].astype(np.float64)
+    assert np.abs((w * o[ok, :3].astype(np.float64)).sum(axis=1)).min() > 1e-3
+
+
 @pytest.mark.parametrize("n,seed", [(4000, 1), (100000, 3)])
 @pytest.mark.parametrize("flags", [api.PPP_COV_PCL110, api.PPP_COV_SHIFTED])
-def test_normals_radius(ctx, n, seed, flags):
+@pytest.mark.parametrize("where", ["origin", "above"])
+def test_normals_radius(ctx, n, seed, flags, where):
     cloud = synth.panel(n, seed)
+    vp = _viewpoint(cloud, where)
     oc = po.OracleCloud(cloud)
     gc = api.Cloud(ctx, cloud)
-    g = gc.normals_radius(2.5, flags=flags)
-    o, _ = oc.normals(radius=2.5, cov_variant=flags)
+    g = gc.normals_radius(2.5, viewpoint=vp, flags=flags)
+    o, _ = oc.normals(radius=2.5, viewpoint=vp, cov_variant=flags)
+    _assert_flip_margin(cloud, o, vp, where)
     mx, frac_exact = _cmp_normals(g, o)
-    print("normals_radius n=%d flags=%d max|diff|=%.3g bit-exact rows=%.4f" % (n, flags, mx, frac_exact))
+    print("normals_radius n=%d flags=%d vp=%s max|diff|=%.3g bit-exact rows=%.4f" % (n, flags, where, mx, frac_exact))
     assert mx <= NORMAL_TOL
     assert np.all(g[:, 3] == 0) and np.all(g[:, 5:8] == 0)  # pcl::Normal padding
     gc.close()
@@ -65,16 +90,20 @@ def test_normals_radius(ctx, n, seed, flags):
 
 @pytest.mark.parametrize("n,seed", [(4000, 1), (100000, 3)])
 @pytest.mark.parametrize("k", [10, 16, 32])
-def test_normals_knn(ctx, n, seed, k):
+@pytest.mark.parametrize("flags", [api.PPP_COV_PCL110, api.PPP_COV_SHIFTED])
+@pytest.mark.parametrize("where", ["origin", "above"])
+def test_normals_knn(ctx, n, seed, k, flags, where):
     cloud = synth.panel(n, seed)
+    vp = _viewpoint(cloud, where)
     oc = po.OracleCloud(cloud)
     gc = api.Cloud(ctx, cloud)
-    g, gi = gc.normals_knn(k, return_idx=True)
-    o, _ = oc.normals(k=k)
+    g, gi = gc.normals_knn(k, viewpoint=vp, flags=flags, return_idx=True)
+    o, _ = oc.normals(k=k, viewpoint=vp, cov_variant=flags)
+    _assert_flip_margin(cloud, o, vp, where)
     oi, _ = oc.knn(k, want_d2=False)
     assert np.array_equal(gi, oi)
     mx, frac_exact = _cmp_normals(g, o)
-    print("normals_knn n=%d k=%d max|diff|=%.3g bit-exact rows=%.4f" % (n, k, mx, frac_exact))
+    print("normals_knn n=%d k=%d flags=%d vp=%s max|diff|=%.3g bit-exact rows=%.4f" % (n, k, flags, where, mx, frac_exact))
     assert mx <= NORMAL_TOL
     gc.close()
 
